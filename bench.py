@@ -24,6 +24,12 @@ is  back-project+quantise -> read (normalise, fp16, gather, pool x3) -> write (c
 `--impl reference` times that CPU implementation alone (the reference cannot run as committed: hard-coded
 .cuda() and detectron2 imports), on a bounded sample of the same workload per step.
 
+`--dump-outputs DIR` writes, after the timed steps, what the last of them handed its caller: the three pooled levels of its
+last frame (level0..2, (E,C,h,w)) and the grid state (sums (E,cells,C), counts (E,cells)), each as DIR/<name>.npy in float32.
+The inputs are seeded, so two builds run with the same arguments can be compared output for output; every step starts from
+a reset grid, so the dumped arrays do not depend on --steps / --warmup either.  Counts repeat bit for bit; the write adds
+fp32 features in a run-dependent order, so sums (and the fp16 levels read from them) may differ in the last bits.
+
 Multi-GPU (torchrun, one process per GPU): episodes are sharded `episode % world == rank`, per-GPU work fixed
 (64 episodes each, "weak"), no collective on the hot path; one all_reduce(MAX) for the time and one
 all_reduce(SUM) for the frame counters after the loop.
@@ -177,6 +183,22 @@ def pcie_info(gpu: int):
     return info
 
 
+DUMP_SAMPLE = 1 << 21          # elements per dumped array at most: 5 arrays x 8 MB in float32
+
+
+def dump_outputs(out_dir: str, arrays: dict, seed: int = 0) -> None:
+    """Write each tensor as out_dir/<name>.npy in float32.  One larger than DUMP_SAMPLE elements is represented by its elements at
+    DUMP_SAMPLE distinct flat positions (row-major over its logical shape, ascending) drawn by numpy's default_rng(seed): the
+    positions depend on the shape alone, so they are the same in every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        n = t.numel()
+        if n > DUMP_SAMPLE:
+            pos = np.sort(np.random.default_rng(seed).choice(n, DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(pos).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def write_launch_bytes(E: int, touched_per_launch: float, c: int = C) -> float:
     """Algorithmic bytes of ONE eod_write_mean launch over E episodes (DESIGN.md 'Roofline accounting'):
     features read once + index plane + touched grid rows read-modify-written + per-cell sample counts."""
@@ -317,12 +339,14 @@ def main_gpu(args, rank, local_rank, world):
     slabs = [torch.randn((E, C, H, W), device=dev, generator=gen) for _ in range(2)]          # 2 x 20.1 GB
     # inputs are resident and static for the whole run, which is what pipeline=True asks of the caller
     batch = eod.EpisodeBatch(E, MAP_W, MAP_H, C, H, W, dev, variant=args.write_variant, pipeline=not args.no_pipeline)
+    last_levels = []                                                 # what step() returned for the last frame of the last step
 
     def one_step():
         batch.reset()
         for t in range(N_FRAMES):
-            batch.step(depth[t], pose[t], shifts, intr, float(CELL), slabs[t & 1])
+            levels = batch.step(depth[t], pose[t], shifts, intr, float(CELL), slabs[t & 1])
         batch.join()                                                 # the timing events sit on the caller's stream
+        last_levels[:] = levels
 
     def barrier():
         if world > 1:
@@ -342,6 +366,8 @@ def main_gpu(args, rank, local_rank, world):
     stage_ms = batch.stage_ms()
     batch.profile(False)
     visible_last_step = float(batch.counts.sum().item())            # +1 per visible cell per frame since the reset
+    if args.dump_outputs and rank == 0:                              # before the extras below reuse the batch
+        dump_outputs(args.dump_outputs, {**{f"level{k}": l for k, l in enumerate(last_levels)}, "sums": batch.sums, "counts": batch.counts})
     totals = sharding.gather_counters({"frames": float(args.steps * E * N_FRAMES), "visible": visible_last_step}, dev)
 
     ms_per_step = ms_total / args.steps
@@ -906,7 +932,8 @@ def run_e2e_variants(eod, batch, dev, depth_h, pose_h, shifts, intr, args, world
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of the headline loop and of value_with_fusion; roofline_1000 "
+                    "times max(2, min(steps, 5)) steps of its larger grid and reports that count as its own 'steps'")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--cpu-frames", type=int, default=8)
@@ -924,7 +951,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the projection+fusion and object-regime stage timings")
     ap.add_argument("--no-numa", action="store_true", help="diagnostics: do not bind the rank to its GPU's NUMA node")
     ap.add_argument("--no-pipeline", action="store_true", help="diagnostics: stream-ordered EpisodeBatch.step (no cross-frame overlap)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's pooled levels and grid state "
+                    f"as DIR/<name>.npy (float32; arrays over {DUMP_SAMPLE} elements as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "cfg1"):
+        ap.error("--dump-outputs applies to the default workload on the GPU (--impl b200 --workload cfg1)")
     rank, local_rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     if args.impl == "reference":
         return main_reference(args, rank, world)

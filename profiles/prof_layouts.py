@@ -3,7 +3,7 @@ channels-last, bf16 channels-last (a bf16 backbone's output: half the bytes of t
 (EpisodeBatch.step, pipelined) for fp32 CHW vs bf16 HWC.  CUDA events."""
 import importlib, json, math, os, sys
 import numpy as np, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 eod = importlib.import_module("embodied-object-detection_b200")
 ops = eod.ops
 dev = torch.device("cuda:0")

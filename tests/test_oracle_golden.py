@@ -99,7 +99,13 @@ def test_read_restatement_matches_reference(golden):
         for fusion in (("sum", "mem_only", "image_only") if t == 0 else ("sum",)):
             fused = R.project_and_fuse(levels, res, ws, bs, 5, fusion)
             for k in range(3):
-                assert np.array_equal(fused[k].numpy(), g[f"fused_{fusion}_{t}_{k}"])
+                ref = g[f"fused_{fusion}_{t}_{k}"]
+                if fusion == "image_only":
+                    assert np.array_equal(fused[k].numpy(), ref)
+                else:
+                    # the 1x1 conv's fp32 sums round with the CPU's conv kernel (its blocking follows the instruction set and the
+                    # thread count), so hosts differ in the last bits (up to ~3e-7 of scale seen): agreement within 1e-6 of scale
+                    assert np.abs(fused[k].numpy() - ref).max() <= 1e-6 * np.abs(ref).max(), (fusion, t, k)
         # plain-C pooling chain == torch chain, bit for bit
         L = oracle.read_pool_f16(mem16.numpy(), g[f"idx{t}"])
         for k in range(3):
@@ -222,7 +228,8 @@ def test_paste_masks_c_oracle_vs_torch_on_threshold_knife_edges():
 def test_bytecode_listings_pin_the_unsourced_write_variants(tmp_path):
     """SURVEY 8a rows A7' / A7'' / A14 exist only as bytecode.  oracle/pyc_disasm.py (own marshal reader: the 3.12 interpreter cannot
     load 3.9 / 3.10 code objects) produced the listings under oracle/disasm/ that the restatements cite; this test pins the
-    facts the canonical rules rest on, and - where /root/reference is present - that the committed listings regenerate."""
+    facts the canonical rules rest on, and - where EOD_REFERENCE_ROOT names a checkout of the original project - that the committed
+    listings regenerate from its .pyc files."""
     import re
     from oracle import pyc_disasm
     d = os.path.join(ROOT, "oracle", "disasm")
@@ -242,11 +249,37 @@ def test_bytecode_listings_pin_the_unsourced_write_variants(tmp_path):
     assert "(interpolate)" in fpn and "(map_merge_forward_projection)" in fpn or "(map_merge_memory_projection)" in fpn
     exp = open(os.path.join(d, "create_explicit_memory_custom_rcnn_py39.txt")).read()
     assert "(zs_weight)" in exp or "(semmap)" in exp
-    if os.path.isdir("/root/reference/Detic"):
-        made = pyc_disasm.emit("/root/reference", str(tmp_path))
+    ref_root = os.environ.get("EOD_REFERENCE_ROOT")
+    if ref_root:
+        made = pyc_disasm.emit(ref_root, str(tmp_path))
         assert len(made) == 4
         for f in made:
             assert open(os.path.join(tmp_path, f)).read() == open(os.path.join(d, f)).read(), f
+
+
+def test_pyc_disasm_reads_a_minimal_py39_pyc(tmp_path):
+    """oracle/pyc_disasm.py on a hand-built CPython 3.9 .pyc (module whose only constant is `def f(): return None`, line 3): the
+    single-file mode names the file as given, --emit names it relative to the reference root."""
+    import struct
+    from oracle import pyc_disasm
+
+    def i32(v):
+        return struct.pack("<i", v)
+
+    def tup(*items):
+        return b")" + bytes([len(items)]) + b"".join(items)
+
+    def code(name, consts, line):
+        ops = b"\x64\x00\x53\x00"                                                      # LOAD_CONST 0, RETURN_VALUE
+        return (b"c" + i32(0) * 4 + i32(1) + i32(64) + b"s" + i32(len(ops)) + ops + consts + tup() * 4
+                + b"z\x04m.py" + b"z" + bytes([len(name)]) + name.encode() + i32(line) + b"s" + i32(2) + b"\x00\x01")
+
+    pyc = tmp_path / "m.cpython-39.pyc"
+    pyc.write_bytes(struct.pack("<H", 3425) + b"\r\n" + bytes(12) + code("<module>", tup(code("f", tup(b"N"), 3)), 1))
+    text = pyc_disasm.listing(str(pyc), "f")
+    assert text.startswith(f"# {pyc}  ::  f   (CPython 3.9 bytecode, first line 3)\n")
+    assert text.splitlines()[-2:] == ["    4      0 LOAD_CONST                   0  (None)", "           2 RETURN_VALUE                  "]
+    assert pyc_disasm.listing(str(pyc), "f", str(tmp_path)).startswith("# m.cpython-39.pyc  ::  f   ")
 
 
 def test_explicit_map_composition_and_read_match_reference(golden):
