@@ -40,8 +40,8 @@ int eod_num_sms()
 // Work tickets for persistent kernels that claim their tiles dynamically: a pool of zeroed {next, done} int pairs per device.
 // A launch takes the next pair of the pool; the kernel's last CTA re-arms it (both words back to 0), so a pair is reusable as
 // soon as its launch has finished.  1024 pairs per device, handed out round-robin: two launches on DIFFERENT streams could only meet on
-// one pair if one stream ran more than a thousand ticketed launches behind the other (launches of one stream are ordered anyway).  The pool is allocated at the first call on a device (do not
-// make that first call inside a CUDA graph capture); nullptr = allocation failed (callers fall back to static partitioning).
+// one pair if one stream ran more than a thousand ticketed launches behind the other (launches of one stream are ordered anyway).  The pool is allocated at the first call on a device (never
+// call it inside a CUDA graph capture: captured launches take the static partition); nullptr = allocation failed (callers fall back to static partitioning).
 int *eod_work_tickets()
 {
     constexpr int kPairs = 1024;

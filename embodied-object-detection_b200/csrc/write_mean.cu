@@ -941,10 +941,12 @@ int launch_tma_kernel(const CUtensorMap &tmap, const int32_t *idx, const uint8_t
     const int n_groups = n_tiles / group;
     const int grid = n_groups < eod_num_sms() ? n_groups : eod_num_sms();
     static const int static_env = [] { const char *v = getenv("EOD_TMA_STATIC_TILES"); return v ? atoi(v) : 0; }();   // comparator: pre-assigned groups
-    int *work = static_env ? nullptr : eod_work_tickets();
+    // a captured launch takes the static partition: a ticket pair would be pinned for the graph's lifetime while eager launches keep
+    // rotating through the pool.  The capture is checked BEFORE the pool is touched: its first use allocates and zero-fills it
+    // (cudaMalloc + cudaMemset), which would invalidate the capture, and every draw advances the round-robin counter.
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    if (work && (cudaStreamIsCapturing(st, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone))
-        work = nullptr;      // a captured launch would pin its ticket pair for the graph's lifetime while eager launches keep rotating through the pool
+    const bool capturing = cudaStreamIsCapturing(st, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone;
+    int *work = (static_env || capturing) ? nullptr : eod_work_tickets();
     static const int chunk_env = [] { const char *v = getenv("EOD_TMA_CHUNK"); return v ? atoi(v) : 8; }();        // groups per ticket
     static const int hint_env = [] { const char *v = getenv("EOD_TMA_WAIT_HINT_NS"); return v ? atoi(v) : 0; }();   // suspend-time hint of the barrier waits
     static const int stages_env = [] { const char *v = getenv("EOD_TMA_STAGES"); const int n = v ? atoi(v) : Cfg::kStages; return n >= 2 && n <= Cfg::kStages ? n : Cfg::kStages; }();

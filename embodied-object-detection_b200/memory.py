@@ -43,11 +43,15 @@ class EpisodeBatch:
 
     ``pipeline=False`` (default): fully stream-ordered for the caller - on return the caller's stream has been made
     to wait for everything ``step`` enqueued.
-    ``pipeline=True``: the caller promises that depth / pose / shifts / samp of a step are ready when ``step`` is
-    called and stay untouched until the next ``step`` (or ``join``) - they are consumed ahead of the caller's stream
-    (``step(..., inputs_ready=False)`` drops the promise for one step: the geometry then waits for the caller's stream,
-    the write of the previous frame still overlaps).  The returned levels are ordered on the caller's stream; grid state
-    (``sums``, ``counts``, ``norm16``) must be read after ``join()``.
+    ``pipeline=True``: the caller promises that the geometry inputs of a step - depth / pose / shifts / samp /
+    ``proj_indices``, and in ``step_detections`` also the detection tensors and ``n_obj`` - are ready when the step is
+    called: they are consumed ahead of the caller's stream (``inputs_ready=False`` drops the promise for one step: the
+    geometry then waits for the caller's stream, the write of the previous frame still overlaps).  ``feat`` and every
+    mask of ``step`` (``active``, ``reset_mask``, ``refresh_mask``) are ordered on the caller's stream in either mode; a
+    step that takes ``active`` does not run ahead of it.  The returned levels are ordered on the caller's stream; grid
+    state (``sums``, ``counts``, ``norm16``) must be read after ``join()``.
+
+    In both modes a step's inputs may be overwritten, on the caller's stream, as soon as the NEXT step has returned.
 
     Lock-step batches of RAGGED episodes (the reference iterates sequences of different lengths one after the other,
     custom_rcnn.py:441-443): ``step(..., active=, reset_mask=, refresh_mask=)`` - slots whose episode has ended are
@@ -271,15 +275,18 @@ class EpisodeBatch:
              reset_mask: Optional[torch.Tensor] = None, refresh_mask: Optional[torch.Tensor] = None,
              inputs_ready: bool = True, proj_indices: Optional[torch.Tensor] = None) -> List[torch.Tensor]:
         """One frame of the hot path for all E episodes, in the reference's order: the read of frame t sees
-        the state written by frame t-1 (custom_rcnn.py:489-515).  See the class docstring for the stream layout.
-        active / reset_mask / refresh_mask: (E) i32 device tensors ordered on the caller's stream (ragged lock-step batches):
-        reset_mask clears those slots BEFORE this frame's read (frame['memory_reset'], :470-477), refresh_mask then brings
-        their fp16 read table up to date (read_frozen mode, :482-486), active <= 0 slots are not written.
+        the state written by frame t-1 (custom_rcnn.py:489-515).  See the class docstring for the stream layout and for which
+        inputs ``inputs_ready`` covers.
+        feat and active / reset_mask / refresh_mask ((E) i32 device tensors, ragged lock-step batches) are ordered on the caller's
+        stream: reset_mask clears those slots BEFORE this frame's read (frame['memory_reset'], :470-477), refresh_mask then brings
+        their fp16 read table up to date (read_frozen mode, :482-486), active <= 0 slots are neither counted nor written.
         proj_indices (E,H,W) int32: precomputed, range-checked cell indices (memory_data/*.h5) used instead of depth / pose."""
         s0 = torch.cuda.current_stream(self.device)
         self._k = self._t & 1
         self._t += 1
-        strict = (not self.pipeline) or self._sync_next or not inputs_ready
+        # active is read by the count on the geometry stream AND by the write: both must see the caller's mask, so a step that
+        # takes one runs its geometry behind the caller's stream
+        strict = (not self.pipeline) or self._sync_next or not inputs_ready or active is not None
         self._sync_next = False
         e_in = torch.cuda.Event()
         e_in.record(s0)
@@ -349,8 +356,10 @@ class EpisodeBatch:
         the latency-bound object write instead of in front of it.  With ``pipeline=True`` the caller's stream is not made to wait for
         this frame's finalize, so project / paste / sample of frame t+1 run under write / flush / finalize of frame t (index plane and
         per-frame counts are double buffered); the state chain read(t) -> finalize(t) -> read(t+1) is what remains serial.  The
-        promise about inputs is the one of ``step`` (``inputs_ready=False`` drops it for one call).  Slots whose episode has ended
-        pass n_obj == 0 (nothing is written, :686); reset_mask / refresh_mask as in ``step``."""
+        promise of ``pipeline=True`` covers depth / pose / shifts / proj_indices AND box_features / mask_probs / boxes / n_obj
+        (``inputs_ready=False`` drops it for one call); reset_mask / refresh_mask are ordered on the caller's stream, as in ``step``.
+        A step's inputs may be overwritten once the next step has returned.  Slots whose episode has ended pass n_obj == 0
+        (nothing is written, :686)."""
         s0 = torch.cuda.current_stream(self.device)
         capturing = torch.cuda.is_current_stream_capturing()
         self._k = self._t & 1
@@ -433,7 +442,8 @@ class EpisodeBatch:
         is ~10 small launches on two streams, so one episode is bound by launch overhead, not by the kernels).  The arguments are
         example inputs of the shapes / dtypes every later frame will have; they are copied into static buffers owned by the returned
         object, whose ``__call__(depth, pose, shifts, box_features, mask_probs, boxes, n_obj)`` copies a frame's inputs in and replays
-        the graph.  Results are identical to the eager call (same kernels, same order)."""
+        the graph.  Results are identical to the eager call (same kernels, same order).  Per-frame keywords (reset_mask, refresh_mask,
+        proj_indices) raise ValueError: a graph would apply them at every replay."""
         return GraphedDetections(self, depth, pose, shifts, intr, cell, box_features, mask_probs, boxes, n_obj, kw)
 
 
@@ -443,7 +453,14 @@ class GraphedDetections:
 
     _KEYS = ("depth", "pose", "shifts", "box_features", "mask_probs", "boxes", "n_obj")
 
+    # per-frame inputs that the graph would bake in: the warm-up frame would apply them once and every replay again
+    _PER_FRAME = ("reset_mask", "refresh_mask", "proj_indices")
+
     def __init__(self, batch: "EpisodeBatch", depth, pose, shifts, intr, cell, box_features, mask_probs, boxes, n_obj, kw):
+        bad = [k for k in self._PER_FRAME if k in kw]
+        if bad:
+            raise ValueError(f"capture_step_detections: {', '.join(bad)} cannot be captured (a replay would reuse it every frame); "
+                             f"reset / refresh with an eager step or EpisodeBatch.reset / refresh_read between replays")
         self.batch = batch
         given = dict(zip(self._KEYS, (depth, pose, shifts, box_features, mask_probs, boxes, n_obj)))
         self.static = {k: (None if v is None else v.detach().to(batch.device).clone().contiguous()) for k, v in given.items()}
@@ -485,6 +502,7 @@ class GraphedDetections:
         b._k = self._k
         b._t += 1
         self.graph.replay()
+        b._sync_next = True                                 # the next eager step must not run ahead of this replay (same planes)
         return self.levels
 
 
