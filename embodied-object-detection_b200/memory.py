@@ -30,6 +30,28 @@ from . import ops
 from ._lib import LAYOUT_CHW, LAYOUT_HWC, ORDER_ZX, WRITE_AUTO, WRITE_DET, EodError
 
 
+def _slot_workspace(slots: Optional[ops.ObjectSlots], E: int, n_cells: int, C: int, HW: int, sample_stride: int,
+                    device: torch.device) -> ops.ObjectSlots:
+    """``slots`` if it fits a frame of HW pixels sampled every ``sample_stride``-th, else a new workspace of the object write."""
+    S = -(-HW // sample_stride)
+    if slots is None or slots.S < S or slots.n_cells != n_cells:
+        slots = ops.ObjectSlots(E, n_cells, C, S, device)
+    return slots
+
+
+def _write_objects(idx: torch.Tensor, samp: torch.Tensor, frame_cnt: torch.Tensor, slots: ops.ObjectSlots, sums: torch.Tensor,
+                   box_features: torch.Tensor, n_obj: Optional[torch.Tensor], masks: Optional[torch.Tensor] = None,
+                   mask_probs: Optional[torch.Tensor] = None, boxes: Optional[torch.Tensor] = None, mask_thresh: float = 0.5) -> None:
+    """count -> object write -> flush of one frame into ``sums``, with the objects' ``masks``, or with their un-pasted
+    ``mask_probs`` and ``boxes`` (pasted inside the write).  frame_cnt stays set for the finalize."""
+    ops.frame_count(idx, samp, frame_cnt, n_obj, slots)
+    if masks is not None:
+        ops.write_objects(box_features, masks, n_obj, idx, samp, slots)
+    else:
+        ops.write_objects_pasted(box_features, mask_probs, boxes, n_obj, idx, samp, slots, mask_thresh)
+    ops.flush_slots(frame_cnt, slots, sums)
+
+
 class EpisodeBatch:
     """E episodes in lock step.  ``step`` runs the frame on two internal streams so that independent stages overlap:
 
@@ -117,6 +139,11 @@ class EpisodeBatch:
         if self._pix_inv_n2 is None:
             self._pix_inv_n2 = [torch.zeros((self.E, self.H, self.W), dtype=torch.float32, device=self.device) for _ in range(2)]
         return self._pix_inv_n2[self._k]
+
+    @property
+    def _per_pixel_divisors(self) -> bool:
+        """The write takes its divisors from ``pix_inv_n`` (expand_counts pre-pass): only the TMA-staged CHW kernel does."""
+        return self.variant != WRITE_DET and self.layout == LAYOUT_CHW and self.pixel_divisors
 
     def profile(self, on: bool = True) -> None:
         """Record a CUDA-event pair around every stage launch (on the stream it is launched on, no synchronisation added)."""
@@ -210,7 +237,7 @@ class EpisodeBatch:
 
     def _count(self, samp: Optional[torch.Tensor], active: Optional[torch.Tensor] = None) -> None:
         self._timed("count", ops.frame_count, self.idx, samp, self.frame_cnt, active)
-        if self.variant != WRITE_DET and self.layout == LAYOUT_CHW and self.pixel_divisors:      # only the TMA-staged CHW kernel takes per-pixel divisors
+        if self._per_pixel_divisors:
             self._timed("expand", ops.expand_counts, self.idx, self.frame_cnt, self.pix_inv_n)
 
     def _write(self, feat: torch.Tensor, samp: Optional[torch.Tensor], active: Optional[torch.Tensor] = None) -> None:
@@ -222,7 +249,7 @@ class EpisodeBatch:
             self._timed("write", ops.write_mean_det, feat, self.idx, samp, self.frame_cnt, self.sums, self._det_ws)
             return
         self._timed("write", ops.write_mean, feat, self.idx, samp, self.frame_cnt, self.sums, self.layout, self.variant,
-                    self.pix_inv_n if (self.layout == LAYOUT_CHW and self.pixel_divisors) else None, active)
+                    self.pix_inv_n if self._per_pixel_divisors else None, active)
 
     def _finalize(self) -> None:
         # read_frozen (TEST_TYPE longterm): counts only - the fp16 table the read gathers from is a snapshot
@@ -244,14 +271,10 @@ class EpisodeBatch:
         """Object-feature regime (the reference's live path, custom_rcnn.py:681-743) for one frame of every episode,
         fused: box_features (E,Kmax,C) f32 (= 50*normalize(feat), :848), masks (E,Kmax,H,W) bool, n_obj (E) i32 kept
         detections per episode (None = Kmax).  Episodes with n_obj == 0 are skipped entirely, counts included (:686)."""
-        S = -(-self.H * self.W // sample_stride)
-        if self._slots is None or self._slots.S < S:
-            self._slots = ops.ObjectSlots(self.E, self.n_cells, self.C, S, self.device)
+        self._slots = _slot_workspace(self._slots, self.E, self.n_cells, self.C, self.H * self.W, sample_stride, self.device)
         observed = ops.masks_observed(masks, n_obj)
         samp = ops.sample_mask(observed, sample_stride)
-        ops.frame_count(self.idx, samp, self.frame_cnt, n_obj, self._slots)
-        ops.write_objects(box_features, masks, n_obj, self.idx, samp, self._slots)
-        ops.flush_slots(self.frame_cnt, self._slots, self.sums)
+        _write_objects(self.idx, samp, self.frame_cnt, self._slots, self.sums, box_features, n_obj, masks=masks)
         self._finalize()
 
     def write_detections(self, box_features: torch.Tensor, mask_probs: torch.Tensor, boxes: torch.Tensor,
@@ -260,17 +283,71 @@ class EpisodeBatch:
         mask head's 28x28 probabilities), boxes (E,Kmax,4) f32 XYXY.  paste_masks_in_image is folded into the write: the
         (K,480,640) masks are never built - one pass ORs the pasted test into ``observed``, the write re-evaluates it for
         the sampled pixels only."""
-        S = -(-self.H * self.W // sample_stride)
-        if self._slots is None or self._slots.S < S:
-            self._slots = ops.ObjectSlots(self.E, self.n_cells, self.C, S, self.device)
+        self._slots = _slot_workspace(self._slots, self.E, self.n_cells, self.C, self.H * self.W, sample_stride, self.device)
         _, observed = ops.paste_masks(mask_probs, boxes, (self.H, self.W), mask_thresh, n_obj, want_masks=False, want_observed=True)
         samp = ops.sample_mask(observed, sample_stride)
-        ops.frame_count(self.idx, samp, self.frame_cnt, n_obj, self._slots)
-        ops.write_objects_pasted(box_features, mask_probs, boxes, n_obj, self.idx, samp, self._slots, mask_thresh)
-        ops.flush_slots(self.frame_cnt, self._slots, self.sums)
+        _write_objects(self.idx, samp, self.frame_cnt, self._slots, self.sums, box_features, n_obj,
+                       mask_probs=mask_probs, boxes=boxes, mask_thresh=mask_thresh)
         self._finalize()
 
     # ---- one frame, overlapped -------------------------------------------------------------------------------
+    # The frame protocol that step and step_detections share, one helper per phase; each of the two lays its own stages out on the
+    # streams between them.
+    def _begin_frame(self, inputs_ready: bool, force_strict: bool) -> Tuple[torch.cuda.Stream, bool, torch.cuda.Event]:
+        """Flip the double buffer and mark the caller's stream (``e_in``).  strict: this frame takes its inputs behind ``e_in``
+        (not pipelined, first step after a reset / refresh / replay, ``inputs_ready=False`` or ``force_strict``)."""
+        s0 = torch.cuda.current_stream(self.device)
+        self._k = self._t & 1
+        self._t += 1
+        strict = (not self.pipeline) or self._sync_next or not inputs_ready or force_strict
+        self._sync_next = False
+        return s0, strict, s0.record_event()
+
+    def _reset_refresh(self, e_in: torch.cuda.Event, reset_mask: Optional[torch.Tensor],
+                       refresh_mask: Optional[torch.Tensor]) -> Optional[torch.cuda.Event]:
+        """reset_mask / refresh_mask on the write stream, behind finalize of frame t-1 (same stream) and the caller's masks; the
+        returned event orders this frame's read behind them."""
+        if reset_mask is None and refresh_mask is None:
+            return None
+        with torch.cuda.stream(self._wr):
+            self._wr.wait_event(e_in)
+            if reset_mask is not None:
+                ops.reset_episodes(self.counts, self.sums, self.norm16, reset_mask)
+            if refresh_mask is not None and self.norm16 is not None:
+                ops.refresh_norm16(self.counts, self.sums, self.norm16, refresh_mask)
+            return self._wr.record_event()
+
+    def _read_frame(self, strict: bool, e_in: torch.cuda.Event,
+                    e_state: Optional[torch.cuda.Event]) -> Tuple[List[torch.Tensor], torch.cuda.Event]:
+        """This frame's read on the geometry stream, after the geometry enqueued there: it sees the state finalised by frame t-1
+        and this frame's reset / refresh."""
+        with torch.cuda.stream(self._geo):
+            if not strict:
+                self._geo.wait_event(e_in)                 # the caller has consumed the previous frame's levels
+            if self._e_fin is not None:
+                self._geo.wait_event(self._e_fin)          # norm16 as finalised by frame t-1
+            if e_state is not None:
+                self._geo.wait_event(e_state)
+            levels = self.read()
+            return levels, self._geo.record_event()
+
+    def _end_frame(self, s0: torch.cuda.Stream, e_read: torch.cuda.Event, wait_fin: bool,
+                   inputs: Sequence[torch.Tensor]) -> torch.cuda.Event:
+        """Finalize on the write stream after its stages, then order the levels on the caller's stream and, with ``wait_fin``,
+        the whole frame; without it ``inputs`` stay allocated until the write stream is done with them."""
+        with torch.cuda.stream(self._wr):
+            self._wr.wait_event(e_read)                    # finalize rewrites the norm16 rows the read gathers from
+            self._finalize()
+            e_fin = self._wr.record_event()
+        self._e_read, self._e_fin = e_read, e_fin
+        s0.wait_event(e_read)
+        if wait_fin:
+            s0.wait_event(e_fin)
+        else:
+            for t in inputs:
+                t.record_stream(self._wr)
+        return e_fin
+
     def step(self, depth, pose, shifts, intr, cell, feat, samp=None, order: int = ORDER_ZX, *, active: Optional[torch.Tensor] = None,
              reset_mask: Optional[torch.Tensor] = None, refresh_mask: Optional[torch.Tensor] = None,
              inputs_ready: bool = True, proj_indices: Optional[torch.Tensor] = None) -> List[torch.Tensor]:
@@ -281,25 +358,10 @@ class EpisodeBatch:
         stream: reset_mask clears those slots BEFORE this frame's read (frame['memory_reset'], :470-477), refresh_mask then brings
         their fp16 read table up to date (read_frozen mode, :482-486), active <= 0 slots are neither counted nor written.
         proj_indices (E,H,W) int32: precomputed, range-checked cell indices (memory_data/*.h5) used instead of depth / pose."""
-        s0 = torch.cuda.current_stream(self.device)
-        self._k = self._t & 1
-        self._t += 1
         # active is read by the count on the geometry stream AND by the write: both must see the caller's mask, so a step that
         # takes one runs its geometry behind the caller's stream
-        strict = (not self.pipeline) or self._sync_next or not inputs_ready or active is not None
-        self._sync_next = False
-        e_in = torch.cuda.Event()
-        e_in.record(s0)
-        e_state = None
-        if reset_mask is not None or refresh_mask is not None:
-            with torch.cuda.stream(self._wr):              # behind finalize of frame t-1 (same stream), ahead of this frame's read
-                self._wr.wait_event(e_in)
-                if reset_mask is not None:
-                    ops.reset_episodes(self.counts, self.sums, self.norm16, reset_mask)
-                if refresh_mask is not None and self.norm16 is not None:
-                    ops.refresh_norm16(self.counts, self.sums, self.norm16, refresh_mask)
-                e_state = torch.cuda.Event()
-                e_state.record()
+        s0, strict, e_in = self._begin_frame(inputs_ready, force_strict=active is not None)
+        e_state = self._reset_refresh(e_in, reset_mask, refresh_mask)
         with torch.cuda.stream(self._geo):
             if strict:
                 self._geo.wait_event(e_in)                 # inputs (and a preceding reset) are ordered on the caller's stream
@@ -307,38 +369,19 @@ class EpisodeBatch:
                 # dense frame, geometry computed here: the per-cell pixel counts are taken inside the back-projection launch
                 self._timed("project", ops.backproject_count, depth, pose, shifts, intr, cell, self.map_w, self.map_h, self.idx, self.frame_cnt,
                             active, order)
-                if self.variant != WRITE_DET and self.layout == LAYOUT_CHW and self.pixel_divisors:
+                if self._per_pixel_divisors:
                     self._timed("expand", ops.expand_counts, self.idx, self.frame_cnt, self.pix_inv_n)
             else:
                 self._geometry(depth, pose, shifts, intr, cell, order, proj_indices)
                 self._count(samp, active)
-            e_geo = torch.cuda.Event()
-            e_geo.record()
-            if not strict:
-                self._geo.wait_event(e_in)                 # the caller has consumed the previous frame's levels
-            if self._e_fin is not None:
-                self._geo.wait_event(self._e_fin)          # norm16 as finalised by frame t-1
-            if e_state is not None:
-                self._geo.wait_event(e_state)
-            levels = self.read()
-            e_read = torch.cuda.Event()
-            e_read.record()
+            e_geo = self._geo.record_event()
+        levels, e_read = self._read_frame(strict, e_in, e_state)
         with torch.cuda.stream(self._wr):
-            self._wr.wait_event(e_in)                      # feat is ordered on the caller's stream
+            self._wr.wait_event(e_in)                      # feat is outside the pipeline promise: always ordered on the caller's stream
             self._wr.wait_event(e_geo)
             self._write(feat, samp, active)
-            self._wr.wait_event(e_read)                    # finalize rewrites the norm16 rows the read gathers from
-            self._finalize()
-            e_fin = torch.cuda.Event()
-            e_fin.record()
-        self._e_read, self._e_fin = e_read, e_fin
-        s0.wait_event(e_read)
-        if self.pipeline:
-            feat.record_stream(self._wr)
-        else:
-            s0.wait_event(e_fin)
+        self._end_frame(s0, e_read, wait_fin=not self.pipeline, inputs=(feat,))
         return levels
-
 
     def step_detections(self, depth, pose, shifts, intr, cell, box_features, mask_probs, boxes, n_obj=None, sample_stride: int = 8,
                         mask_thresh: float = 0.5, order: int = ORDER_ZX, *, reset_mask: Optional[torch.Tensor] = None,
@@ -360,30 +403,14 @@ class EpisodeBatch:
         (``inputs_ready=False`` drops it for one call); reset_mask / refresh_mask are ordered on the caller's stream, as in ``step``.
         A step's inputs may be overwritten once the next step has returned.  Slots whose episode has ended pass n_obj == 0
         (nothing is written, :686)."""
-        s0 = torch.cuda.current_stream(self.device)
         capturing = torch.cuda.is_current_stream_capturing()
-        self._k = self._t & 1
-        self._t += 1
-        strict = (not self.pipeline) or self._sync_next or not inputs_ready or capturing
-        self._sync_next = False
         if self._pre is None:
             with torch.cuda.device(self.device):
                 self._pre = torch.cuda.Stream(priority=0)
-        S = -(-self.H * self.W // sample_stride)
-        if self._slots is None or self._slots.S < S:
-            self._slots = ops.ObjectSlots(self.E, self.n_cells, self.C, S, self.device)
-        e_in = torch.cuda.Event()
-        e_in.record(s0)
-        e_state = None
-        if reset_mask is not None or refresh_mask is not None:
-            with torch.cuda.stream(self._wr):              # behind finalize of frame t-1 (same stream), ahead of this frame's read
-                self._wr.wait_event(e_in)
-                if reset_mask is not None:
-                    ops.reset_episodes(self.counts, self.sums, self.norm16, reset_mask)
-                if refresh_mask is not None and self.norm16 is not None:
-                    ops.refresh_norm16(self.counts, self.sums, self.norm16, refresh_mask)
-                e_state = torch.cuda.Event()
-                e_state.record()
+        self._slots = _slot_workspace(self._slots, self.E, self.n_cells, self.C, self.H * self.W, sample_stride, self.device)
+        # a side stream joins a capture only by waiting for the capturing stream
+        s0, strict, e_in = self._begin_frame(inputs_ready, force_strict=capturing)
+        e_state = self._reset_refresh(e_in, reset_mask, refresh_mask)
         with torch.cuda.stream(self._pre):
             if strict:
                 self._pre.wait_event(e_in)
@@ -393,48 +420,29 @@ class EpisodeBatch:
                 self._obs2 = [torch.empty((self.E, self.H * self.W), dtype=torch.uint8, device=self.device) for _ in range(2)]
                 self._samp2 = [torch.empty((self.E, self.H * self.W), dtype=torch.uint8, device=self.device) for _ in range(2)]
                 self._fin2 = [None, None]
-            if self._fin2[self._k] is not None and not capturing:
+            if self._fin2[self._k] is not None and not capturing:      # a capture cannot wait for an event recorded outside it
                 self._pre.wait_event(self._fin2[self._k])      # the write side of frame t-2 has finished with this half
             _, observed = ops.paste_masks(mask_probs, boxes, (self.H, self.W), mask_thresh, n_obj, want_masks=False, want_observed=True,
                                           observed_out=self._obs2[self._k])
             samp = ops.sample_mask(observed, sample_stride, self._samp2[self._k])
-            e_samp = torch.cuda.Event()
-            e_samp.record()
+            e_samp = self._pre.record_event()
         with torch.cuda.stream(self._geo):
             if strict:
                 self._geo.wait_event(e_in)
             self._geometry(depth, pose, shifts, intr, cell, order, proj_indices)
-            e_geo = torch.cuda.Event()
-            e_geo.record()
-            if not strict:
-                self._geo.wait_event(e_in)                 # the caller has consumed the previous frame's levels
-            if self._e_fin is not None:
-                self._geo.wait_event(self._e_fin)          # norm16 as finalised by frame t-1
-            if e_state is not None:
-                self._geo.wait_event(e_state)
-            levels = self.read()
-            e_read = torch.cuda.Event()
-            e_read.record()
+            e_geo = self._geo.record_event()
+        levels, e_read = self._read_frame(strict, e_in, e_state)
         with torch.cuda.stream(self._wr):
             if strict:
-                self._wr.wait_event(e_in)
+                self._wr.wait_event(e_in)                  # the detection inputs are inside the pipeline promise
             self._wr.wait_event(e_geo)
             self._wr.wait_event(e_samp)
-            ops.frame_count(self.idx, samp, self.frame_cnt, n_obj, self._slots)
-            ops.write_objects_pasted(box_features, mask_probs, boxes, n_obj, self.idx, samp, self._slots, mask_thresh)
-            ops.flush_slots(self.frame_cnt, self._slots, self.sums)
-            self._wr.wait_event(e_read)                    # finalize rewrites the norm16 rows the read gathers from
-            self._finalize()
-            e_fin = torch.cuda.Event()
-            e_fin.record()
-        self._e_read, self._e_fin = e_read, e_fin
-        self._fin2[self._k] = None if capturing else e_fin
-        s0.wait_event(e_read)
-        if self.pipeline and not capturing:
-            for t in (box_features, mask_probs, boxes) + ((n_obj,) if n_obj is not None else ()):
-                t.record_stream(self._wr)
-        else:
-            s0.wait_event(e_fin)
+            _write_objects(self.idx, samp, self.frame_cnt, self._slots, self.sums, box_features, n_obj,
+                           mask_probs=mask_probs, boxes=boxes, mask_thresh=mask_thresh)
+        # a capture must join every side stream back into the capturing stream
+        e_fin = self._end_frame(s0, e_read, wait_fin=not self.pipeline or capturing,
+                                inputs=(box_features, mask_probs, boxes) + ((n_obj,) if n_obj is not None else ()))
+        self._fin2[self._k] = None if capturing else e_fin      # an event recorded in a capture cannot be waited for outside it
         return levels
 
     def capture_step_detections(self, depth, pose, shifts, intr, cell, box_features, mask_probs, boxes, n_obj=None, **kw) -> "GraphedDetections":
@@ -583,10 +591,12 @@ class SpatialFeatureMemory:
             return None
         return ops.semmap_decode(self._intensity, self._cls, self.obs_score_thresh)[0]
 
-    def _semmap_update(self) -> None:
+    def _finalize(self, idx: torch.Tensor) -> None:
+        """End of a write into the live state: the explicit map of the cells the frame saw, then their counts (_frame_cnt back to zero)."""
         if self.zs_weight is not None:
             ops.semmap_update(self._frame_cnt, self.observations.unsqueeze(0), self.implicit_memory.unsqueeze(0), self.zs_weight,
                               self.n_semmap_classes, self._intensity, self._cls)
+        ops.finalize_counts(idx, self._frame_cnt, self.observations.unsqueeze(0))
 
     # ---- read ----------------------------------------------------------------------------------------
     def create_implicit_memory(self, frame: Dict) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -611,12 +621,7 @@ class SpatialFeatureMemory:
             raise EodError("create_explicit_memory: no semantic map (pass semmap= or construct the memory with zs_weight)")
         if sm.dtype not in (torch.int32, torch.int64):
             sm = sm.to(torch.int64)
-        idx = torch.as_tensor(frame["proj_indices"]).to(self.device)
-        if idx.dim() == 3 and idx.shape[-1] == 1:
-            idx = idx.squeeze(2)
-        if idx.dtype not in (torch.int32, torch.int64):
-            idx = idx.to(torch.int64)
-        idx = idx.contiguous()
+        idx = self._index_plane(frame["proj_indices"]).contiguous()
         proj = ops.remap_indices(idx, sm.reshape(-1).contiguous(), memory.shape[0], add=1)
         obs = frame.get("observations")
         ego_obs = None if obs is None else torch.as_tensor(obs).to(self.device).reshape(-1)[idx.long()]
@@ -627,9 +632,7 @@ class SpatialFeatureMemory:
         memory, projection, observations = [], [], []
         for x in batched_inputs:
             m = torch.as_tensor(x["memory"]).to(self.device)
-            p = torch.as_tensor(x["proj_indices"]).to(self.device)
-            if p.dim() == 3:
-                p = p.squeeze(2)
+            p = self._index_plane(x["proj_indices"])
             o = x.get("observations")
             if o is not None and not torch.is_tensor(o):
                 o = torch.as_tensor(o).to(self.device).to(torch.half)
@@ -646,12 +649,7 @@ class SpatialFeatureMemory:
         counts = self.observations if memory is None else observations
         if table.dtype == torch.float16:
             counts = None
-        idx = torch.as_tensor(proj_indices).to(self.device)
-        if idx.dim() == 3 and idx.shape[-1] == 1:
-            idx = idx.squeeze(2)
-        if idx.dtype not in (torch.int32, torch.int64):
-            idx = idx.to(torch.int64)
-        idx = idx.unsqueeze(0).contiguous()
+        idx = self._index_plane(proj_indices).unsqueeze(0).contiguous()
         if self.validate_indices:
             ops.check_indices(idx, table.shape[0])
         return ops.read_pool(table.unsqueeze(0).contiguous(), None if counts is None else counts.unsqueeze(0).contiguous(), idx)
@@ -662,18 +660,36 @@ class SpatialFeatureMemory:
         return ops.box_to_image_features(box_features.to(self.device, torch.float32).contiguous(),
                                          masks.to(self.device).contiguous())
 
-    def _idx32(self, proj_indices: torch.Tensor, n_cells: Optional[int] = None) -> torch.Tensor:
-        """(1, HW) int32 view of an externally supplied plane (h5 / npz proj_indices, int32 or int64).  With n_cells the ids are
-        range-checked on the device (IndexError like the reference's gather, one 4-byte read-back); ``validate_indices =
-        False`` on the instance skips that for callers whose planes come from eod_backproject_quantize for this very grid."""
+    def _index_plane(self, proj_indices) -> torch.Tensor:
+        """An externally supplied plane (h5 / npz proj_indices, (H,W) or (H,W,1)) on the device as int32 / int64 (H,W)."""
         p = torch.as_tensor(proj_indices).to(self.device)
         if p.dim() == 3 and p.shape[-1] == 1:
             p = p.squeeze(2)
         if p.dtype not in (torch.int32, torch.int64):
             p = p.to(torch.int64)
+        return p
+
+    def _idx32(self, proj_indices: torch.Tensor, n_cells: Optional[int] = None) -> torch.Tensor:
+        """(1, HW) int32 view of an externally supplied plane (see ``_index_plane``).  With n_cells the ids are
+        range-checked on the device (IndexError like the reference's gather, one 4-byte read-back); ``validate_indices =
+        False`` on the instance skips that for callers whose planes come from eod_backproject_quantize for this very grid."""
+        p = self._index_plane(proj_indices)
         if n_cells is not None and self.validate_indices:
             return ops.check_indices(p.contiguous(), n_cells, want_i32=True).reshape(1, -1)
         return p.to(torch.int32).reshape(1, -1).contiguous()
+
+    def _fresh_mean(self, feat: torch.Tensor, idx: torch.Tensor, samp: Optional[torch.Tensor], n_cells: int, C: int,
+                    layout: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Per-cell mean of one frame into a fresh zero table, the live state untouched: (table (cells,C) f32, observed_mem
+        (cells,) bool = the cells the frame wrote)."""
+        table = torch.zeros((1, n_cells, C), dtype=torch.float32, device=self.device)
+        cnt = torch.zeros((1, n_cells), dtype=torch.int32, device=self.device)
+        touched = torch.zeros((1, n_cells), dtype=torch.uint8, device=self.device)
+        dummy_counts = torch.zeros((1, n_cells), dtype=torch.float32, device=self.device)
+        ops.frame_count(idx, samp, cnt)
+        ops.write_mean(feat, idx, samp, cnt, table, layout)
+        ops.finalize_counts(idx, cnt, dummy_counts, touched)
+        return table[0], touched[0].view(torch.bool)
 
     def project_image_features(self, image_features: torch.Tensor, observed_pixels: torch.Tensor,
                                proj_indices: Sequence[torch.Tensor], memory: Sequence[torch.Tensor]):
@@ -682,16 +698,9 @@ class SpatialFeatureMemory:
         C = image_features.shape[1]
         idx = self._idx32(proj_indices[0], n_cells)
         samp = ops.sample_mask(observed_pixels.to(self.device).reshape(1, -1).view(torch.uint8).contiguous(), self.sample_stride)
-        scratch = torch.zeros((1, n_cells, C), dtype=torch.float32, device=self.device)
-        cnt = torch.zeros((1, n_cells), dtype=torch.int32, device=self.device)
-        touched = torch.zeros((1, n_cells), dtype=torch.uint8, device=self.device)
-        dummy_counts = torch.zeros((1, n_cells), dtype=torch.float32, device=self.device)
         feat = image_features.to(self.device, torch.float32).reshape(1, C, -1).contiguous()
-        ops.frame_count(idx, samp, cnt)
-        ops.write_mean(feat, idx, samp, cnt, scratch, LAYOUT_CHW)
-        ops.finalize_counts(idx, cnt, dummy_counts, touched)
-        observed_mem = touched[0].view(torch.bool)
-        return scratch[0][observed_mem], observed_mem
+        mean, observed_mem = self._fresh_mean(feat, idx, samp, n_cells, C, LAYOUT_CHW)
+        return mean[observed_mem], observed_mem
 
     def update_implicit_memory(self, inference_results, proj_indices: torch.Tensor, memory: torch.Tensor, frame: Dict,
                                visualise: bool = False) -> None:
@@ -735,37 +744,25 @@ class SpatialFeatureMemory:
         bf = box_features.to(self.device, torch.float32).contiguous().unsqueeze(0)
         mp = mask_probs.to(self.device, torch.float32).contiguous().unsqueeze(0)
         bx = boxes.to(self.device, torch.float32).contiguous().unsqueeze(0)
-        HW = self.H * self.W
-        S = -(-HW // self.sample_stride)
-        n_cells = self.implicit_memory.shape[0]
-        if self._slots is None or self._slots.S < S or self._slots.n_cells != n_cells:
-            self._slots = ops.ObjectSlots(1, n_cells, self.C, S, self.device)
+        self._slots = _slot_workspace(self._slots, 1, self.implicit_memory.shape[0], self.C, self.H * self.W, self.sample_stride, self.device)
         _, observed = ops.paste_masks(mp, bx, (self.H, self.W), mask_thresh, want_masks=False, want_observed=True)
         samp = ops.sample_mask(observed, self.sample_stride)
-        ops.frame_count(idx, samp, self._frame_cnt, None, self._slots)
-        ops.write_objects_pasted(bf, mp, bx, None, idx, samp, self._slots, mask_thresh)
-        ops.flush_slots(self._frame_cnt, self._slots, self.implicit_memory.unsqueeze(0))
-        self._semmap_update()
-        ops.finalize_counts(idx, self._frame_cnt, self.observations.unsqueeze(0))
+        _write_objects(idx, samp, self._frame_cnt, self._slots, self.implicit_memory.unsqueeze(0), bf, None,
+                       mask_probs=mp, boxes=bx, mask_thresh=mask_thresh)
+        self._finalize(idx)
 
     def write_object_features(self, box_features: torch.Tensor, masks: torch.Tensor, proj_indices: torch.Tensor) -> None:
         """A6 + A7 + A8 without the (1,C,H,W) image (custom_rcnn.py:690-701,738-743): the per-pixel object mean is
         formed only for the every-``sample_stride``-th observed pixels, on the fly."""
-        idx = self._idx32(proj_indices, self.implicit_memory.shape[0])
+        h, w = masks.shape[-2:]
+        idx = self._idx32(proj_indices, self.implicit_memory.shape[0]).view(1, h, w)
         bf = box_features.to(self.device, torch.float32).contiguous().unsqueeze(0)
         m = masks.to(self.device).contiguous().unsqueeze(0)
-        HW = masks.shape[-2] * masks.shape[-1]
-        S = -(-HW // self.sample_stride)
-        n_cells = self.implicit_memory.shape[0]
-        if self._slots is None or self._slots.S < S or self._slots.n_cells != n_cells:
-            self._slots = ops.ObjectSlots(1, n_cells, self.C, S, self.device)
+        self._slots = _slot_workspace(self._slots, 1, self.implicit_memory.shape[0], self.C, h * w, self.sample_stride, self.device)
         observed = ops.masks_observed(m)
         samp = ops.sample_mask(observed, self.sample_stride)
-        ops.frame_count(idx, samp, self._frame_cnt, None, self._slots)
-        ops.write_objects(bf, m, None, idx.view(1, masks.shape[-2], masks.shape[-1]), samp, self._slots)
-        ops.flush_slots(self._frame_cnt, self._slots, self.implicit_memory.unsqueeze(0))
-        self._semmap_update()
-        ops.finalize_counts(idx, self._frame_cnt, self.observations.unsqueeze(0))
+        _write_objects(idx, samp, self._frame_cnt, self._slots, self.implicit_memory.unsqueeze(0), bf, None, masks=m)
+        self._finalize(idx)
 
     def dense_backbone_write(self, p3: torch.Tensor, proj_indices: torch.Tensor, n_cells: int,
                              weight: Optional[torch.Tensor] = None, bias: Optional[torch.Tensor] = None, step: int = 8):
@@ -773,9 +770,7 @@ class SpatialFeatureMemory:
         bilinear (H,W) align_corners=True -> [::step, ::step] -> optional 1x1 projection (map_merge_forward_projection,
         eod_linear_rows) -> per-cell mean with proj_indices[::step, ::step]; returns (memory (cells,C') f32 with the mean in the
         observed cells and zeros elsewhere - the reference REPLACES the memory - and observed_mem (cells,) bool)."""
-        idx_full = proj_indices.to(self.device)
-        if idx_full.dim() == 3 and idx_full.shape[-1] == 1:
-            idx_full = idx_full.squeeze(2)
+        idx_full = self._index_plane(proj_indices)
         H, W = idx_full.shape
         f = ops.bilinear_lattice(p3.to(self.device, torch.float32).contiguous(), (H, W), step)
         layout = LAYOUT_CHW
@@ -788,14 +783,7 @@ class SpatialFeatureMemory:
         else:
             f = f.reshape(1, C, -1).contiguous()
         idx = self._idx32(idx_full[::step, ::step].contiguous(), n_cells)
-        table = torch.zeros((1, n_cells, C), dtype=torch.float32, device=self.device)
-        cnt = torch.zeros((1, n_cells), dtype=torch.int32, device=self.device)
-        touched = torch.zeros((1, n_cells), dtype=torch.uint8, device=self.device)
-        dummy = torch.zeros((1, n_cells), dtype=torch.float32, device=self.device)
-        ops.frame_count(idx, None, cnt)
-        ops.write_mean(f, idx, None, cnt, table, layout)
-        ops.finalize_counts(idx, cnt, dummy, touched)
-        return table[0], touched[0].view(torch.bool)
+        return self._fresh_mean(f, idx, None, n_cells, C, layout)
 
     def write_image_features(self, image_features: torch.Tensor, observed_pixels: Optional[torch.Tensor],
                              proj_indices: torch.Tensor, layout: int = LAYOUT_CHW) -> None:
@@ -809,5 +797,4 @@ class SpatialFeatureMemory:
         feat = image_features.to(self.device, torch.float32).reshape(1, -1).contiguous()
         ops.frame_count(idx, samp, self._frame_cnt)
         ops.write_mean(feat, idx, samp, self._frame_cnt, self.implicit_memory.unsqueeze(0), layout)
-        self._semmap_update()
-        ops.finalize_counts(idx, self._frame_cnt, self.observations.unsqueeze(0))
+        self._finalize(idx)
