@@ -6,15 +6,16 @@
 //
 // The main pass streams the per-pixel feature tensor exactly once (N*C*4 bytes per frame - the term that
 // bounds the whole path) and is written for HBM bandwidth:
-//   * CHW features (the reference's (1,C,480,640) layout): a persistent CTA per SM, 12 consumer warps + 1 producer
-//     warp.  Unit of work = (32-pixel tile, 128-channel block) = one 16 KB 3-D TMA box (128B-swizzled) plus bulk
-//     copies of the tile's cell ids / sample mask (/ reciprocal divisors in pixel_divisors mode); the producer CLAIMS chunks of
-//     tile groups from a global ticket (eod_work_tickets), the stage a unit lands in belongs to one consumer warp (the
-//     full/empty mbarrier pair of the stage is the only synchronisation; the unit's {tile, channel block} travels in the
-//     stage's aux area).  All pixels of the tile that fall into one cell form a group (MATCH.ANY; runs in the deterministic
-//     variant): lane l sums channels l, l+32, l+64, l+96 over the group's pixels with conflict-free LDS.128, scales by
-//     1/n_cell (looked up in frame_cnt) and the group leaves the SM as four warp-wide red.global.add.f32 (128 contiguous
-//     bytes of the cell row each) - one L2 reduction per (tile, cell, channel) instead of one per pixel.  DESIGN.md 3.1.
+//   * CHW features (the reference's (1,C,480,640) layout): a persistent CTA per SM, 6 consumer warps + 1 producer
+//     warp.  Unit of work = (32-pixel tile, 256-channel block) = one 32 KB 3-D TMA box (128B-swizzled; at C=128 the whole
+//     tile, 16 KB, with 12 consumer warps) plus bulk copies of the tile's cell ids / sample mask (/ reciprocal divisors in
+//     pixel_divisors mode); the producer CLAIMS chunks of tile groups from a global ticket (eod_work_tickets), the stage a
+//     unit lands in belongs to one consumer warp (the full/empty mbarrier pair of the stage is the only synchronisation; the
+//     unit's {tile, channel block} travels in the stage's aux area).  All pixels of the tile that fall into one cell form a
+//     group (MATCH.ANY; runs in the deterministic variant): lane l sums channels l, l+32, ..., l+224 over the group's pixels
+//     with conflict-free LDS.128, scales by 1/n_cell (looked up in frame_cnt) and the group leaves the SM as eight warp-wide
+//     red.global.add.f32 (128 contiguous bytes of the cell row each) - one L2 reduction per (tile, cell, channel) instead of
+//     one per pixel.  DESIGN.md 3.1.
 //   * an LDG-staged variant of the same algorithm (padded smem tile, runs) handles shapes the TMA path does
 //     not (HW % 32 != 0) and is the bring-up comparator (variant = EOD_WRITE_LDG).
 //   * HWC features (fp32 / bf16 / fp16): a warp owns a strip of 32 pixels, lanes own float4 channel groups; the strip's pixels
@@ -512,28 +513,32 @@ __global__ void __launch_bounds__(C) write_mean_chw_ldg_kernel(const float *__re
 // ------------------------------------------------------------------------------------------------------
 // main pass, CHW, TMA-staged persistent kernel
 //
-// One CTA per SM: kStages consumer warps + 1 producer warp.  The unit of work is (32-pixel tile, block of 128
-// channels) = one 16 KB TMA box; unit u of the CTA lands in ring stage u % kStages and is consumed by warp
-// u % kStages, i.e. every consumer warp OWNS one stage: no CTA- or group-level barrier anywhere, the only
-// synchronisation is the full/empty mbarrier pair of the stage.  Per unit the warp
-//   waits full[stage] -> derives the run-head / sample masks from the staged cell ids (ballot) ->
-//   per run (consecutive pixels of one map cell): lane l sums channels l, l+32, l+64, l+96 over the run's
-//   pixels straight from the swizzled tile (4 independent LDS.128 + FADD chains), scales by the staged
-//   1/n_cell and issues 4 x red.global.add.f32 (each a warp-wide 128-byte segment of the cell row) ->
+// One CTA per SM: kStages consumer warps + 1 producer warp.  The unit of work is (32-pixel tile, block of 256
+// channels) = one 32 KB TMA box (C=128: the whole 16 KB tile); unit u of the CTA lands in ring stage u % kStages and
+// is consumed by warp u % kStages, i.e. every consumer warp OWNS one stage: no CTA- or group-level barrier anywhere,
+// the only synchronisation is the full/empty mbarrier pair of the stage.  The ring holds 192 KB whatever the unit
+// (6 x 32 KB, or 12 x 16 KB at C=128).  Per unit the warp
+//   waits full[stage] -> derives the group / sample masks from the staged cell ids (MATCH.ANY, ballot) ->
+//   per group (the tile's pixels of one map cell): lane l sums channels l, l+32, ..., l+32*(kJ-1) over the group's
+//   pixels straight from the swizzled tile (kJ = 8 independent LDS.128 + FADD chains; 4 at C=128), scales by
+//   1/n_cell and issues kJ x red.global.add.f32 (each a warp-wide 128-byte segment of the cell row) ->
 //   __syncwarp, one arrive on empty[stage].
+// A 256-channel unit does the per-tile work (barrier wait, group derivation, divisor look-up, chunk walk) once for
+// what two 128-channel units did twice; the box height is the TMA limit, so C=512 is two units per tile.
 // ------------------------------------------------------------------------------------------------------
 
 template <int C>
 struct TmaCfg {
-    static constexpr int kChanBlk = 128;                                  // channels per unit (TMA box height)
+    static constexpr int kChanBlk = C < 256 ? C : 256;                    // channels per unit (TMA box height; 256 is the box limit)
     static constexpr int kBlocks = C / kChanBlk;                          // units per tile
-    static constexpr int kStages = 12;                                    // ring depth == consumer warps
+    static constexpr int kJ = kChanBlk / 32;                              // channels (accumulator chains) per lane
+    static constexpr int kUnitBytes = kChanBlk * TILE_PX * 4;             // 32 KB (16 KB at C=128), keeps every stage 1 KB aligned (SWIZZLE_128B)
+    static constexpr int kStages = (192 * 1024) / kUnitBytes;             // ring depth == consumer warps: 192 KB in flight per SM
     static constexpr int kThreads = 32 * (kStages + 1);
-    static constexpr int kUnitBytes = kChanBlk * TILE_PX * 4;             // 16 KB, keeps every stage 1 KB aligned (SWIZZLE_128B)
     // aux area per stage: cells (128 B) | samp (32 B) | pad | per-pixel 1/n (128 B) | unit descriptor {tile, channel block} (8 B)
     static constexpr int kAuxCells = 0, kAuxSamp = 128, kAuxPixN = 256, kAuxUnit = 384, kAuxBytes = 512;
     static constexpr int kSmemBytes = kStages * (kUnitBytes + kAuxBytes) + 1024 /*align slack*/ + 256 /*barriers*/;
-    static_assert(C % kChanBlk == 0, "C must be a multiple of 128");
+    static_assert(C % kChanBlk == 0 && kChanBlk % 128 == 0, "C must be 128 or a multiple of 256");
     static_assert(kSmemBytes <= 232448, "exceeds 227 KB of shared memory");
 };
 
@@ -721,7 +726,8 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
     }
 
     if (warp >= n_stages) return;                                  // diagnostics: a shallower ring (EOD_TMA_STAGES)
-    // ===== consumer warp `warp`: owns ring stage `warp`, lane l owns channels l, l+32, l+64, l+96 of the block =====
+    // ===== consumer warp `warp`: owns ring stage `warp`, lane l owns channels l, l+32, ..., l+32*(kJ-1) of the block =====
+    constexpr int kJ = Cfg::kJ;
     const uint32_t tile = base + warp * Cfg::kUnitBytes + lane * (TILE_PX * 4);   // row `lane` of the box
     const uint32_t aux = aux0 + warp * Cfg::kAuxBytes;
     const uint32_t fullb = full0 + 8 * warp, emptyb = empty0 + 8 * warp;
@@ -760,25 +766,38 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
                     m = samps & __shfl_sync(0xffffffffu, grp, p0);
                 }
                 if (m == 0) continue;                                  // no sampled pixel in this run / group
-                float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
+                float acc[kJ];
+#pragma unroll
+                for (int k = 0; k < kJ; ++k) acc[k] = 0.f;
                 const int j1 = (31 - __clz(m)) >> 2;
 #pragma unroll 1
                 for (int j = (__ffs(m) - 1) >> 2; j <= j1; ++j) {
                     const unsigned mj = (m >> (4 * j)) & 15u;
                     if (mj == 0) continue;
                     const uint32_t a = tile + (((uint32_t)j ^ sw) << 4);
-                    const float4 v0 = lds128(a), v1 = lds128(a + 32 * TILE_PX * 4), v2 = lds128(a + 64 * TILE_PX * 4),
-                                 v3 = lds128(a + 96 * TILE_PX * 4);
+                    float4 v[kJ];
+#pragma unroll
+                    for (int k = 0; k < kJ; ++k) v[k] = lds128(a + k * 32 * TILE_PX * 4);
                     if (mj == 15u) {                                   // whole chunk inside the run, all sampled
-                        a0 = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(a0, v0.x), v0.y), v0.z), v0.w);
-                        a1 = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(a1, v1.x), v1.y), v1.z), v1.w);
-                        a2 = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(a2, v2.x), v2.y), v2.z), v2.w);
-                        a3 = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(a3, v3.x), v3.y), v3.z), v3.w);
+#pragma unroll
+                        for (int k = 0; k < kJ; ++k) acc[k] = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(acc[k], v[k].x), v[k].y), v[k].z), v[k].w);
                     } else {                                           // run edge / sparsely sampled chunk (warp-uniform predicates)
-                        if (mj & 1u) { a0 = __fadd_rn(a0, v0.x); a1 = __fadd_rn(a1, v1.x); a2 = __fadd_rn(a2, v2.x); a3 = __fadd_rn(a3, v3.x); }
-                        if (mj & 2u) { a0 = __fadd_rn(a0, v0.y); a1 = __fadd_rn(a1, v1.y); a2 = __fadd_rn(a2, v2.y); a3 = __fadd_rn(a3, v3.y); }
-                        if (mj & 4u) { a0 = __fadd_rn(a0, v0.z); a1 = __fadd_rn(a1, v1.z); a2 = __fadd_rn(a2, v2.z); a3 = __fadd_rn(a3, v3.z); }
-                        if (mj & 8u) { a0 = __fadd_rn(a0, v0.w); a1 = __fadd_rn(a1, v1.w); a2 = __fadd_rn(a2, v2.w); a3 = __fadd_rn(a3, v3.w); }
+                        if (mj & 1u) {
+#pragma unroll
+                            for (int k = 0; k < kJ; ++k) acc[k] = __fadd_rn(acc[k], v[k].x);
+                        }
+                        if (mj & 2u) {
+#pragma unroll
+                            for (int k = 0; k < kJ; ++k) acc[k] = __fadd_rn(acc[k], v[k].y);
+                        }
+                        if (mj & 4u) {
+#pragma unroll
+                            for (int k = 0; k < kJ; ++k) acc[k] = __fadd_rn(acc[k], v[k].z);
+                        }
+                        if (mj & 8u) {
+#pragma unroll
+                            for (int k = 0; k < kJ; ++k) acc[k] = __fadd_rn(acc[k], v[k].w);
+                        }
                     }
                 }
                 const int rc = __shfl_sync(0xffffffffu, cell, p0);
@@ -786,7 +805,8 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
                     const int pos = run_pos++;
                     if (pos < det.cap) {
                         float *d = det.partials + ((size_t)e * det.cap + pos) * C + cb * Cfg::kChanBlk + lane;
-                        d[0] = a0; d[32] = a1; d[64] = a2; d[96] = a3;
+#pragma unroll
+                        for (int k = 0; k < kJ; ++k) d[32 * k] = acc[k];
                         if (cb == 0 && lane == 0) det.run_cell[(size_t)e * det.cap + pos] = rc;
                         continue;
                     }
@@ -796,10 +816,8 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
                 if (!kPixN) inv = __frcp_rn((float)(__ldg(cnt_e + rc) & 0x7fffffffu));
                 float *d = dst + (size_t)rc * C;
                 if (no_red) continue;                                  // diagnostics (EOD_TMA_NO_RED): everything but the reductions
-                red_add_f32(d, __fmul_rn(a0, inv));
-                red_add_f32(d + 32, __fmul_rn(a1, inv));
-                red_add_f32(d + 64, __fmul_rn(a2, inv));
-                red_add_f32(d + 96, __fmul_rn(a3, inv));
+#pragma unroll
+                for (int k = 0; k < kJ; ++k) red_add_f32(d + 32 * k, __fmul_rn(acc[k], inv));
             }
         }
         __syncwarp();                                                  // every lane's tile reads are done: release the stage

@@ -28,7 +28,7 @@ if len(sys.argv) > 1:
     ms = a.elapsed_time(b) / 20
     print(json.dumps({"setting": sys.argv[1], "write_ms": ms, "GBps": E * (H * W * C * 4 + H * W * 4) / ms / 1e6}))
 else:
-    for name, env in (("default", {}), ("no_red", {"EOD_TMA_NO_RED": "1"}), ("stages10", {"EOD_TMA_STAGES": "10"}), ("stages8", {"EOD_TMA_STAGES": "8"}),
+    for name, env in (("default", {}), ("no_red", {"EOD_TMA_NO_RED": "1"}), ("stages5", {"EOD_TMA_STAGES": "5"}), ("stages4", {"EOD_TMA_STAGES": "4"}),
                       ("dry", None), ("default2", {})):
         e = dict(os.environ)
         if env is None:
