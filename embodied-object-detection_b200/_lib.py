@@ -13,7 +13,7 @@ from .build import SO_PATH
 
 EOD_OK = 0
 ORDER_ZX, ORDER_XZ = 0, 1
-LAYOUT_CHW, LAYOUT_HWC, LAYOUT_HWC_BF16, LAYOUT_HWC_F16 = 0, 1, 2, 3
+LAYOUT_CHW, LAYOUT_HWC, LAYOUT_HWC_BF16, LAYOUT_HWC_F16, LAYOUT_CHW_BF16, LAYOUT_CHW_F16 = 0, 1, 2, 3, 4, 5
 FUSE_SUM, FUSE_MEM_ONLY, FUSE_IMAGE_ONLY = 0, 1, 2
 WRITE_AUTO, WRITE_LDG, WRITE_TMA, WRITE_TMA_DRY, WRITE_DET = 0, 1, 2, 3, 4
 

@@ -16,8 +16,11 @@
 //     with conflict-free LDS.128, scales by 1/n_cell (looked up in frame_cnt) and the group leaves the SM as eight warp-wide
 //     red.global.add.f32 (128 contiguous bytes of the cell row each) - one L2 reduction per (tile, cell, channel) instead of
 //     one per pixel.  DESIGN.md 3.1.
+//   * bf16 / fp16 CHW features (EOD_LAYOUT_CHW_BF16 / _F16: a 16-bit backbone's NCHW output) take the same ring with 64-pixel
+//     units - a box row is again 128 bytes, so the unit, the swizzle and the ring are unchanged - and are widened exactly before the
+//     fp32 arithmetic above (DESIGN.md 3.1c).
 //   * an LDG-staged variant of the same algorithm (padded smem tile, runs) handles shapes the TMA path does
-//     not (HW % 32 != 0) and is the bring-up comparator (variant = EOD_WRITE_LDG).
+//     not (HW % 32 != 0; 16-bit: HW % 64 != 0) and is the bring-up comparator (variant = EOD_WRITE_LDG).
 //   * HWC features (fp32 / bf16 / fp16): a warp owns a strip of 32 pixels, lanes own float4 channel groups; the strip's pixels
 //     are grouped by cell the same way, a group's rows are requested in batches before they are added, and the group is
 //     flushed straight from registers (red.global.add.v4.f32).
@@ -30,6 +33,25 @@
 namespace {
 
 constexpr int TILE_PX = 32;
+
+// feature element type: fp32, or bf16 / fp16 widened exactly to fp32 before any arithmetic
+enum { FEAT_F32 = 0, FEAT_BF16 = 1, FEAT_F16 = 2 };
+template <int F> struct FeatElem { using T = uint16_t; };
+template <> struct FeatElem<FEAT_F32> { using T = float; };
+template <int F>
+__device__ __forceinline__ float widen1(typename FeatElem<F>::T x)
+{
+    if constexpr (F == FEAT_F32) return x;
+    else if constexpr (F == FEAT_BF16) return __uint_as_float((uint32_t)x << 16);
+    else return __half2float(__ushort_as_half(x));
+}
+// the two 16-bit elements of a 32-bit word (element 0 in the low half), widened exactly
+template <int F>
+__device__ __forceinline__ float2 widen2(uint32_t w)
+{
+    if constexpr (F == FEAT_BF16) return make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u));
+    else return __half22float2(*reinterpret_cast<const __half2 *>(&w));
+}
 
 // ------------------------------------------------------------------------------------------------------
 // pre-pass / post-pass: one thread per pixel, warp-level run aggregation of the cell id
@@ -474,8 +496,8 @@ __device__ __forceinline__ void tile_masks(const int *s_cells, const uint8_t *s_
 // ------------------------------------------------------------------------------------------------------
 // main pass, CHW, LDG-staged
 // ------------------------------------------------------------------------------------------------------
-template <int C>
-__global__ void __launch_bounds__(C) write_mean_chw_ldg_kernel(const float *__restrict__ feat, const int32_t *__restrict__ idx,
+template <int C, int F = FEAT_F32>
+__global__ void __launch_bounds__(C) write_mean_chw_ldg_kernel(const typename FeatElem<F>::T *__restrict__ feat, const int32_t *__restrict__ idx,
                                                                const uint8_t *__restrict__ samp, const uint32_t *__restrict__ frame_cnt,
                                                                const int32_t *__restrict__ active, int HW, int64_t n_cells, int tiles_per_ep, int n_tiles,
                                                                float *__restrict__ sums)
@@ -491,11 +513,11 @@ __global__ void __launch_bounds__(C) write_mean_chw_ldg_kernel(const float *__re
         const int e = t / tiles_per_ep, p0 = (t - e * tiles_per_ep) * TILE_PX;
         if (active && __ldg(active + e) <= 0) continue;              // CTA-uniform: an idle slot of the batch is not even read
         const int pvalid = min(TILE_PX, HW - p0);
-        const float *feat_e = feat + (size_t)e * C * HW;
-        // coalesced 128 B row segments: warp w loads channels w, w+NW, ...
+        const typename FeatElem<F>::T *feat_e = feat + (size_t)e * C * HW;
+        // coalesced 128 B (16-bit features: 64 B) row segments: warp w loads channels w, w+NW, ...; widened on the way into the tile
 #pragma unroll 4
         for (int c = warp; c < C; c += NW)
-            tile[swz(c, lane)] = lane < pvalid ? __ldg(feat_e + (size_t)c * HW + p0 + lane) : 0.f;
+            tile[swz(c, lane)] = lane < pvalid ? widen1<F>(__ldg(feat_e + (size_t)c * HW + p0 + lane)) : 0.f;
         if (tid < TILE_PX) {
             s_cells[tid] = tid < pvalid ? __ldg(idx + (size_t)e * HW + p0 + tid) : -1;
             s_samp[tid] = (samp && tid < pvalid) ? __ldg(samp + (size_t)e * HW + p0 + tid) : 1;
@@ -525,18 +547,23 @@ __global__ void __launch_bounds__(C) write_mean_chw_ldg_kernel(const float *__re
 //   __syncwarp, one arrive on empty[stage].
 // A 256-channel unit does the per-tile work (barrier wait, group derivation, divisor look-up, chunk walk) once for
 // what two 128-channel units did twice; the box height is the TMA limit, so C=512 is two units per tile.
+// 16-bit features (F = FEAT_BF16 / FEAT_F16): a tile is 64 pixels, so a box row is again 128 bytes and the unit, the swizzle,
+// the ring and the raster-neighbour pairs are those of fp32; lane l holds pixels l and l + 32 of the tile (chw16_unit).
 // ------------------------------------------------------------------------------------------------------
 
-template <int C>
+template <int C, int F = FEAT_F32>
 struct TmaCfg {
+    static constexpr int kTilePx = F == FEAT_F32 ? TILE_PX : 2 * TILE_PX; // pixels per tile: one 128-byte box row
+    static constexpr int kRowBytes = 128;
     static constexpr int kChanBlk = C < 256 ? C : 256;                    // channels per unit (TMA box height; 256 is the box limit)
     static constexpr int kBlocks = C / kChanBlk;                          // units per tile
     static constexpr int kJ = kChanBlk / 32;                              // channels (accumulator chains) per lane
-    static constexpr int kUnitBytes = kChanBlk * TILE_PX * 4;             // 32 KB (16 KB at C=128), keeps every stage 1 KB aligned (SWIZZLE_128B)
+    static constexpr int kUnitBytes = kChanBlk * kRowBytes;               // 32 KB (16 KB at C=128), keeps every stage 1 KB aligned (SWIZZLE_128B)
     static constexpr int kStages = (192 * 1024) / kUnitBytes;             // ring depth == consumer warps: 192 KB in flight per SM
     static constexpr int kThreads = 32 * (kStages + 1);
-    // aux area per stage: cells (128 B) | samp (32 B) | pad | per-pixel 1/n (128 B) | unit descriptor {tile, channel block} (8 B)
-    static constexpr int kAuxCells = 0, kAuxSamp = 128, kAuxPixN = 256, kAuxUnit = 384, kAuxBytes = 512;
+    // aux area per stage: cells (128 B) | samp (32 B) | pad | per-pixel 1/n (128 B) | unit descriptor {tile, channel block} (8 B);
+    // 16-bit features: cells (256 B) | samp (64 B) | pad | unit descriptor (no per-pixel divisors)
+    static constexpr int kAuxCells = 0, kAuxSamp = 4 * kTilePx, kAuxPixN = 256, kAuxUnit = 384, kAuxBytes = 512;
     static constexpr int kSmemBytes = kStages * (kUnitBytes + kAuxBytes) + 1024 /*align slack*/ + 256 /*barriers*/;
     static_assert(C % kChanBlk == 0 && kChanBlk % 128 == 0, "C must be 128 or a multiple of 256");
     static_assert(kSmemBytes <= 232448, "exceeds 227 KB of shared memory");
@@ -614,6 +641,89 @@ __device__ __forceinline__ uint32_t lds8(uint32_t addr)
     return v;
 }
 
+// One staged unit of 16-bit features: 64 pixels x kChanBlk channels, row `lane` of the box at `tile`.  Lane l looks at pixels l and
+// l + 32.  Groups are formed per half (MATCH.ANY) and joined across the halves with one ballot per group of the lower half; the
+// upper-half groups no lower-half group claimed are cells the lower half does not see.  Per group, lane l sums channels l, l+32, ...
+// over the group's sampled pixels in raster order, 8 pixels (one LDS.128) per chunk, widened exactly, then scales by 1/n_cell and
+// issues kJ red.global.add.f32 - the arithmetic of the fp32 consumer on the widened values.
+template <int C, int F>
+__device__ __forceinline__ void chw16_unit(uint32_t tile, uint32_t aux, int t, int cb, int tiles_per_ep, bool has_samp, unsigned lane,
+                                           int64_t n_cells, const uint32_t *__restrict__ frame_cnt, float *__restrict__ sums, int no_red)
+{
+    using Cfg = TmaCfg<C, F>;
+    constexpr int kJ = Cfg::kJ;
+    const uint32_t sw = lane & 7;
+    const int e = t / tiles_per_ep;
+    const int cell_lo = (int)lds32(aux + Cfg::kAuxCells + 4 * lane), cell_hi = (int)lds32(aux + Cfg::kAuxCells + 128 + 4 * lane);
+    const unsigned grp_lo = __match_any_sync(0xffffffffu, cell_lo), grp_hi = __match_any_sync(0xffffffffu, cell_hi);
+    unsigned lead_lo = __ballot_sync(0xffffffffu, (unsigned)(__ffs(grp_lo) - 1) == lane);
+    unsigned lead_hi = __ballot_sync(0xffffffffu, (unsigned)(__ffs(grp_hi) - 1) == lane);
+    const unsigned samp_lo = has_samp ? __ballot_sync(0xffffffffu, lds8(aux + Cfg::kAuxSamp + lane) != 0) : 0xffffffffu;
+    const unsigned samp_hi = has_samp ? __ballot_sync(0xffffffffu, lds8(aux + Cfg::kAuxSamp + 32 + lane) != 0) : 0xffffffffu;
+    float *dst = sums + ((size_t)e * n_cells) * C + cb * Cfg::kChanBlk + lane;
+    const uint32_t *cnt_e = frame_cnt + (size_t)e * n_cells;
+
+    while (lead_lo | lead_hi) {                                    // warp-uniform
+        int rc;
+        uint64_t m;                                                // sampled pixels of the group, bit p = pixel p of the tile
+        if (lead_lo) {
+            const int p0 = __ffs(lead_lo) - 1;
+            lead_lo &= lead_lo - 1;
+            rc = __shfl_sync(0xffffffffu, cell_lo, p0);
+            const unsigned hi = __ballot_sync(0xffffffffu, cell_hi == rc);
+            lead_hi &= ~hi;                                        // the upper half of this cell belongs to this group
+            m = ((uint64_t)(samp_hi & hi) << 32) | (samp_lo & __shfl_sync(0xffffffffu, grp_lo, p0));
+        } else {
+            const int p0 = __ffs(lead_hi) - 1;
+            lead_hi &= lead_hi - 1;
+            rc = __shfl_sync(0xffffffffu, cell_hi, p0);
+            m = (uint64_t)(samp_hi & __shfl_sync(0xffffffffu, grp_hi, p0)) << 32;
+        }
+        if (m == 0) continue;                                      // no sampled pixel in this group
+        float acc[kJ];
+#pragma unroll
+        for (int k = 0; k < kJ; ++k) acc[k] = 0.f;
+        const int j1 = (63 - __clzll((long long)m)) >> 3;
+#pragma unroll 1
+        for (int j = (__ffsll((long long)m) - 1) >> 3; j <= j1; ++j) {
+            const unsigned mj = (unsigned)(m >> (8 * j)) & 0xffu;
+            if (mj == 0) continue;
+            const uint32_t a = tile + (((uint32_t)j ^ sw) << 4);
+            float4 v[kJ];
+#pragma unroll
+            for (int k = 0; k < kJ; ++k) v[k] = lds128(a + k * 32 * Cfg::kRowBytes);
+            if (mj == 0xffu) {                                     // whole chunk inside the group, all sampled
+#pragma unroll
+                for (int k = 0; k < kJ; ++k) {
+                    const uint32_t w[4] = {__float_as_uint(v[k].x), __float_as_uint(v[k].y), __float_as_uint(v[k].z), __float_as_uint(v[k].w)};
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        const float2 f = widen2<F>(w[q]);
+                        acc[k] = __fadd_rn(__fadd_rn(acc[k], f.x), f.y);
+                    }
+                }
+            } else {                                               // group edge / sparsely sampled chunk (warp-uniform predicates)
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    if (mj & (1u << i)) {
+#pragma unroll
+                        for (int k = 0; k < kJ; ++k) {
+                            const float *vk = reinterpret_cast<const float *>(&v[k]);
+                            const float2 f = widen2<F>(__float_as_uint(vk[i >> 1]));
+                            acc[k] = __fadd_rn(acc[k], (i & 1) ? f.y : f.x);
+                        }
+                    }
+                }
+            }
+        }
+        const float inv = __frcp_rn((float)(__ldg(cnt_e + rc) & 0x7fffffffu));
+        float *d = dst + (size_t)rc * C;
+        if (no_red) continue;                                      // diagnostics (EOD_TMA_NO_RED): everything but the reductions
+#pragma unroll
+        for (int k = 0; k < kJ; ++k) red_add_f32(d + 32 * k, __fmul_rn(acc[k], inv));
+    }
+}
+
 // kDry: consumers only wait and release (no accumulation, no atomics) - measures the pure streaming
 // ceiling of this tile shape; selected with variant EOD_WRITE_TMA_DRY (bring-up / profiling only).
 // kPixN: the per-pixel reciprocal divisors 1/n_cell arrive with the tile (pix_n workspace); otherwise the
@@ -629,14 +739,17 @@ struct DetArgs {
     int cap;                     // runs per episode the workspace holds
 };
 
-template <int C, bool kDry, bool kPixN, bool kDet>
-__global__ void __launch_bounds__(TmaCfg<C>::kThreads, 1)
+// F: feature element type (FEAT_BF16 / FEAT_F16 take the 64-pixel unit and chw16_unit; neither kPixN nor kDet)
+template <int C, bool kDry, bool kPixN, bool kDet, int F = FEAT_F32>
+__global__ void __launch_bounds__(TmaCfg<C, F>::kThreads, 1)
 write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_t *__restrict__ idx, const uint8_t *__restrict__ samp,
                           const uint32_t *__restrict__ frame_cnt, const float *__restrict__ pix_n, const int32_t *__restrict__ active, int HW,
                           int64_t n_cells, int tiles_per_ep, int n_tiles, int group, float *__restrict__ sums, const DetArgs det,
                           int *__restrict__ work, int chunk, uint32_t wait_hint, int n_stages, int no_red)
 {
-    using Cfg = TmaCfg<C>;
+    using Cfg = TmaCfg<C, F>;
+    static_assert(F == FEAT_F32 || (!kPixN && !kDet), "16-bit features: no per-pixel divisors, no deterministic variant");
+    constexpr int kTilePx = Cfg::kTilePx;
     extern __shared__ unsigned char smem_dyn[];
     const uint32_t base = (smem_u32(smem_dyn) + 1023u) & ~1023u;          // shared-window address of stage 0
     const uint32_t aux0 = base + Cfg::kStages * Cfg::kUnitBytes;
@@ -672,7 +785,7 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
         // ===== producer warp: one elected lane issues all copies =====
         if (lane == 0) {
             const uint64_t pol = make_evict_first_policy();     // the feature stream is read exactly once
-            const uint32_t tx = Cfg::kUnitBytes + TILE_PX * 4 + (has_samp ? TILE_PX : 0) + (kPixN ? TILE_PX * 4 : 0);
+            const uint32_t tx = Cfg::kUnitBytes + kTilePx * 4 + (has_samp ? kTilePx : 0) + (kPixN ? kTilePx * 4 : 0);
             int stage = 0;
             uint32_t phase = 0;
             // a ticket = `chunk` consecutive groups; the next ticket is drawn one chunk ahead (the round trip of an atomic under a
@@ -685,7 +798,7 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
               for (int q = c * chunk; q < q_end; ++q) {
                 for (int k = 0; k < units_per_group; ++k) {
                     const int cb = k / group, t = group * q + (k - cb * group);
-                    const int e = t / tiles_per_ep, p0 = (t - e * tiles_per_ep) * TILE_PX;
+                    const int e = t / tiles_per_ep, p0 = (t - e * tiles_per_ep) * kTilePx;
                     const uint32_t fullb = full0 + 8 * stage, aux = aux0 + stage * Cfg::kAuxBytes;
                     mbar_wait_hint(empty0 + 8 * stage, phase ^ 1, wait_hint);
                     const bool idle = active && __ldg(active + e) <= 0;
@@ -696,9 +809,9 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
                     } else {
                         asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(fullb), "r"(tx) : "memory");
                         tma_load_3d_hint(base + stage * Cfg::kUnitBytes, &tmap, p0, cb * Cfg::kChanBlk, e, fullb, pol);
-                        bulk_load_1d_s(aux + Cfg::kAuxCells, idx + (size_t)e * HW + p0, TILE_PX * 4, fullb);
-                        if (has_samp) bulk_load_1d_s(aux + Cfg::kAuxSamp, samp + (size_t)e * HW + p0, TILE_PX, fullb);
-                        if (kPixN) bulk_load_1d_s(aux + Cfg::kAuxPixN, pix_n + (size_t)e * HW + p0, TILE_PX * 4, fullb);
+                        bulk_load_1d_s(aux + Cfg::kAuxCells, idx + (size_t)e * HW + p0, kTilePx * 4, fullb);
+                        if (has_samp) bulk_load_1d_s(aux + Cfg::kAuxSamp, samp + (size_t)e * HW + p0, kTilePx, fullb);
+                        if (kPixN) bulk_load_1d_s(aux + Cfg::kAuxPixN, pix_n + (size_t)e * HW + p0, kTilePx * 4, fullb);
                     }
                     if (++stage == n_stages) { stage = 0; phase ^= 1; }
                 }
@@ -728,7 +841,7 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
     if (warp >= n_stages) return;                                  // diagnostics: a shallower ring (EOD_TMA_STAGES)
     // ===== consumer warp `warp`: owns ring stage `warp`, lane l owns channels l, l+32, ..., l+32*(kJ-1) of the block =====
     constexpr int kJ = Cfg::kJ;
-    const uint32_t tile = base + warp * Cfg::kUnitBytes + lane * (TILE_PX * 4);   // row `lane` of the box
+    const uint32_t tile = base + warp * Cfg::kUnitBytes + lane * Cfg::kRowBytes;  // row `lane` of the box
     const uint32_t aux = aux0 + warp * Cfg::kAuxBytes;
     const uint32_t fullb = full0 + 8 * warp, emptyb = empty0 + 8 * warp;
     const uint32_t sw = lane & 7;                                                  // rows l + 32k share the swizzle phase
@@ -740,7 +853,9 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
         const int cb = (int)(cbw & 0xffu);
         const bool idle = (cbw & 0x100u) != 0;
         int run_pos = kDet ? __ldg(det.tile_off + t) : 0;
-        if (!kDry && !idle) {
+        if constexpr (F != FEAT_F32) {
+            if (!kDry && !idle) chw16_unit<C, F>(tile, aux, t, cb, tiles_per_ep, has_samp, lane, n_cells, frame_cnt, sums, no_red);
+        } else if (!kDry && !idle) {
             const int e = t / tiles_per_ep;
             // run structure of the tile: lane p looks at pixel p
             const int cell = (int)lds32(aux + Cfg::kAuxCells + 4 * lane);
@@ -829,7 +944,6 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
 // main pass, HWC: warp per strip of 32 pixels, lanes own float4 channel groups
 // ------------------------------------------------------------------------------------------------------
 // four consecutive channels of one pixel as fp32: fp32 features (16 B), or bf16 / fp16 features (8 B) widened exactly
-enum { FEAT_F32 = 0, FEAT_BF16 = 1, FEAT_F16 = 2 };
 template <int F> struct FeatRaw { uint2 q; };
 template <> struct FeatRaw<FEAT_F32> { float4 q; };
 template <int F>
@@ -945,14 +1059,14 @@ PFN_encodeTiled get_encode_fn()
     return fn;
 }
 
-template <int C, bool kDry, bool kPixN, bool kDet = false>
+template <int C, bool kDry, bool kPixN, bool kDet = false, int F = FEAT_F32>
 int launch_tma_kernel(const CUtensorMap &tmap, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const float *pix_n,
                       const int32_t *active, int E, int HW, int64_t n_cells, float *sums, cudaStream_t st, const DetArgs det = DetArgs{})
 {
-    using Cfg = TmaCfg<C>;
+    using Cfg = TmaCfg<C, F>;
     static unsigned long long attr_done = 0ull;
-    if (int rc_attr = eod_ensure_dyn_smem(write_mean_chw_tma_kernel<C, kDry, kPixN, kDet>, Cfg::kSmemBytes, &attr_done, "eod_write_mean[tma]")) return rc_attr;
-    const int tiles_per_ep = HW / TILE_PX, n_tiles = tiles_per_ep * E;
+    if (int rc_attr = eod_ensure_dyn_smem(write_mean_chw_tma_kernel<C, kDry, kPixN, kDet, F>, Cfg::kSmemBytes, &attr_done, "eod_write_mean[tma]")) return rc_attr;
+    const int tiles_per_ep = HW / Cfg::kTilePx, n_tiles = tiles_per_ep * E;
     static const int group_env = [] { const char *v = getenv("EOD_TMA_TILE_GROUP"); return v ? atoi(v) : 2; }();   // tuning knob: 1 | 2 | 4 | 8
     int group = (group_env == 1 || group_env == 2 || group_env == 4 || group_env == 8) ? group_env : 2;
     while (group > 1 && n_tiles % group) group >>= 1;
@@ -970,23 +1084,26 @@ int launch_tma_kernel(const CUtensorMap &tmap, const int32_t *idx, const uint8_t
     static const int stages_env = [] { const char *v = getenv("EOD_TMA_STAGES"); const int n = v ? atoi(v) : Cfg::kStages; return n >= 2 && n <= Cfg::kStages ? n : Cfg::kStages; }();
     static const int nored_env = [] { const char *v = getenv("EOD_TMA_NO_RED"); return v ? atoi(v) : 0; }();   // profiling only: wrong results
     const int chunk = work ? (chunk_env > 0 ? chunk_env : 8) : 1;
-    write_mean_chw_tma_kernel<C, kDry, kPixN, kDet><<<grid, Cfg::kThreads, Cfg::kSmemBytes, st>>>(tmap, idx, samp, frame_cnt, pix_n, active, HW, n_cells, tiles_per_ep, n_tiles, group, sums, det, work, chunk, (uint32_t)hint_env, stages_env, nored_env);
+    write_mean_chw_tma_kernel<C, kDry, kPixN, kDet, F><<<grid, Cfg::kThreads, Cfg::kSmemBytes, st>>>(tmap, idx, samp, frame_cnt, pix_n, active, HW, n_cells, tiles_per_ep, n_tiles, group, sums, det, work, chunk, (uint32_t)hint_env, stages_env, nored_env);
     return eod_check_launch("eod_write_mean[tma]");
 }
 
-template <int C>
-int make_feature_tmap(const float *feat, int E, int HW, CUtensorMap *tmap)
+template <int C, int F = FEAT_F32>
+int make_feature_tmap(const void *feat, int E, int HW, CUtensorMap *tmap)
 {
-    using Cfg = TmaCfg<C>;
+    using Cfg = TmaCfg<C, F>;
     PFN_encodeTiled enc = get_encode_fn();
     EOD_REQUIRE(enc, EOD_ERR_LAUNCH, "eod_write_mean: cuTensorMapEncodeTiled entry point unavailable");
+    constexpr cuuint64_t esz = F == FEAT_F32 ? 4 : 2;
+    constexpr CUtensorMapDataType dtype = F == FEAT_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
+                                          : (F == FEAT_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16);
     const cuuint64_t gdim[3] = {(cuuint64_t)HW, (cuuint64_t)C, (cuuint64_t)E};
-    const cuuint64_t gstr[2] = {(cuuint64_t)HW * 4, (cuuint64_t)HW * C * 4};
-    const cuuint32_t box[3] = {TILE_PX, (cuuint32_t)Cfg::kChanBlk, 1};
+    const cuuint64_t gstr[2] = {(cuuint64_t)HW * esz, (cuuint64_t)HW * C * esz};
+    const cuuint32_t box[3] = {(cuuint32_t)Cfg::kTilePx, (cuuint32_t)Cfg::kChanBlk, 1};
     static const int promo_env = [] { const char *v = getenv("EOD_TMA_L2_PROMOTION"); return v ? atoi(v) : 256; }();   // tuning knob: 0 | 128 | 256
     const CUtensorMapL2promotion promo = promo_env == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE
                                          : (promo_env == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
-    const CUresult r = eod_encode_tmap_cached(enc, tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, feat, gdim, gstr, box, promo);
+    const CUresult r = eod_encode_tmap_cached(enc, tmap, dtype, 3, feat, gdim, gstr, box, promo);
     EOD_REQUIRE(r == CUDA_SUCCESS, EOD_ERR_LAUNCH, "eod_write_mean: cuTensorMapEncodeTiled failed (%d)", (int)r);
     return EOD_OK;
 }
@@ -1000,6 +1117,17 @@ int launch_tma(const float *feat, const int32_t *idx, const uint8_t *samp, const
     if (rc) return rc;
     if (pix_n) return launch_tma_kernel<C, kDry, true>(tmap, idx, samp, frame_cnt, pix_n, active, E, HW, n_cells, sums, st);
     return launch_tma_kernel<C, kDry, false>(tmap, idx, samp, frame_cnt, nullptr, active, E, HW, n_cells, sums, st);
+}
+
+// 16-bit CHW features (the host has refused pix_n for them)
+template <int C, int F, bool kDry>
+int launch_tma16(const void *feat, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const int32_t *active, int E, int HW,
+                 int64_t n_cells, float *sums, cudaStream_t st)
+{
+    CUtensorMap tmap;
+    const int rc = make_feature_tmap<C, F>(feat, E, HW, &tmap);
+    if (rc) return rc;
+    return launch_tma_kernel<C, kDry, false, false, F>(tmap, idx, samp, frame_cnt, nullptr, active, E, HW, n_cells, sums, st);
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -1482,17 +1610,18 @@ int launch_det(const float *feat, const int32_t *idx, const uint8_t *samp, const
     return eod_check_launch("eod_write_mean_det[reduce]");
 }
 
-template <int C>
-int launch_ldg(const float *feat, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const int32_t *active, int E, int HW,
+template <int C, int F = FEAT_F32>
+int launch_ldg(const void *feat, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const int32_t *active, int E, int HW,
                int64_t n_cells, float *sums, cudaStream_t st)
 {
     const int smem = C * TILE_PX * 4 + TILE_PX * 4 + TILE_PX;
     static unsigned long long attr_done = 0ull;
-    if (int rc_attr = eod_ensure_dyn_smem(write_mean_chw_ldg_kernel<C>, smem, &attr_done, "eod_write_mean[ldg]")) return rc_attr;
+    if (int rc_attr = eod_ensure_dyn_smem(write_mean_chw_ldg_kernel<C, F>, smem, &attr_done, "eod_write_mean[ldg]")) return rc_attr;
     const int tiles_per_ep = (HW + TILE_PX - 1) / TILE_PX, n_tiles = tiles_per_ep * E;
     const int per_sm = (C >= 512) ? 3 : (C == 256 ? 6 : 8);
     const int grid = min(n_tiles, eod_num_sms() * per_sm);
-    write_mean_chw_ldg_kernel<C><<<grid, C, smem, st>>>(feat, idx, samp, frame_cnt, active, HW, n_cells, tiles_per_ep, n_tiles, sums);
+    write_mean_chw_ldg_kernel<C, F><<<grid, C, smem, st>>>(reinterpret_cast<const typename FeatElem<F>::T *>(feat), idx, samp, frame_cnt, active, HW,
+                                                           n_cells, tiles_per_ep, n_tiles, sums);
     return eod_check_launch("eod_write_mean[ldg]");
 }
 
@@ -1508,6 +1637,19 @@ int launch_hwc(const void *feat, int feat_type, const int32_t *idx, const uint8_
     return eod_check_launch("eod_write_mean[hwc]");
 }
 
+// 16-bit CHW features: the TMA ring takes 64-pixel tiles, the LDG kernel any HW with 16-byte aligned rows (checked by the caller)
+template <int C, int F>
+int dispatch_chw16(const void *feat, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const int32_t *active, int E, int HW,
+                   int64_t n_cells, float *sums, int variant, cudaStream_t st)
+{
+    const bool tma_ok = (HW % TmaCfg<C, F>::kTilePx == 0) && (!samp || (reinterpret_cast<uintptr_t>(samp) % 16 == 0));
+    if (variant == EOD_WRITE_TMA || variant == EOD_WRITE_TMA_DRY)
+        EOD_REQUIRE(tma_ok, EOD_ERR_UNSUPPORTED, "eod_write_mean: TMA variant of 16-bit CHW features needs HW %% 64 == 0 and a 16-byte aligned samp");
+    if (variant == EOD_WRITE_TMA_DRY) return launch_tma16<C, F, true>(feat, idx, samp, frame_cnt, active, E, HW, n_cells, sums, st);
+    if (variant == EOD_WRITE_LDG || !tma_ok) return launch_ldg<C, F>(feat, idx, samp, frame_cnt, active, E, HW, n_cells, sums, st);
+    return launch_tma16<C, F, false>(feat, idx, samp, frame_cnt, active, E, HW, n_cells, sums, st);
+}
+
 template <int C>
 int dispatch(const float *feat, int layout, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const float *pix_n,
              const int32_t *active, int E, int HW, int64_t n_cells, float *sums, int variant, cudaStream_t st)
@@ -1515,6 +1657,8 @@ int dispatch(const float *feat, int layout, const int32_t *idx, const uint8_t *s
     if (layout == EOD_LAYOUT_HWC) return launch_hwc<C>(feat, FEAT_F32, idx, samp, frame_cnt, active, E, HW, n_cells, sums, st);
     if (layout == EOD_LAYOUT_HWC_BF16) return launch_hwc<C>(feat, FEAT_BF16, idx, samp, frame_cnt, active, E, HW, n_cells, sums, st);
     if (layout == EOD_LAYOUT_HWC_F16) return launch_hwc<C>(feat, FEAT_F16, idx, samp, frame_cnt, active, E, HW, n_cells, sums, st);
+    if (layout == EOD_LAYOUT_CHW_BF16) return dispatch_chw16<C, FEAT_BF16>(feat, idx, samp, frame_cnt, active, E, HW, n_cells, sums, variant, st);
+    if (layout == EOD_LAYOUT_CHW_F16) return dispatch_chw16<C, FEAT_F16>(feat, idx, samp, frame_cnt, active, E, HW, n_cells, sums, variant, st);
     const bool tma_ok = (HW % TILE_PX == 0) && (!samp || (reinterpret_cast<uintptr_t>(samp) % 16 == 0));
     if (variant == EOD_WRITE_TMA || variant == EOD_WRITE_TMA_DRY) EOD_REQUIRE(tma_ok, EOD_ERR_UNSUPPORTED, "eod_write_mean: TMA variant needs HW %% 32 == 0");
     if (variant == EOD_WRITE_TMA_DRY) return launch_tma<C, true>(feat, idx, samp, frame_cnt, pix_n, active, E, HW, n_cells, sums, st);
@@ -1622,10 +1766,13 @@ extern "C" int eod_write_mean(const void *feat_any, int layout, const int32_t *i
     EOD_REQUIRE(!pix_inv_n || eod_aligned16(pix_inv_n), EOD_ERR_ALIGN, "eod_write_mean: pix_inv_n must be 16-byte aligned");
     EOD_REQUIRE(feat && idx && frame_cnt && sums, EOD_ERR_BADARG, "eod_write_mean: null pointer");
     EOD_REQUIRE(n_episodes > 0 && HW > 0 && n_cells > 0, EOD_ERR_BADARG, "eod_write_mean: bad sizes");
-    EOD_REQUIRE(layout >= EOD_LAYOUT_CHW && layout <= EOD_LAYOUT_HWC_F16, EOD_ERR_BADARG, "eod_write_mean: bad layout");
+    EOD_REQUIRE(layout >= EOD_LAYOUT_CHW && layout <= EOD_LAYOUT_CHW_F16, EOD_ERR_BADARG, "eod_write_mean: bad layout");
     EOD_REQUIRE(variant >= EOD_WRITE_AUTO && variant <= EOD_WRITE_TMA_DRY, EOD_ERR_BADARG, "eod_write_mean: bad variant");
     EOD_REQUIRE(eod_aligned16(feat) && eod_aligned16(sums) && eod_aligned16(idx), EOD_ERR_ALIGN, "eod_write_mean: pointers must be 16-byte aligned");
     EOD_REQUIRE(layout != EOD_LAYOUT_CHW || HW % 4 == 0, EOD_ERR_ALIGN, "eod_write_mean: CHW rows must be 16-byte aligned (HW %% 4 == 0)");
+    const bool chw16 = layout == EOD_LAYOUT_CHW_BF16 || layout == EOD_LAYOUT_CHW_F16;
+    EOD_REQUIRE(!chw16 || HW % 8 == 0, EOD_ERR_ALIGN, "eod_write_mean: 16-bit CHW rows must be 16-byte aligned (HW %% 8 == 0)");
+    EOD_REQUIRE(!chw16 || !pix_inv_n, EOD_ERR_UNSUPPORTED, "eod_write_mean: pix_inv_n is not supported with 16-bit CHW features");
     cudaStream_t st = (cudaStream_t)stream;
     switch (C) {
     case 128: return dispatch<128>(feat, layout, idx, samp, frame_cnt, pix_inv_n, active, n_episodes, HW, n_cells, sums, variant, st);

@@ -87,6 +87,9 @@ class EpisodeBatch:
                  pipeline: bool = False, fp16_table: bool = True):
         if torch.device(device).type != "cuda":
             raise EodError("EpisodeBatch needs a CUDA device (no CPU fallback)")
+        if variant == WRITE_DET and layout in ops.LAYOUT_DTYPE:
+            raise EodError("variant=WRITE_DET takes fp32 CHW features only: there is no deterministic write for 16-bit features "
+                           "(use the default variant, or feed feat.float() with LAYOUT_CHW)")
         self.E, self.map_w, self.map_h, self.C, self.H, self.W = n_episodes, map_w, map_h, channels, height, width
         self.n_cells = map_w * map_h
         self.device, self.layout, self.variant, self.pipeline = torch.device(device), layout, variant, pipeline
@@ -259,8 +262,8 @@ class EpisodeBatch:
             self._timed("finalize", ops.finalize_counts, self.idx, self.frame_cnt, self.counts, None, self.sums, self.norm16)
 
     def write(self, feat: torch.Tensor, samp: Optional[torch.Tensor] = None, active: Optional[torch.Tensor] = None) -> None:
-        """A7 + A8 for one frame of every episode: feat (E,C,H,W) [CHW] or (E,H,W,C) [HWC] fp32, or (E,H,W,C) bf16 / fp16
-        [LAYOUT_HWC_BF16 / LAYOUT_HWC_F16];
+        """A7 + A8 for one frame of every episode: feat (E,C,H,W) [CHW] or (E,H,W,C) [HWC] fp32, (E,H,W,C) bf16 / fp16
+        [LAYOUT_HWC_BF16 / LAYOUT_HWC_F16] or (E,C,H,W) bf16 / fp16 [LAYOUT_CHW_BF16 / LAYOUT_CHW_F16];
         samp (E,H,W) u8 selects the contributing pixels (None = all); active (E) i32: slots with active <= 0 are skipped."""
         self._count(samp, active)
         self._write(feat, samp, active)
@@ -678,6 +681,15 @@ class SpatialFeatureMemory:
             return ops.check_indices(p.contiguous(), n_cells, want_i32=True).reshape(1, -1)
         return p.to(torch.int32).reshape(1, -1).contiguous()
 
+    def _feat_in(self, image_features: torch.Tensor, layout: int, C: int) -> Tuple[torch.Tensor, int]:
+        """Image features on the device, contiguous, and the layout the write takes them in: bf16 / fp16 stay 16-bit (half the bytes
+        of the write's feature stream, same sums), any other dtype - or a 16-bit image whose rows are not 16-byte aligned
+        (H*W % 8 != 0) - is cast to fp32 as before."""
+        x = torch.as_tensor(image_features)
+        if x.dtype not in (torch.bfloat16, torch.float16) or (x.numel() // C) % 8:
+            return x.to(self.device, torch.float32).contiguous(), layout
+        return x.to(self.device).contiguous(), ops.layout_for_dtype(layout, x.dtype)
+
     def _fresh_mean(self, feat: torch.Tensor, idx: torch.Tensor, samp: Optional[torch.Tensor], n_cells: int, C: int,
                     layout: int) -> Tuple[torch.Tensor, torch.Tensor]:
         """Per-cell mean of one frame into a fresh zero table, the live state untouched: (table (cells,C) f32, observed_mem
@@ -693,13 +705,14 @@ class SpatialFeatureMemory:
 
     def project_image_features(self, image_features: torch.Tensor, observed_pixels: torch.Tensor,
                                proj_indices: Sequence[torch.Tensor], memory: Sequence[torch.Tensor]):
-        """custom_rcnn.py:903-936: (mean (M,C) f32 in ascending cell order, observed_mem (cells,) bool)."""
+        """custom_rcnn.py:903-936: (mean (M,C) f32 in ascending cell order, observed_mem (cells,) bool).  bf16 / fp16 images are
+        written as they are (16-bit CHW layout, widened exactly in the kernel: the reference sums ``float()`` of them, :930)."""
         n_cells = memory[0].shape[0]
         C = image_features.shape[1]
         idx = self._idx32(proj_indices[0], n_cells)
         samp = ops.sample_mask(observed_pixels.to(self.device).reshape(1, -1).view(torch.uint8).contiguous(), self.sample_stride)
-        feat = image_features.to(self.device, torch.float32).reshape(1, C, -1).contiguous()
-        mean, observed_mem = self._fresh_mean(feat, idx, samp, n_cells, C, LAYOUT_CHW)
+        feat, layout = self._feat_in(image_features, LAYOUT_CHW, C)
+        mean, observed_mem = self._fresh_mean(feat.reshape(1, C, -1), idx, samp, n_cells, C, layout)
         return mean[observed_mem], observed_mem
 
     def update_implicit_memory(self, inference_results, proj_indices: torch.Tensor, memory: torch.Tensor, frame: Dict,
@@ -788,13 +801,14 @@ class SpatialFeatureMemory:
     def write_image_features(self, image_features: torch.Tensor, observed_pixels: Optional[torch.Tensor],
                              proj_indices: torch.Tensor, layout: int = LAYOUT_CHW) -> None:
         """A7 + A8 on the live state: per-cell mean of every ``sample_stride``-th observed pixel, sums +=,
-        counts += 1 for all visible cells."""
+        counts += 1 for all visible cells.  bf16 / fp16 features are written as they are (the 16-bit variant of ``layout``)."""
         idx = self._idx32(proj_indices, self.implicit_memory.shape[0])
         samp = None
         if observed_pixels is not None:
             samp = ops.sample_mask(observed_pixels.to(self.device).reshape(1, -1).view(torch.uint8).contiguous(), self.sample_stride)
         C = self.C
-        feat = image_features.to(self.device, torch.float32).reshape(1, -1).contiguous()
+        feat, layout = self._feat_in(image_features, layout, C)
+        feat = feat.reshape(1, -1)
         ops.frame_count(idx, samp, self._frame_cnt)
         ops.write_mean(feat, idx, samp, self._frame_cnt, self.implicit_memory.unsqueeze(0), layout)
         self._finalize(idx)

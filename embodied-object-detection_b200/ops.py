@@ -9,8 +9,19 @@ from typing import Optional, Sequence, Tuple
 import torch
 
 from . import _lib
-from ._lib import (FUSE_IMAGE_ONLY, FUSE_MEM_ONLY, FUSE_SUM, LAYOUT_CHW, LAYOUT_HWC, LAYOUT_HWC_BF16, LAYOUT_HWC_F16, ORDER_XZ, ORDER_ZX, WRITE_AUTO,
-                   WRITE_DET, WRITE_LDG, WRITE_TMA, EodError, check)
+from ._lib import (FUSE_IMAGE_ONLY, FUSE_MEM_ONLY, FUSE_SUM, LAYOUT_CHW, LAYOUT_CHW_BF16, LAYOUT_CHW_F16, LAYOUT_HWC, LAYOUT_HWC_BF16, LAYOUT_HWC_F16,
+                   ORDER_XZ, ORDER_ZX, WRITE_AUTO, WRITE_DET, WRITE_LDG, WRITE_TMA, EodError, check)
+
+# feature dtype of each layout of the mean write (every layout not listed takes fp32)
+LAYOUT_DTYPE = {LAYOUT_HWC_BF16: torch.bfloat16, LAYOUT_HWC_F16: torch.float16, LAYOUT_CHW_BF16: torch.bfloat16, LAYOUT_CHW_F16: torch.float16}
+# the layout that takes features of a given dtype in the same memory order as an fp32 layout
+_LAYOUT_16 = {(LAYOUT_CHW, torch.bfloat16): LAYOUT_CHW_BF16, (LAYOUT_CHW, torch.float16): LAYOUT_CHW_F16,
+              (LAYOUT_HWC, torch.bfloat16): LAYOUT_HWC_BF16, (LAYOUT_HWC, torch.float16): LAYOUT_HWC_F16}
+
+
+def layout_for_dtype(layout: int, dtype: torch.dtype) -> int:
+    """The 16-bit variant of an fp32 layout for bf16 / fp16 features; ``layout`` itself for any other dtype."""
+    return _LAYOUT_16.get((int(layout), dtype), int(layout))
 
 # kernels launched through this module since import (bench.py reports it as gpu_launches)
 launch_count = 0
@@ -175,10 +186,11 @@ def expand_counts(idx: torch.Tensor, frame_cnt: torch.Tensor, pix_inv_n: torch.T
 def write_mean(feat: torch.Tensor, idx: torch.Tensor, samp: Optional[torch.Tensor], frame_cnt: torch.Tensor,
                sums: torch.Tensor, layout: int = LAYOUT_CHW, variant: int = WRITE_AUTO,
                pix_inv_n: Optional[torch.Tensor] = None, active: Optional[torch.Tensor] = None) -> None:
-    """feat (E,C,HW) [CHW] or (E,HW,C) [HWC] f32, or (E,HW,C) bf16 / fp16 [LAYOUT_HWC_BF16 / _F16]; sums (E,cells,C) f32
-    accumulated in place.  pix_inv_n: output of expand_counts for this frame (optional, faster).
+    """feat (E,C,HW) [CHW] or (E,HW,C) [HWC] f32, (E,HW,C) bf16 / fp16 [LAYOUT_HWC_BF16 / _F16] or (E,C,HW) bf16 / fp16
+    [LAYOUT_CHW_BF16 / _F16: widened exactly, fp32 arithmetic; HW % 8 == 0, no pix_inv_n]; sums (E,cells,C) f32 accumulated in
+    place.  pix_inv_n: output of expand_counts for this frame (fp32 CHW only).
     active (E) i32 | None: slots with active <= 0 are skipped (give frame_count the same mask)."""
-    feat_dtype = {LAYOUT_HWC_BF16: torch.bfloat16, LAYOUT_HWC_F16: torch.float16}.get(int(layout), torch.float32)
+    feat_dtype = LAYOUT_DTYPE.get(int(layout), torch.float32)
     _dev(feat, feat_dtype, "feat"), _dev(idx, torch.int32, "idx"), _dev(sums, torch.float32, "sums")
     _dev(frame_cnt, torch.int32, "frame_cnt")
     E, n_cells, C = sums.shape

@@ -145,11 +145,14 @@ class HostEpisodeProvider:
         geometry : ``proj_indices`` (H,W[,1]) int32  (memory_data/*.h5)   or   ``depth`` (H,W) f32 + ``pose`` (12,) f32
         write    : ``feat`` (C,H,W) f32 [dense]   or   ``box_features`` (K,C), ``mask_probs`` (K,S,S), ``boxes`` (K,4) [detections]
     ``shifts``: per episode (6,) f32 (world_shift_origin xyz, map_world_shift xyz), needed with depth.
+    ``feat_dtype``: the dtype ``feat`` is staged in - torch.bfloat16 / torch.float16 feed the 16-bit layouts of ``EpisodeRunner``
+    (LAYOUT_CHW_BF16 / _F16 for (C,H,W) frames, LAYOUT_HWC_BF16 / _F16 for (H,W,C) ones) at half the bytes; a frame's ``feat`` may
+    be a numpy array or a CPU tensor of any dtype.
     Frames are staged through pinned buffers and copied to the device on the caller's stream."""
 
     def __init__(self, episodes: Sequence[Sequence[dict]], device: torch.device, shifts: Optional[Sequence[np.ndarray]] = None,
-                 k_max: int = 16):
-        self.episodes, self.device, self.k_max = episodes, torch.device(device), int(k_max)
+                 k_max: int = 16, feat_dtype: torch.dtype = torch.float32):
+        self.episodes, self.device, self.k_max, self.feat_dtype = episodes, torch.device(device), int(k_max), feat_dtype
         self.shifts = None if shifts is None else [np.asarray(s, np.float32) for s in shifts]
         self._st = _Staging(self.device)
 
@@ -174,7 +177,7 @@ class HostEpisodeProvider:
         def put(key, s, value, shape, dtype):
             if key not in host:
                 host[key], out[key] = self._st.buf(key, (R,) + tuple(shape), dtype)
-            host[key][s] = torch.as_tensor(np.asarray(value)).reshape(shape).to(dtype)
+            host[key][s] = (value if torch.is_tensor(value) else torch.as_tensor(np.asarray(value))).reshape(shape).to(dtype)
 
         for s, a in enumerate(assign):
             if a is None:
@@ -189,7 +192,8 @@ class HostEpisodeProvider:
                 put("pose", s, fr["pose"], (12,), torch.float32)
                 put("shifts", s, self.shifts[a[0]], (6,), torch.float32)
             if "feat" in fr:
-                put("feat", s, fr["feat"], np.asarray(fr["feat"]).shape, torch.float32)
+                f = fr["feat"]
+                put("feat", s, f, tuple(f.shape) if torch.is_tensor(f) else np.asarray(f).shape, self.feat_dtype)
             elif "box_features" in fr:
                 bf, mp, bx = np.asarray(fr["box_features"], np.float32), np.asarray(fr["mask_probs"], np.float32), np.asarray(fr["boxes"], np.float32)
                 K = bf.shape[0]
@@ -314,12 +318,14 @@ class PooledSyntheticProvider:
     """Synthetic dense-regime episodes for workloads too large to hold as depth maps (BASELINE configs[4]: 512 episodes x 100
     frames = 63 GB of fp32 depth): ``pool`` distinct trajectories are ray-cast once on the device (episodes.DeviceEpisodes) and
     episode e replays trajectory e % pool into ITS OWN grid; every episode starts with memory_reset (independent episodes,
-    TEST_TYPE episodic).  Features: two resident random (R,C,H,W) slabs used alternately (>> L2), as in bench.py.  Input
-    generation only - nothing here is on the measured path except one gather of the step's depth / pose rows."""
+    TEST_TYPE episodic).  Features: two resident random (R,C,H,W) slabs used alternately (>> L2), as in bench.py, drawn in fp32 and
+    held as ``feat_dtype`` (torch.bfloat16 / torch.float16 feed LAYOUT_CHW_BF16 / _F16).  Input generation only - nothing here is on
+    the measured path except one gather of the step's depth / pose rows."""
     trusted_indices = True
 
     def __init__(self, n_episodes: int, n_frames: int, channels: int, n_slots: int, device, height: int = 480, width: int = 640,
-                 map_w: int = 1000, map_h: int = 1000, cell: float = 0.2, pool: int = 64, seed0: int = 1234, lengths=None):
+                 map_w: int = 1000, map_h: int = 1000, cell: float = 0.2, pool: int = 64, seed0: int = 1234, lengths=None,
+                 feat_dtype: torch.dtype = torch.float32):
         from . import episodes as E_
         from .geometry import transform3d
         self.device = torch.device(device)
@@ -335,7 +341,7 @@ class PooledSyntheticProvider:
         self.pose = T[:, :, :3, :].reshape(self.pool, n_frames, 12).contiguous().to(self.device)
         self.shifts = torch.from_numpy(np.concatenate([np.zeros_like(dev_eps.shift), dev_eps.shift], 1)).to(self.device)
         gen = torch.Generator(device=self.device).manual_seed(seed0)
-        self.feat = [torch.randn((n_slots, channels, height, width), device=self.device, generator=gen) for _ in range(2)]
+        self.feat = [torch.randn((n_slots, channels, height, width), device=self.device, generator=gen).to(feat_dtype) for _ in range(2)]
         self._st = _Staging(self.device)
         self._keep: List[dict] = []
         self._k = 0

@@ -43,6 +43,8 @@ extern "C" {
 #define EOD_LAYOUT_HWC 1 /* features (E, H*W, C): channels-last                                         */
 #define EOD_LAYOUT_HWC_BF16 2 /* channels-last bf16 features (a bf16 backbone's output): widened exactly, summed in fp32 */
 #define EOD_LAYOUT_HWC_F16 3  /* channels-last fp16 features                                                             */
+#define EOD_LAYOUT_CHW_BF16 4 /* (E, C, H*W) bf16 features (what a bf16 / autocast backbone emits in NCHW): widened exactly  */
+#define EOD_LAYOUT_CHW_F16 5  /* (E, C, H*W) fp16 features                                                                 */
 
 #define EOD_FUSE_SUM 0        /* res + w*mem   timm.py:181-182 */
 #define EOD_FUSE_MEM_ONLY 1   /* w*mem         timm.py:183-184 */
@@ -129,8 +131,11 @@ int eod_expand_counts(const int32_t *idx, const uint32_t *frame_cnt, int n_episo
  * of custom_rcnn.py:917-934 accumulated as in :696-697,742.  Warp-aggregated fp32 reductions
  * (red.global.add.f32, one per run of equal cell id and channel): run-to-run results agree to ~1e-7 of
  * scale, not bitwise.  pix_inv_n: nullable, output of eod_expand_counts for this frame.
- * feat is fp32 for EOD_LAYOUT_CHW / _HWC and bf16 / fp16 for EOD_LAYOUT_HWC_BF16 / _HWC_F16 (half the bytes of the dominant
- * stream: the 16-bit values are widened exactly and everything downstream is the fp32 arithmetic of the fp32 layouts).
+ * feat is fp32 for EOD_LAYOUT_CHW / _HWC and bf16 / fp16 for EOD_LAYOUT_HWC_BF16 / _HWC_F16 / _CHW_BF16 / _CHW_F16 (half the
+ * bytes of the dominant stream: the 16-bit values are widened exactly and everything downstream is the fp32 arithmetic of the fp32
+ * layouts).  16-bit CHW rows must be 16-byte aligned (HW % 8 == 0, else EOD_ERR_ALIGN); their TMA kernel takes 64-pixel tiles
+ * (HW % 64 == 0 and a 16-byte aligned samp, else the LDG kernel - or EOD_ERR_UNSUPPORTED for EOD_WRITE_TMA / _TMA_DRY);
+ * pix_inv_n with a 16-bit CHW layout is EOD_ERR_UNSUPPORTED.  eod_write_mean_det takes fp32 CHW features only.
  * active (E) i32 nullable: the same mask eod_frame_count takes - slots of the lock-step batch with active[e] <= 0 (an episode
  * that has ended, custom_rcnn.py:441-443 iterates ragged sequences) are skipped without reading their features. */
 int eod_write_mean(const void *feat, int layout, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt,
