@@ -36,6 +36,7 @@ SIGNATURES = {
     "eod_write_mean_det_workspace_bytes": [c_int, c_int, c_int, c_int64, c_int],
     "eod_write_mean_det_status_offset": [c_int, c_int64],
     "eod_write_mean_det": [_P, _P, _P, _P, c_int, c_int, c_int, c_int64, _P, _P, c_int64, _P],
+    "eod_write_mean_det_layout": [_P, c_int, _P, _P, _P, _P, c_int, c_int, c_int, c_int64, _P, _P, c_int64, _P],
     "eod_finalize_counts": [_P, c_int, c_int, c_int64, _P, _P, _P, _P, _P, c_int, _P],
     "eod_box_to_image_features": [_P, _P, c_int, c_int, c_int, _P, _P, _P],
     "eod_masks_observed": [_P, _P, c_int, c_int, c_int, _P, _P],

@@ -24,6 +24,8 @@
 //   * HWC features (fp32 / bf16 / fp16): a warp owns a strip of 32 pixels, lanes own float4 channel groups; the strip's pixels
 //     are grouped by cell the same way, a group's rows are requested in batches before they are added, and the group is
 //     flushed straight from registers (red.global.add.v4.f32).
+//   * deterministic variant (eod_write_mean_det_layout): fp32 CHW through the TMA ring, fp32 / bf16 / fp16 channels-last through the
+//     HWC kernel; both store raster-ordered run sums that the same segmented reduce adds in a fixed order.
 #include <cuda.h>
 #include <stdlib.h>
 
@@ -966,11 +968,14 @@ __device__ __forceinline__ float4 widen_feat(const FeatRaw<F> &r)
     }
 }
 
-template <int C, int F>
+// kDet: deterministic variant (HW % 32 == 0: a strip is one tile of the det pre-passes) - the strip's RUNS of equal cell id in raster
+// order (det_tile_masks) take the place of the groups, and a run's unscaled sums are stored to partials[tile_off[strip] + r] like the
+// CHW kDet consumer does: every layout sums a run's sampled pixels in raster order from +0.f, so the partials are the same fp32 values.
+template <int C, int F, bool kDet = false>
 __global__ void __launch_bounds__(256, 3) write_mean_hwc_kernel(const void *__restrict__ feat, const int32_t *__restrict__ idx,
                                                              const uint8_t *__restrict__ samp, const uint32_t *__restrict__ frame_cnt,
                                                              const int32_t *__restrict__ active, int HW, int64_t n_cells, int strips_per_ep,
-                                                             int n_strips, float *__restrict__ sums)
+                                                             int n_strips, float *__restrict__ sums, const DetArgs det)
 {
     constexpr int V = C / 128;                 // float4 per lane per pixel
     const unsigned lane = threadIdx.x & 31;
@@ -990,13 +995,26 @@ __global__ void __launch_bounds__(256, 3) write_mean_hwc_kernel(const void *__re
         // served in the order of their first pixel; a group's pixels are walked in raster order, in batches of PB whose rows are all
         // requested before the first one is added (32 registers of raw data per lane: 4 fp32 pixels or 8 sixteen-bit ones at C=256 -
         // the same bytes in flight whatever the feature type).
-        const unsigned grp = __match_any_sync(0xffffffffu, my_cell);
-        unsigned leaders = __ballot_sync(0xffffffffu, (int)lane < pvalid && (unsigned)(__ffs(grp) - 1) == lane);
+        unsigned grp = 0u, leaders;
+        if constexpr (kDet) {
+            const int prev = __shfl_up_sync(0xffffffffu, my_cell, 1);
+            leaders = __ballot_sync(0xffffffffu, lane == 0 || prev != my_cell);   // run heads (pvalid == 32)
+        } else {
+            grp = __match_any_sync(0xffffffffu, my_cell);
+            leaders = __ballot_sync(0xffffffffu, (int)lane < pvalid && (unsigned)(__ffs(grp) - 1) == lane);
+        }
+        int run_pos = kDet ? __ldg(det.tile_off + s) : 0;
         constexpr int PB = (F == FEAT_F32 ? 8 : 16) / V > 0 ? (F == FEAT_F32 ? 8 : 16) / V : 1;
         while (leaders) {
             const int lead = __ffs(leaders) - 1;
             leaders &= leaders - 1;
-            unsigned rem = __shfl_sync(0xffffffffu, grp, lead) & samps;          // sampled pixels of this cell
+            unsigned rem;
+            if constexpr (kDet) {
+                const int p1 = leaders ? (__ffs(leaders) - 1) : TILE_PX;
+                rem = samps & (0xffffffffu >> (32 - p1)) & (0xffffffffu << lead);   // sampled pixels of this run
+            } else {
+                rem = __shfl_sync(0xffffffffu, grp, lead) & samps;                 // sampled pixels of this cell
+            }
             if (rem == 0u) continue;
             const int cell = __shfl_sync(0xffffffffu, my_cell, lead);
             float4 acc[V];
@@ -1030,6 +1048,17 @@ __global__ void __launch_bounds__(256, 3) write_mean_hwc_kernel(const void *__re
                         }
                     }
                 }
+            }
+            if constexpr (kDet) {
+                const int pos = run_pos++;
+                if (pos < det.cap) {
+                    float *d = det.partials + ((size_t)e * det.cap + pos) * C + 4 * lane;
+#pragma unroll
+                    for (int v = 0; v < V; ++v) *reinterpret_cast<float4 *>(d + v * 128) = acc[v];
+                    if (lane == 0) det.run_cell[(size_t)e * det.cap + pos] = cell;
+                    continue;
+                }
+                if (lane == 0) *det.status = 1;                                  // workspace too small: correct, but not reproducible
             }
             const float n = (float)(__ldg(cnt_e + cell) & 0x7fffffffu);
 #pragma unroll
@@ -1163,8 +1192,9 @@ __device__ __forceinline__ bool det_run_sampled(unsigned heads, unsigned samps, 
     return m != 0;
 }
 
-__global__ void __launch_bounds__(256) det_tile_runs_kernel(const int32_t *__restrict__ idx, const uint8_t *__restrict__ samp, int HW,
-                                                            int tiles_per_ep, int32_t *__restrict__ tile_off, int32_t *__restrict__ n_list,
+__global__ void __launch_bounds__(256) det_tile_runs_kernel(const int32_t *__restrict__ idx, const uint8_t *__restrict__ samp,
+                                                            const int32_t *__restrict__ active, int HW, int tiles_per_ep,
+                                                            int32_t *__restrict__ tile_off, int32_t *__restrict__ n_list,
                                                             int32_t *__restrict__ chunk_rows, int32_t *__restrict__ n_long)
 {
     const int e = blockIdx.y, tile = blockIdx.x * 8 + (threadIdx.x >> 5);
@@ -1175,6 +1205,10 @@ __global__ void __launch_bounds__(256) det_tile_runs_kernel(const int32_t *__res
         n_long[e] = 0;
     }
     if (tile >= tiles_per_ep) return;
+    if (active && __ldg(active + e) <= 0) {                        // idle slot: no runs, its planes are not read
+        if (lane == 0) tile_off[(size_t)e * tiles_per_ep + tile] = 0;
+        return;
+    }
     int cell;
     unsigned heads, samps;
     det_tile_masks(idx, samp, (size_t)e * HW + (size_t)tile * 32, lane, cell, heads, samps);
@@ -1228,14 +1262,14 @@ __global__ void __launch_bounds__(1024) det_scan_tiles_kernel(int32_t *__restric
     det_block_exclusive_scan(tile_off + (size_t)e * tiles_per_ep, tile_off + (size_t)e * tiles_per_ep, tiles_per_ep, n_runs + e);
 }
 
-__global__ void __launch_bounds__(256) det_cell_runs_kernel(const int32_t *__restrict__ idx, const uint8_t *__restrict__ samp, int HW,
-                                                            int tiles_per_ep, int64_t n_cells, const int32_t *__restrict__ tile_off, int cap,
-                                                            int32_t *__restrict__ cell_runs, int32_t *__restrict__ cell_list,
-                                                            int32_t *__restrict__ n_list)
+__global__ void __launch_bounds__(256) det_cell_runs_kernel(const int32_t *__restrict__ idx, const uint8_t *__restrict__ samp,
+                                                            const int32_t *__restrict__ active, int HW, int tiles_per_ep, int64_t n_cells,
+                                                            const int32_t *__restrict__ tile_off, int cap, int32_t *__restrict__ cell_runs,
+                                                            int32_t *__restrict__ cell_list, int32_t *__restrict__ n_list)
 {
     const int e = blockIdx.y, tile = blockIdx.x * 8 + (threadIdx.x >> 5);
     const unsigned lane = threadIdx.x & 31;
-    if (tile >= tiles_per_ep) return;
+    if (tile >= tiles_per_ep || (active && __ldg(active + e) <= 0)) return;     // an idle slot's cell list stays empty
     int cell;
     unsigned heads, samps;
     det_tile_masks(idx, samp, (size_t)e * HW + (size_t)tile * 32, lane, cell, heads, samps);
@@ -1564,9 +1598,15 @@ size_t det_carve(void *ws, int E, int C, int tiles_per_ep, int64_t n_cells, int 
     return o;
 }
 
+template <int C, bool kDet = false>
+int launch_hwc(const void *feat, int feat_type, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const int32_t *active, int E,
+               int HW, int64_t n_cells, float *sums, cudaStream_t st, const DetArgs det = DetArgs{});
+
+// layout: EOD_LAYOUT_CHW (TMA kDet consumer) or a channels-last layout (write_mean_hwc_kernel kDet); the pre-passes and the reduce do
+// not depend on it.  active: idle slots get no runs and their features are not read.
 template <int C>
-int launch_det(const float *feat, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, int E, int HW, int64_t n_cells,
-               float *sums, void *ws, size_t ws_bytes, cudaStream_t st)
+int launch_det(const void *feat, int layout, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const int32_t *active, int E,
+               int HW, int64_t n_cells, float *sums, void *ws, size_t ws_bytes, cudaStream_t st)
 {
     EOD_REQUIRE(HW % TILE_PX == 0 && (!samp || (reinterpret_cast<uintptr_t>(samp) % 16 == 0)), EOD_ERR_UNSUPPORTED,
                 "eod_write_mean_det: needs HW %% 32 == 0 and a 16-byte aligned sample mask");
@@ -1583,16 +1623,20 @@ int launch_det(const float *feat, const int32_t *idx, const uint8_t *samp, const
     DetWorkspace w;
     while (det_carve(ws, E, C, tiles_per_ep, n_cells, (int)cap, &w) > ws_bytes) --cap;
     CUtensorMap tmap;
-    int rc = make_feature_tmap<C>(feat, E, HW, &tmap);
+    int rc = layout == EOD_LAYOUT_CHW ? make_feature_tmap<C>(feat, E, HW, &tmap) : EOD_OK;
     if (rc) return rc;
     dim3 gt((tiles_per_ep + 7) / 8, E);
-    det_tile_runs_kernel<<<gt, 256, 0, st>>>(idx, samp, HW, tiles_per_ep, w.tile_off, w.n_list, w.L.chunk_rows, w.L.n_long);
+    det_tile_runs_kernel<<<gt, 256, 0, st>>>(idx, samp, active, HW, tiles_per_ep, w.tile_off, w.n_list, w.L.chunk_rows, w.L.n_long);
     det_scan_tiles_kernel<<<E, 1024, 0, st>>>(w.tile_off, tiles_per_ep, w.n_runs);
-    det_cell_runs_kernel<<<gt, 256, 0, st>>>(idx, samp, HW, tiles_per_ep, n_cells, w.tile_off, w.cap, w.cell_runs, w.cell_list, w.n_list);
+    det_cell_runs_kernel<<<gt, 256, 0, st>>>(idx, samp, active, HW, tiles_per_ep, n_cells, w.tile_off, w.cap, w.cell_runs, w.cell_list, w.n_list);
     det_scan_list_kernel<<<E, 1024, 0, st>>>(w.cell_runs, w.cell_list, w.n_list, w.cap, n_cells, w.list_off, w.cell_off);
     if ((rc = eod_check_launch("eod_write_mean_det[prepass]"))) return rc;
     DetArgs det{w.tile_off, w.partials, w.run_cell, w.status, w.cap};
-    rc = launch_tma_kernel<C, false, false, true>(tmap, idx, samp, frame_cnt, nullptr, nullptr, E, HW, n_cells, sums, st, det);
+    if (layout == EOD_LAYOUT_CHW)
+        rc = launch_tma_kernel<C, false, false, true>(tmap, idx, samp, frame_cnt, nullptr, active, E, HW, n_cells, sums, st, det);
+    else
+        rc = launch_hwc<C, true>(feat, layout == EOD_LAYOUT_HWC_BF16 ? FEAT_BF16 : (layout == EOD_LAYOUT_HWC_F16 ? FEAT_F16 : FEAT_F32), idx, samp,
+                                 frame_cnt, active, E, HW, n_cells, sums, st, det);
     if (rc) return rc;
     dim3 gc((w.cap + 255) / 256, E);
     det_claim_kernel<<<gc, 256, 0, st>>>(w.run_cell, w.n_runs, w.cap, n_cells, w.cell_off, w.cell_runs, w.seg);
@@ -1625,16 +1669,16 @@ int launch_ldg(const void *feat, const int32_t *idx, const uint8_t *samp, const 
     return eod_check_launch("eod_write_mean[ldg]");
 }
 
-template <int C>
+template <int C, bool kDet>
 int launch_hwc(const void *feat, int feat_type, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const int32_t *active, int E,
-               int HW, int64_t n_cells, float *sums, cudaStream_t st)
+               int HW, int64_t n_cells, float *sums, cudaStream_t st, const DetArgs det)
 {
     const int strips_per_ep = (HW + TILE_PX - 1) / TILE_PX, n_strips = strips_per_ep * E;
     const int blocks = min((n_strips + 7) / 8, eod_num_sms() * 8);
-    if (feat_type == FEAT_BF16) write_mean_hwc_kernel<C, FEAT_BF16><<<blocks, 256, 0, st>>>(feat, idx, samp, frame_cnt, active, HW, n_cells, strips_per_ep, n_strips, sums);
-    else if (feat_type == FEAT_F16) write_mean_hwc_kernel<C, FEAT_F16><<<blocks, 256, 0, st>>>(feat, idx, samp, frame_cnt, active, HW, n_cells, strips_per_ep, n_strips, sums);
-    else write_mean_hwc_kernel<C, FEAT_F32><<<blocks, 256, 0, st>>>(feat, idx, samp, frame_cnt, active, HW, n_cells, strips_per_ep, n_strips, sums);
-    return eod_check_launch("eod_write_mean[hwc]");
+    if (feat_type == FEAT_BF16) write_mean_hwc_kernel<C, FEAT_BF16, kDet><<<blocks, 256, 0, st>>>(feat, idx, samp, frame_cnt, active, HW, n_cells, strips_per_ep, n_strips, sums, det);
+    else if (feat_type == FEAT_F16) write_mean_hwc_kernel<C, FEAT_F16, kDet><<<blocks, 256, 0, st>>>(feat, idx, samp, frame_cnt, active, HW, n_cells, strips_per_ep, n_strips, sums, det);
+    else write_mean_hwc_kernel<C, FEAT_F32, kDet><<<blocks, 256, 0, st>>>(feat, idx, samp, frame_cnt, active, HW, n_cells, strips_per_ep, n_strips, sums, det);
+    return eod_check_launch(kDet ? "eod_write_mean_det[hwc]" : "eod_write_mean[hwc]");
 }
 
 // 16-bit CHW features: the TMA ring takes 64-pixel tiles, the LDG kernel any HW with 16-byte aligned rows (checked by the caller)
@@ -1726,21 +1770,31 @@ extern "C" int64_t eod_write_mean_det_status_offset(int n_episodes, int64_t n_ce
     return (int64_t)det_align((size_t)n_episodes * n_cells * 4);
 }
 
-extern "C" int eod_write_mean_det(const float *feat, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, int n_episodes, int C,
-                                  int HW, int64_t n_cells, float *sums, void *workspace, int64_t workspace_bytes, eod_stream_t stream)
+extern "C" int eod_write_mean_det_layout(const void *feat, int layout, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt,
+                                         const int32_t *active, int n_episodes, int C, int HW, int64_t n_cells, float *sums, void *workspace,
+                                         int64_t workspace_bytes, eod_stream_t stream)
 {
     EOD_REQUIRE(feat && idx && frame_cnt && sums, EOD_ERR_BADARG, "eod_write_mean_det: null pointer");
     EOD_REQUIRE(n_episodes > 0 && n_episodes <= 65535 && HW > 0 && n_cells > 0 && workspace_bytes > 0, EOD_ERR_BADARG, "eod_write_mean_det: bad sizes");
+    EOD_REQUIRE(layout >= EOD_LAYOUT_CHW && layout <= EOD_LAYOUT_CHW_F16, EOD_ERR_BADARG, "eod_write_mean_det: bad layout");
+    EOD_REQUIRE(layout != EOD_LAYOUT_CHW_BF16 && layout != EOD_LAYOUT_CHW_F16, EOD_ERR_UNSUPPORTED,
+                "eod_write_mean_det: no deterministic write for 16-bit CHW features (use EOD_LAYOUT_CHW with fp32 features)");
     EOD_REQUIRE(eod_aligned16(feat) && eod_aligned16(idx) && eod_aligned16(sums), EOD_ERR_ALIGN, "eod_write_mean_det: pointers must be 16-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
     switch (C) {
-    case 128: return launch_det<128>(feat, idx, samp, frame_cnt, n_episodes, HW, n_cells, sums, workspace, (size_t)workspace_bytes, st);
-    case 256: return launch_det<256>(feat, idx, samp, frame_cnt, n_episodes, HW, n_cells, sums, workspace, (size_t)workspace_bytes, st);
-    case 512: return launch_det<512>(feat, idx, samp, frame_cnt, n_episodes, HW, n_cells, sums, workspace, (size_t)workspace_bytes, st);
+    case 128: return launch_det<128>(feat, layout, idx, samp, frame_cnt, active, n_episodes, HW, n_cells, sums, workspace, (size_t)workspace_bytes, st);
+    case 256: return launch_det<256>(feat, layout, idx, samp, frame_cnt, active, n_episodes, HW, n_cells, sums, workspace, (size_t)workspace_bytes, st);
+    case 512: return launch_det<512>(feat, layout, idx, samp, frame_cnt, active, n_episodes, HW, n_cells, sums, workspace, (size_t)workspace_bytes, st);
     default:
         eod_set_error("eod_write_mean_det: C=%d not compiled in (128, 256, 512)", C);
         return EOD_ERR_UNSUPPORTED;
     }
+}
+
+extern "C" int eod_write_mean_det(const float *feat, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, int n_episodes, int C,
+                                  int HW, int64_t n_cells, float *sums, void *workspace, int64_t workspace_bytes, eod_stream_t stream)
+{
+    return eod_write_mean_det_layout(feat, EOD_LAYOUT_CHW, idx, samp, frame_cnt, nullptr, n_episodes, C, HW, n_cells, sums, workspace, workspace_bytes, stream);
 }
 
 extern "C" int eod_expand_counts(const int32_t *idx, const uint32_t *frame_cnt, int n_episodes, int HW, int64_t n_cells,

@@ -27,7 +27,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import torch
 
 from . import ops
-from ._lib import LAYOUT_CHW, LAYOUT_HWC, ORDER_ZX, WRITE_AUTO, WRITE_DET, EodError
+from ._lib import LAYOUT_CHW, LAYOUT_CHW_BF16, LAYOUT_CHW_F16, LAYOUT_HWC, ORDER_ZX, WRITE_AUTO, WRITE_DET, EodError
 
 
 def _slot_workspace(slots: Optional[ops.ObjectSlots], E: int, n_cells: int, C: int, HW: int, sample_stride: int,
@@ -87,9 +87,9 @@ class EpisodeBatch:
                  pipeline: bool = False, fp16_table: bool = True):
         if torch.device(device).type != "cuda":
             raise EodError("EpisodeBatch needs a CUDA device (no CPU fallback)")
-        if variant == WRITE_DET and layout in ops.LAYOUT_DTYPE:
-            raise EodError("variant=WRITE_DET takes fp32 CHW features only: there is no deterministic write for 16-bit features "
-                           "(use the default variant, or feed feat.float() with LAYOUT_CHW)")
+        if variant == WRITE_DET and layout in (LAYOUT_CHW_BF16, LAYOUT_CHW_F16):
+            raise EodError("variant=WRITE_DET has no deterministic write for 16-bit CHW features (use LAYOUT_HWC_BF16 / _HWC_F16 "
+                           "channels-last features, or feed feat.float() with LAYOUT_CHW)")
         self.E, self.map_w, self.map_h, self.C, self.H, self.W = n_episodes, map_w, map_h, channels, height, width
         self.n_cells = map_w * map_h
         self.device, self.layout, self.variant, self.pipeline = torch.device(device), layout, variant, pipeline
@@ -245,11 +245,9 @@ class EpisodeBatch:
 
     def _write(self, feat: torch.Tensor, samp: Optional[torch.Tensor], active: Optional[torch.Tensor] = None) -> None:
         if self.variant == WRITE_DET:
-            if active is not None:
-                raise EodError("the deterministic write does not take an active mask (advance ragged episodes with the default variant)")
             if self._det_ws is None:
                 self._det_ws = ops.DetWorkspace(self.E, self.C, self.H * self.W, self.n_cells, self.device, self.det_runs_per_episode)
-            self._timed("write", ops.write_mean_det, feat, self.idx, samp, self.frame_cnt, self.sums, self._det_ws)
+            self._timed("write", ops.write_mean_det, feat, self.idx, samp, self.frame_cnt, self.sums, self._det_ws, self.layout, active)
             return
         self._timed("write", ops.write_mean, feat, self.idx, samp, self.frame_cnt, self.sums, self.layout, self.variant,
                     self.pix_inv_n if self._per_pixel_divisors else None, active)

@@ -27,6 +27,7 @@ def layout_for_dtype(layout: int, dtype: torch.dtype) -> int:
 launch_count = 0
 
 _LAUNCHES = {"eod_backproject_quantize": 1, "eod_backproject_quantize_u16": 1, "eod_backproject_count": 1, "eod_quantize_world": 1, "eod_sample_mask": 1, "eod_frame_count": 1, "eod_expand_counts": 1, "eod_write_mean": 1, "eod_write_mean_det": 9,
+             "eod_write_mean_det_layout": 9,
              "eod_finalize_counts": 1, "eod_box_to_image_features": 1, "eod_masks_observed": 1, "eod_paste_masks": 1, "eod_write_objects_pasted": 1, "eod_bilinear_lattice": 1, "eod_write_objects": 1, "eod_flush_slots": 2, "eod_write_max": 2, "eod_read_pool": 2,
              "eod_fuse": 1, "eod_project_split_weights": 1, "eod_project_fuse": 1, "eod_project_fuse_levels": 1, "eod_normalize_memory": 1, "eod_reset_touched": 1, "eod_semmap_update": 1, "eod_semmap_decode": 2,
              "eod_reset_episodes": 1, "eod_refresh_norm16": 1, "eod_check_indices": 1, "eod_remap_indices": 1, "eod_max_winner_list": 1, "eod_linear_rows": 1, "eod_read_roi": 1}
@@ -319,9 +320,11 @@ class DetWorkspace:
 
 
 def write_mean_det(feat: torch.Tensor, idx: torch.Tensor, samp: Optional[torch.Tensor], frame_cnt: torch.Tensor,
-                   sums: torch.Tensor, ws: DetWorkspace) -> None:
-    """Deterministic main pass (CHW features, HW % 32 == 0): same contract as write_mean, bitwise reproducible."""
-    _dev(feat, torch.float32, "feat"), _dev(idx, torch.int32, "idx"), _dev(sums, torch.float32, "sums")
+                   sums: torch.Tensor, ws: DetWorkspace, layout: int = LAYOUT_CHW, active: Optional[torch.Tensor] = None) -> None:
+    """Deterministic main pass (HW % 32 == 0): same contract as write_mean, bitwise reproducible.  layout: LAYOUT_CHW (fp32) or
+    LAYOUT_HWC / _HWC_BF16 / _HWC_F16 - the same features give the same bits in every layout (16-bit ones widened exactly); the
+    16-bit CHW layouts raise EodError.  active (E) i32 | None: slots with active <= 0 are skipped (give frame_count the same mask)."""
+    _dev(feat, LAYOUT_DTYPE.get(int(layout), torch.float32), "feat"), _dev(idx, torch.int32, "idx"), _dev(sums, torch.float32, "sums")
     _dev(frame_cnt, torch.int32, "frame_cnt")
     E, n_cells, C = sums.shape
     HW = idx[0].numel()
@@ -329,8 +332,12 @@ def write_mean_det(feat: torch.Tensor, idx: torch.Tensor, samp: Optional[torch.T
         raise ValueError(f"feat has {feat.numel()} elements, expected E*C*HW = {E * C * HW}")
     if samp is not None:
         _dev(samp, torch.uint8, "samp")
-    _call("eod_write_mean_det", feat.data_ptr(), idx.data_ptr(), _ptr(samp), frame_cnt.data_ptr(), E, C, HW, n_cells,
-          sums.data_ptr(), ws.buf.data_ptr(), ws.nbytes, _stream())
+    if active is not None:
+        _dev(active, torch.int32, "active")
+        if active.numel() != E:
+            raise ValueError("active must hold one int32 per episode")
+    _call("eod_write_mean_det_layout", feat.data_ptr(), int(layout), idx.data_ptr(), _ptr(samp), frame_cnt.data_ptr(), _ptr(active), E, C, HW,
+          n_cells, sums.data_ptr(), ws.buf.data_ptr(), ws.nbytes, _stream())
 
 
 def finalize_counts(idx: torch.Tensor, frame_cnt: torch.Tensor, counts: torch.Tensor,

@@ -33,7 +33,7 @@ import numpy as np
 import torch
 
 from . import formats, ops
-from ._lib import LAYOUT_CHW, ORDER_ZX, EodError
+from ._lib import LAYOUT_CHW, ORDER_ZX, WRITE_AUTO, WRITE_DET, EodError
 
 
 def split_streams(reset_first: Sequence[bool]) -> List[List[int]]:
@@ -227,13 +227,17 @@ class EpisodeRunner:
     tensors ordered on the caller's stream: ``idx`` (R,H,W) i32 or ``depth`` (R,H,W) + ``pose`` (R,12) + ``shifts`` (R,6);
     ``feat`` (R,C,H,W) [dense regime] or ``box_features`` (R,K,C) + ``mask_probs`` (R,K,S,S) + ``boxes`` (R,K,4) + ``n_obj`` (R).
     ``trusted_indices = True`` on the provider skips the range check of staged ``idx`` planes.
+    ``variant = WRITE_DET``: the dense write is the deterministic one, so a run reproduces bit for bit whatever the slot count and the
+    wave a stream lands in (size its workspace with ``batch.det_runs_per_episode``); the detection regime has no deterministic write
+    and raises EodError.
     """
 
     def __init__(self, provider, map_w: int, map_h: int, channels: int, n_slots: int, *, height: int = 480, width: int = 640,
                  device: torch.device = torch.device("cuda"), test_type: str = "default", rank: int = 0, world: int = 1,
                  intr: Optional[Sequence[float]] = None, cell: float = 0.2, order: int = ORDER_ZX, layout: int = LAYOUT_CHW,
                  save_dir: Optional[str] = None, zs_weight: Optional[torch.Tensor] = None, obs_score_thresh: float = 0.4,
-                 n_semmap_classes: int = 20, sample_stride: int = 8, mask_thresh: float = 0.5, pipeline: bool = True):
+                 n_semmap_classes: int = 20, sample_stride: int = 8, mask_thresh: float = 0.5, pipeline: bool = True,
+                 variant: int = WRITE_AUTO):
         from .memory import EpisodeBatch
         if test_type not in ("default", "episodic", "longterm"):
             raise ValueError(f"unknown TEST_TYPE {test_type!r}")           # detic/config.py:74
@@ -241,7 +245,7 @@ class EpisodeRunner:
         n = provider.n_episodes
         self.schedule = LockStepSchedule([provider.n_frames(i) for i in range(n)],
                                          [provider.n_frames(i) > 0 and provider.reset_flag(i, 0) for i in range(n)], n_slots, rank, world)
-        self.batch = EpisodeBatch(n_slots, map_w, map_h, channels, height, width, self.device, layout=layout, pipeline=pipeline)
+        self.batch = EpisodeBatch(n_slots, map_w, map_h, channels, height, width, self.device, layout=layout, variant=variant, pipeline=pipeline)
         self.batch.read_frozen = test_type == "longterm"
         self.intr, self.cell, self.order = intr, float(cell), order
         self.save_dir, self.sample_stride, self.mask_thresh = save_dir, sample_stride, mask_thresh
@@ -273,7 +277,9 @@ class EpisodeRunner:
 
     def run(self, on_levels: Optional[Callable[[Step, List[torch.Tensor]], None]] = None, max_steps: Optional[int] = None) -> dict:
         """Process this rank's share of the dataset.  on_levels(step, levels): consumer hook, called after every frame-step
-        with the three pooled fp16 levels (R,C,h,w) ordered on the caller's stream (idle slots hold stale values)."""
+        with the three pooled fp16 levels (R,C,h,w) ordered on the caller's stream (idle slots hold stale values).
+        With WRITE_DET the stats carry ``det_overflowed``: some run did not fit the workspace (since it was created) and took the
+        order-dependent reductions - the result is correct but no longer reproducible."""
         b = self.batch
         self.stats = {k: 0 for k in self.stats}                  # per run() call
         with torch.cuda.device(self.device):
@@ -297,6 +303,8 @@ class EpisodeRunner:
                     levels = b.step(depth, pose, shifts, self.intr, self.cell, inp["feat"], None, self.order, active=dev[0],
                                     inputs_ready=False, **masks, **geo)
                 else:
+                    if b.variant == WRITE_DET:
+                        raise EodError("EpisodeRunner(variant=WRITE_DET): the object-regime write (detections) is not deterministic")
                     n_obj = torch.where(dev[0] > 0, inp["n_obj"], torch.zeros_like(inp["n_obj"]))
                     levels = b.step_detections(depth, pose, shifts, self.intr, self.cell, inp["box_features"], inp["mask_probs"], inp["boxes"],
                                                n_obj, self.sample_stride, self.mask_thresh, self.order, inputs_ready=False, **masks, **geo)
@@ -311,6 +319,8 @@ class EpisodeRunner:
                         if a is not None and st:
                             self._save(s, self.provider.name(a[0]))
             b.join()
+            if b.variant == WRITE_DET:
+                self.stats["det_overflowed"] = b._det_ws is not None and b._det_ws.overflowed()
         return dict(self.stats)
 
 

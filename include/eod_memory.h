@@ -135,17 +135,22 @@ int eod_expand_counts(const int32_t *idx, const uint32_t *frame_cnt, int n_episo
  * bytes of the dominant stream: the 16-bit values are widened exactly and everything downstream is the fp32 arithmetic of the fp32
  * layouts).  16-bit CHW rows must be 16-byte aligned (HW % 8 == 0, else EOD_ERR_ALIGN); their TMA kernel takes 64-pixel tiles
  * (HW % 64 == 0 and a 16-byte aligned samp, else the LDG kernel - or EOD_ERR_UNSUPPORTED for EOD_WRITE_TMA / _TMA_DRY);
- * pix_inv_n with a 16-bit CHW layout is EOD_ERR_UNSUPPORTED.  eod_write_mean_det takes fp32 CHW features only.
+ * pix_inv_n with a 16-bit CHW layout is EOD_ERR_UNSUPPORTED.  eod_write_mean_det_layout takes every layout but the 16-bit CHW ones.
  * active (E) i32 nullable: the same mask eod_frame_count takes - slots of the lock-step batch with active[e] <= 0 (an episode
  * that has ended, custom_rcnn.py:441-443 iterates ragged sequences) are skipped without reading their features. */
 int eod_write_mean(const void *feat, int layout, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt,
                    int n_episodes, int C, int HW, int64_t n_cells, float *sums, int variant, const float *pix_inv_n,
                    const int32_t *active, eod_stream_t stream);
 
-/* Deterministic variant of the main pass (CHW features, HW %% 32 == 0): run sums are stored in raster run order
+/* Deterministic variant of the main pass (HW %% 32 == 0): run sums are stored in raster run order
  * (no atomics), then every touched cell adds the partial sums of its runs in ascending run position, divides by
  * n_cell and adds the mean ONCE to sums[cell] - bitwise reproducible run to run and independent of how episodes are
  * batched, and the arithmetic shape of custom_rcnn.py:930-934,742 (sum, divide, add).
+ * layout: EOD_LAYOUT_CHW, _HWC, _HWC_BF16 or _HWC_F16 (EOD_LAYOUT_CHW_BF16 / _F16: EOD_ERR_UNSUPPORTED).  Every layout sums a run's
+ * sampled pixels in raster order from +0 with 16-bit values widened exactly, so the result does not depend on the layout: channels-last
+ * x gives the bits of CHW x, bf16 / fp16 x those of CHW fp32 x.float().
+ * active (E) i32 nullable: the mask eod_frame_count took - slots with active[e] <= 0 get no runs, their features are not read and
+ * their sums are left alone.  eod_write_mean_det is eod_write_mean_det_layout with EOD_LAYOUT_CHW and no mask.
  * workspace: caller-owned, 256-byte aligned, zero-filled ONCE before first use (the library leaves its persistent
  * planes zero again after every call); eod_write_mean_det_workspace_bytes(E, C, HW, cells, runs_per_episode) sizes
  * it for runs_per_episode runs of equal cell id per episode and frame (<= 0: HW/4).  Runs that do not fit fall back
@@ -156,6 +161,9 @@ int64_t eod_write_mean_det_status_offset(int n_episodes, int64_t n_cells);
 int eod_write_mean_det(const float *feat, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, int n_episodes,
                        int C, int HW, int64_t n_cells, float *sums, void *workspace, int64_t workspace_bytes,
                        eod_stream_t stream);
+int eod_write_mean_det_layout(const void *feat, int layout, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt,
+                              const int32_t *active, int n_episodes, int C, int HW, int64_t n_cells, float *sums, void *workspace,
+                              int64_t workspace_bytes, eod_stream_t stream);
 
 /* Post-pass: counts[cell] += 1 for every visible cell (custom_rcnn.py:699-701,743) and frame_cnt := 0.
  * touched (E,cells) u8 nullable: |= 1 where the cell received samples this frame (observed_mem, :922).
