@@ -3,6 +3,7 @@
 #include <string.h>
 
 #include "eod_common.cuh"
+#include "tmap_cache.cuh"
 
 static thread_local char g_err[512] = "";
 
@@ -35,6 +36,17 @@ int eod_num_sms()
         n = (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && v > 0) ? v : EOD_NUM_SMS_FALLBACK;
     }
     return n;
+}
+
+PFN_eodEncodeTiled eod_encode_tiled_fn()
+{
+    static const PFN_eodEncodeTiled fn = [] {
+        void *p = nullptr;
+        cudaDriverEntryPointQueryResult qres;
+        const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess;
+        return ok ? reinterpret_cast<PFN_eodEncodeTiled>(p) : nullptr;
+    }();
+    return fn;
 }
 
 // Work tickets for persistent kernels that claim their tiles dynamically: a pool of zeroed {next, done} int pairs per device.

@@ -31,48 +31,6 @@ constexpr int LN_B_BYTES = LN_MAXN * 128;
 constexpr int LN_STAGE_BYTES = 2 * LN_A_BYTES + 2 * LN_B_BYTES;     // 96 KB
 constexpr int LN_SMEM_BYTES = 2 * LN_STAGE_BYTES + 1024 + 64;
 
-__device__ __forceinline__ void ln_tmem_alloc(uint32_t *dst_smem, uint32_t ncols)
-{
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void ln_tmem_dealloc(uint32_t taddr, uint32_t ncols)
-{
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void ln_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void ln_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void ln_commit(uint64_t *bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void ln_tmem_ld16(uint32_t taddr, uint32_t (&v)[16])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]), "=r"(v[10]),
-          "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void ln_tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// K-major SWIZZLE_128B matrix descriptor (same encoding as csrc/project_fuse.cu): 8-row atoms of 1024 B
-__device__ __forceinline__ uint64_t ln_desc_sw128(uint32_t smem_addr)
-{
-    return (uint64_t)((smem_addr >> 4) & 0x3fffu) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
-}
 // instruction descriptor: D = F32 (1 << 4), A = B = TF32 (2 << 7, 2 << 10), both K-major, N >> 3 in [17,23), M >> 4 in [24,29)
 __device__ __forceinline__ uint32_t ln_idesc(int n) { return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(LN_BM >> 4) << 24); }
 
@@ -99,6 +57,7 @@ __device__ __forceinline__ void ln_store4(uint32_t big_base, uint32_t small_base
     float4 b, s;
     b.x = tf32_big(x.x); b.y = tf32_big(x.y); b.z = tf32_big(x.z); b.w = tf32_big(x.w);
     s.x = tf32_small(x.x, b.x); s.y = tf32_small(x.y, b.y); s.z = tf32_small(x.z, b.z); s.w = tf32_small(x.w, b.w);
+    // f32 stores, not sts128: moving the halves into .b32 registers makes ptxas spill in linear_rows_kernel
     asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(big_base + off), "f"(b.x), "f"(b.y), "f"(b.z), "f"(b.w) : "memory");
     asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(small_base + off), "f"(s.x), "f"(s.y), "f"(s.z), "f"(s.w) : "memory");
 }
@@ -153,10 +112,10 @@ __global__ void __launch_bounds__(128) linear_rows_kernel(const LinearParams P)
         mbar_init(bars + 2, 1);
         mbar_fence_init();
     }
-    if (warp == 0) ln_tmem_alloc(tmem_slot, tmem_cols);
-    ln_fence_before();
+    if (warp == 0) tmem_alloc(tmem_slot, tmem_cols);
+    tc_fence_before();
     __syncthreads();
-    ln_fence_after();
+    tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
 
     // this thread's operand rows
@@ -177,31 +136,31 @@ __global__ void __launch_bounds__(128) linear_rows_kernel(const LinearParams P)
         fence_proxy_async();                                 // generic-proxy stores -> visible to the tensor core's async-proxy reads
         __syncthreads();
         if (tid == 0) {
-            ln_fence_after();
+            tc_fence_after();
 #pragma unroll
             for (int k = 0; k < LN_BK / 8; ++k) {            // 8 tf32 = 32 bytes along K inside the swizzle row
-                const uint64_t ab = ln_desc_sw128(a_big + k * 32), as = ln_desc_sw128(a_small + k * 32);
-                const uint64_t bb = ln_desc_sw128(b_big + k * 32), bs = ln_desc_sw128(b_small + k * 32);
+                const uint64_t ab = umma_desc_sw128(a_big + k * 32), as = umma_desc_sw128(a_small + k * 32);
+                const uint64_t bb = umma_desc_sw128(b_big + k * 32), bs = umma_desc_sw128(b_small + k * 32);
                 umma_tf32(tmem_base, as, bb, idesc, (kb | k) != 0);       // small terms first, the dominant one last
                 umma_tf32(tmem_base, ab, bs, idesc, 1u);
                 umma_tf32(tmem_base, ab, bb, idesc, 1u);
             }
-            ln_commit(bars + s);
-            if (kb == n_kb - 1) ln_commit(bars + 2);
+            umma_commit(bars + s);
+            if (kb == n_kb - 1) umma_commit(bars + 2);
         }
     }
 
     // ===== epilogue: warp w owns TMEM lanes [32w, 32w + 32) = rows m0 + 32w + lane =====
     mbar_wait(bars + 2, 0);
-    ln_fence_after();
+    tc_fence_after();
     const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16);
     float *y_row = a_valid ? P.Y + (P.y_dst ? __ldg(P.y_dst + m) : (int64_t)m) * P.y_rs : nullptr;
     const bool y_vec = (P.y_rs & 3) == 0 && ((reinterpret_cast<uintptr_t>(P.Y) & 15u) == 0);
 #pragma unroll 1
     for (int c0 = 0; c0 < N; c0 += 16) {
         uint32_t acc[16];
-        ln_tmem_ld16(taddr + c0, acc);
-        ln_tmem_ld_wait();
+        tmem_ld16(taddr + c0, acc);
+        tmem_ld_wait();
         if (a_valid) {
             float v[16];
 #pragma unroll
@@ -219,9 +178,9 @@ __global__ void __launch_bounds__(128) linear_rows_kernel(const LinearParams P)
             }
         }
     }
-    ln_fence_before();
+    tc_fence_before();
     __syncthreads();
-    if (warp == 0) ln_tmem_dealloc(tmem_base, tmem_cols);
+    if (warp == 0) tmem_dealloc(tmem_base, tmem_cols);
 }
 
 // winners of eod_write_max -> compact (source element offset, destination row) list for the 'replace' update

@@ -39,65 +39,6 @@ constexpr int PF_TMEM_COLS = 2 * PF_BN;                   // 256 fp32 columns
 constexpr int PF_SMEM_BYTES = PF_STAGES * PF_STAGE_BYTES + 1024 /* alignment slack */ + 64 /* barriers + tmem ptr */;
 constexpr float PF_LO_SCALE = 2048.f, PF_LO_INV = 1.f / 2048.f;
 
-// ---- PTX wrappers -------------------------------------------------------------------------------------------
-__device__ __forceinline__ void tma_load_2d(void *dst, const void *tmap, int x, int y, uint64_t *bar)
-{
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(smem_u32(dst)),
-                 "l"(tmap), "r"(x), "r"(y), "r"(smem_u32(bar))
-                 : "memory");
-}
-// L2 prefetch of a 3-D tile (no shared-memory destination): takes the DRAM latency out of the small smem rings
-__device__ __forceinline__ void tma_prefetch_3d(const void *tmap, int x, int y, int z)
-{
-    asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];" ::"l"(tmap), "r"(x), "r"(y), "r"(z) : "memory");
-}
-__device__ __forceinline__ void tmem_alloc(uint32_t *dst_smem, uint32_t ncols)
-{
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols)
-{
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-// D[tmem] (+)= A[smem desc] * B[smem desc], fp16 inputs, fp32 accumulate; issued by ONE thread
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// mbarrier arrive once all tcgen05.mma issued so far by this thread have completed (implies fence::before_thread_sync)
-__device__ __forceinline__ void umma_commit(uint64_t *bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// 16 consecutive fp32 columns of this thread's TMEM lane
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]), "=r"(v[10]),
-          "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// K-major, SWIZZLE_128B shared-memory matrix descriptor (cute/arch/mma_sm100_desc.hpp SmemDescriptor): start address >> 4 in
-// bits [0,14), leading byte offset (unused for swizzled K-major; 1) in [16,30), stride byte offset = 1024 B (one 8-row
-// swizzle atom) >> 4 in [32,46), version 1 in [46,48), layout type 2 (SWIZZLE_128B) in [61,64).
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr)
-{
-    return (uint64_t)((smem_addr >> 4) & 0x3fffu) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
-}
 // instruction descriptor (InstrDescriptor): D = F32 (1 << 4), A = B = F16 (0), both K-major, N >> 3 in [17,23), M >> 4 in [24,29)
 constexpr uint32_t PF_IDESC = (1u << 4) | ((uint32_t)(2 * PF_BN >> 3) << 17) | ((uint32_t)(PF_BM >> 4) << 24);
 
@@ -421,60 +362,32 @@ __global__ void __launch_bounds__(256) split_weights_kernel(const float *__restr
     out[(row_hi + PF_BN) * K + k] = lo;
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                    const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-PFN_encodeTiled pf_encode_fn()
-{
-    static PFN_encodeTiled fn = nullptr;
-    if (!fn) {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_encodeTiled>(p);
-    }
-    return fn;
-}
-
 // (rows, K) fp16 row-major -> 2-D map with a {64, box_rows} SWIZZLE_128B box; rows beyond `rows` read as zero
 int pf_make_tmap(const void *ptr, int64_t rows, int K, int box_rows, CUtensorMap *tm)
 {
-    PFN_encodeTiled enc = pf_encode_fn();
-    EOD_REQUIRE(enc, EOD_ERR_LAUNCH, "eod_project_fuse: cuTensorMapEncodeTiled entry point unavailable");
     const cuuint64_t gdim[2] = {(cuuint64_t)K, (cuuint64_t)rows};
     const cuuint64_t gstr[1] = {(cuuint64_t)K * 2};
     const cuuint32_t box[2] = {PF_BK, (cuuint32_t)box_rows};
-    const CUresult r = eod_encode_tmap_cached(enc, tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, ptr, gdim, gstr, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
-    EOD_REQUIRE(r == CUDA_SUCCESS, EOD_ERR_LAUNCH, "eod_project_fuse: cuTensorMapEncodeTiled failed (%d)", (int)r);
-    return EOD_OK;
+    return eod_encode_tmap("eod_project_fuse", tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, ptr, gdim, gstr, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
 }
 
 // level (E, hw, K) f16 -> 3-D map, box {64, 256, 1}: rows beyond hw of an episode read as zero (never the next episode)
 int p2_make_tmap_a(const void *ptr, int E, int hw, int K, CUtensorMap *tm)
 {
-    PFN_encodeTiled enc = pf_encode_fn();
-    EOD_REQUIRE(enc, EOD_ERR_LAUNCH, "eod_project_fuse: cuTensorMapEncodeTiled entry point unavailable");
     const cuuint64_t gdim[3] = {(cuuint64_t)K, (cuuint64_t)hw, (cuuint64_t)E};
     const cuuint64_t gstr[2] = {(cuuint64_t)K * 2, (cuuint64_t)hw * K * 2};
     const cuuint32_t box[3] = {PF_BK, P2_BM, 1};
-    const CUresult r = eod_encode_tmap_cached(enc, tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, ptr, gdim, gstr, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
-    EOD_REQUIRE(r == CUDA_SUCCESS, EOD_ERR_LAUNCH, "eod_project_fuse: cuTensorMapEncodeTiled(level) failed (%d)", (int)r);
-    return EOD_OK;
+    return eod_encode_tmap("eod_project_fuse", tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, ptr, gdim, gstr, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
 }
 
 // res (E, N, hw) f32 -> 3-D map, box {256 px, 16 channels, 1}
 int p2_make_tmap_r(const float *ptr, int E, int hw, int N, CUtensorMap *tm)
 {
-    PFN_encodeTiled enc = pf_encode_fn();
-    EOD_REQUIRE(enc, EOD_ERR_LAUNCH, "eod_project_fuse: cuTensorMapEncodeTiled entry point unavailable");
     const cuuint64_t gdim[3] = {(cuuint64_t)hw, (cuuint64_t)N, (cuuint64_t)E};
     const cuuint64_t gstr[2] = {(cuuint64_t)hw * 4, (cuuint64_t)hw * N * 4};
     const cuuint32_t box[3] = {P2_BM, P2_RCH, 1};
-    const CUresult r = eod_encode_tmap_cached(enc, tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ptr, gdim, gstr, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                                              CU_TENSOR_MAP_SWIZZLE_NONE);
-    EOD_REQUIRE(r == CUDA_SUCCESS, EOD_ERR_LAUNCH, "eod_project_fuse: cuTensorMapEncodeTiled(res) failed (%d)", (int)r);
-    return EOD_OK;
+    return eod_encode_tmap("eod_project_fuse", tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ptr, gdim, gstr, box, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                           CU_TENSOR_MAP_SWIZZLE_NONE);
 }
 
 // the single-level, one-tile-per-CTA kernel: any hw (no TMA on res), also the comparator for the persistent one

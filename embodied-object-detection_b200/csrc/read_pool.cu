@@ -204,33 +204,6 @@ __device__ __forceinline__ QuadIdx load_quad_idx(const IdxT *src, int W)
     return q;
 }
 
-// shared memory by 32-bit shared-window address (inline PTX): the compiler keeps ONE base register per warp instead of
-// re-deriving `&array[warp][...]` from %tid / %cluster_ctaid inside the loops (v4a: ~10 uniform-datapath instructions per window)
-__device__ __forceinline__ int4 rp_lds128(uint32_t a)
-{
-    int4 v;
-    asm volatile("ld.shared.v4.s32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ int2 rp_lds64(uint32_t a)
-{
-    int2 v;
-    asm volatile("ld.shared.v2.s32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ int rp_lds32(uint32_t a)
-{
-    int v;
-    asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(a));
-    return v;
-}
-__device__ __forceinline__ void rp_sts128(uint32_t a, int x, int y, int z, int w)
-{
-    asm volatile("st.shared.v4.s32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w) : "memory");
-}
-__device__ __forceinline__ void rp_sts32(uint32_t a, int x) { asm volatile("st.shared.s32 [%0], %1;" ::"r"(a), "r"(x) : "memory"); }
-__device__ __forceinline__ void rp_sts16(uint32_t a, unsigned x) { asm volatile("st.shared.u16 [%0], %1;" ::"r"(a), "h"((unsigned short)x) : "memory"); }
-
 // per-warp slice: ids window-major (1024 B) | window descriptors {first cell, second cell or -1, run-head mask, 0} (16 x 16 B) |
 // first cells (16 x 4 B) | run-head masks (16 x 2 B)
 constexpr int kRpIdx = 0, kRpDesc = 1024, kRpWc = 1280, kRpWm = 1344, kRpSlice = 1376;
@@ -279,8 +252,8 @@ __global__ void __launch_bounds__(kReadWarps * 32, (C >= 512 ? 2 : (C >= 256 ? 3
         e += se;
         if (item + stride < n_items) nxt = load_quad_idx<IdxT>(src_of(e, qy, qx), W);
         // stage the ids window-major; derive the window's run heads in summation (row-major) order
-        rp_sts128(sm_ids, q.a[0], q.a[1], q.a[2], q.a[3]);
-        rp_sts128(sm_ids + 16, q.b[0], q.b[1], q.b[2], q.b[3]);
+        sts128(sm_ids, q.a[0], q.a[1], q.a[2], q.a[3]);
+        sts128(sm_ids + 16, q.b[0], q.b[1], q.b[2], q.b[3]);
         const int prev = __shfl_up_sync(0xffffffffu, q.b[3], 1);             // last pixel of the window's second row (for hh == 1)
         unsigned m8 = (hh == 0 || q.a[0] != prev) ? 1u : 0u;
         m8 |= (q.a[1] != q.a[0]) << 1 | (q.a[2] != q.a[1]) << 2 | (q.a[3] != q.a[2]) << 3 | (q.b[0] != q.a[3]) << 4 | (q.b[1] != q.b[0]) << 5 |
@@ -301,9 +274,9 @@ __global__ void __launch_bounds__(kReadWarps * 32, (C >= 512 ? 2 : (C >= 256 ? 3
         const bool in2_o = __shfl_xor_sync(0xffffffffu, (int)in2, 1) != 0;
         if (hh == 0) {
             const unsigned m16 = m8 | (other << 8);
-            rp_sts128(sm + kRpDesc + w * 16, cA, (in2 && in2_o && cB != cA) ? cB : -1, (int)m16, 0);
-            rp_sts32(sm + kRpWc + w * 4, cA);
-            rp_sts16(sm + kRpWm + w * 2, m16);
+            sts128(sm + kRpDesc + w * 16, cA, (in2 && in2_o && cB != cA) ? cB : -1, m16, 0);
+            sts32(sm + kRpWc + w * 4, cA);
+            sts16(sm + kRpWm + w * 2, m16);
         }
         __syncwarp();
 
@@ -322,13 +295,13 @@ __global__ void __launch_bounds__(kReadWarps * 32, (C >= 512 ? 2 : (C >= 256 ? 3
             // gathered value x is an fp16 number, so the sequential fp32 sum 0+x+x+...+x is exact at every step
             // (k*x, k <= 16, has at most 15 significant bits) and avg_pool2d(4) returns x itself - except that -0.0
             // becomes +0.0 (0 + -0 = +0), which the shortcuts reproduce by adding +0 (found by the read stress sweep).
-            const int4 wc4 = rp_lds128(sm + kRpWc + l0 * 16);
-            const int2 wm2 = rp_lds64(sm + kRpWm + l0 * 8);
+            const uint4 wc4 = lds128(sm + kRpWc + l0 * 16);
+            const uint2 wm2 = lds64(sm + kRpWm + l0 * 8);
             Vec<V> v0;
             if (wm2.x == 0x00010001 && wm2.y == 0x00010001 && wc4.x == wc4.y && wc4.x == wc4.z && wc4.x == wc4.w) {
                 // whole 8x8 block in one cell: pool(4), pool(2) and the fp16 rounding all return the gathered value
-                if (wc4.x != cur_cell) cur = finish<V>(fetch(wc4.x));
-                cur_cell = wc4.x;
+                if ((int)wc4.x != cur_cell) cur = finish<V>(fetch((int)wc4.x));
+                cur_cell = (int)wc4.x;
                 v0 = vadd<V>(cur, vzero<V>());               // the reference's sums start from +0: a gathered -0.0 comes out as +0.0
             } else {
                 Vec<V> s2 = vzero<V>();
@@ -338,9 +311,9 @@ __global__ void __launch_bounds__(kReadWarps * 32, (C >= 512 ? 2 : (C >= 256 ? 3
                 uint32_t dsc = sm + kRpDesc + l0 * 64;
 #pragma unroll 1
                 for (int win = 0; win < 4; ++win, dsc += 16) {   // 4x4 windows of the avg_pool2d(4) (timm.py:152), row-major
-                    const int4 d = rp_lds128(dsc);
-                    const int wc = d.x, wb = d.y;
-                    unsigned rest = (unsigned)d.z & ~1u;        // run heads after the first pixel
+                    const uint4 d = lds128(dsc);
+                    const int wc = (int)d.x, wb = (int)d.y;
+                    unsigned rest = d.z & ~1u;        // run heads after the first pixel
                     if (wc != cur_cell) cur = finish<V>(fetch(wc));
                     cur_cell = wc;
                     Vec<V> s4;
@@ -378,7 +351,7 @@ __global__ void __launch_bounds__(kReadWarps * 32, (C >= 512 ? 2 : (C >= 256 ? 3
                             Raw raw;
                             int ncell = cur_cell;
                             if (pn < 16) {                   // next run's row in flight under the adds
-                                ncell = rp_lds32(cells + pn * 4);
+                                ncell = (int)lds32(cells + pn * 4);
                                 raw = fetch(ncell);
                             }
                             int len = pn - p;                // 1..15, warp-uniform; sequential fp32 sum: `len` times + cur

@@ -6,9 +6,13 @@
 #include <cuda.h>
 #include <string.h>
 
+#include "eod_common.cuh"
+
 typedef CUresult (*PFN_eodEncodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
                                        const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                        CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+PFN_eodEncodeTiled eod_encode_tiled_fn();      // the driver's cuTensorMapEncodeTiled, looked up once per process; nullptr if absent (api.cu)
 
 struct EodTmapKey {
     const void *ptr;
@@ -17,10 +21,13 @@ struct EodTmapKey {
     int rank, dtype, promo, swizzle;
 };
 
-static inline CUresult eod_encode_tmap_cached(PFN_eodEncodeTiled enc, CUtensorMap *tm, CUtensorMapDataType dtype, cuuint32_t rank, const void *ptr,
-                                             const cuuint64_t *gdim, const cuuint64_t *gstr, const cuuint32_t *box, CUtensorMapL2promotion promo,
-                                             CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B)
+// Returns EOD_OK, or EOD_ERR_LAUNCH with the message prefixed by `what` (the calling entry point).
+static inline int eod_encode_tmap(const char *what, CUtensorMap *tm, CUtensorMapDataType dtype, cuuint32_t rank, const void *ptr,
+                                  const cuuint64_t *gdim, const cuuint64_t *gstr, const cuuint32_t *box, CUtensorMapL2promotion promo,
+                                  CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B)
 {
+    const PFN_eodEncodeTiled enc = eod_encode_tiled_fn();
+    EOD_REQUIRE(enc, EOD_ERR_LAUNCH, "%s: cuTensorMapEncodeTiled entry point unavailable", what);
     constexpr int N = 16;
     static thread_local EodTmapKey keys[N];
     static thread_local CUtensorMap maps[N];
@@ -33,14 +40,14 @@ static inline CUresult eod_encode_tmap_cached(PFN_eodEncodeTiled enc, CUtensorMa
     for (int i = 0; i < used; ++i)
         if (memcmp(&keys[i], &k, sizeof(k)) == 0) {
             *tm = maps[i];
-            return CUDA_SUCCESS;
+            return EOD_OK;
         }
     const cuuint32_t estr[3] = {1, 1, 1};
     const CUresult r = enc(tm, dtype, rank, const_cast<void *>(ptr), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, promo,
                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return r;
+    EOD_REQUIRE(r == CUDA_SUCCESS, EOD_ERR_LAUNCH, "%s: cuTensorMapEncodeTiled failed (%d)", what, (int)r);
     const int slot = used < N ? used++ : (next = (next + 1) % N);
     keys[slot] = k;
     maps[slot] = *tm;
-    return r;
+    return EOD_OK;
 }

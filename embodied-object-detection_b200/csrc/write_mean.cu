@@ -571,78 +571,6 @@ struct TmaCfg {
     static_assert(kSmemBytes <= 232448, "exceeds 227 KB of shared memory");
 };
 
-__device__ __forceinline__ uint64_t make_evict_first_policy()
-{
-    uint64_t pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
-
-__device__ __forceinline__ void tma_load_3d_hint(uint32_t dst, const void *tmap, int x, int y, int z, uint32_t bar, uint64_t pol)
-{
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3, %4}], [%5], %6;" ::"r"(dst),
-        "l"(tmap), "r"(x), "r"(y), "r"(z), "r"(bar), "l"(pol)
-        : "memory");
-}
-__device__ __forceinline__ void bulk_load_1d_s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait_s(uint32_t bar, uint32_t parity)
-{
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAIT_LOOP_S:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE_S;\n\t"
-        "bra WAIT_LOOP_S;\n\t"
-        "DONE_S:\n\t"
-        "}" ::"r"(bar),
-        "r"(parity)
-        : "memory");
-}
-// same wait with a suspend-time hint (ns): the warp sleeps in hardware instead of re-issuing the poll
-__device__ __forceinline__ void mbar_wait_hint(uint32_t bar, uint32_t parity, uint32_t hint_ns)
-{
-    if (hint_ns == 0) { mbar_wait_s(bar, parity); return; }
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAIT_LOOP_H:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
-        "@p bra DONE_H;\n\t"
-        "bra WAIT_LOOP_H;\n\t"
-        "DONE_H:\n\t"
-        "}" ::"r"(bar),
-        "r"(parity), "r"(hint_ns)
-        : "memory");
-}
-__device__ __forceinline__ float4 lds128(uint32_t addr)
-{
-    float4 v;
-    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ uint32_t lds32(uint32_t addr)
-{
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ void sts64(uint32_t addr, uint32_t a, uint32_t b)
-{
-    asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(addr), "r"(a), "r"(b) : "memory");
-}
-__device__ __forceinline__ uint32_t lds8(uint32_t addr)
-{
-    uint32_t v;
-    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(addr));
-    return v;
-}
-
 // One staged unit of 16-bit features: 64 pixels x kChanBlk channels, row `lane` of the box at `tile`.  Lane l looks at pixels l and
 // l + 32.  Groups are formed per half (MATCH.ANY) and joined across the halves with one ballot per group of the lower half; the
 // upper-half groups no lower-half group claimed are cells the lower half does not see.  Per group, lane l sums channels l, l+32, ...
@@ -691,13 +619,13 @@ __device__ __forceinline__ void chw16_unit(uint32_t tile, uint32_t aux, int t, i
             const unsigned mj = (unsigned)(m >> (8 * j)) & 0xffu;
             if (mj == 0) continue;
             const uint32_t a = tile + (((uint32_t)j ^ sw) << 4);
-            float4 v[kJ];
+            uint4 v[kJ];
 #pragma unroll
             for (int k = 0; k < kJ; ++k) v[k] = lds128(a + k * 32 * Cfg::kRowBytes);
             if (mj == 0xffu) {                                     // whole chunk inside the group, all sampled
 #pragma unroll
                 for (int k = 0; k < kJ; ++k) {
-                    const uint32_t w[4] = {__float_as_uint(v[k].x), __float_as_uint(v[k].y), __float_as_uint(v[k].z), __float_as_uint(v[k].w)};
+                    const uint32_t w[4] = {v[k].x, v[k].y, v[k].z, v[k].w};
 #pragma unroll
                     for (int q = 0; q < 4; ++q) {
                         const float2 f = widen2<F>(w[q]);
@@ -710,8 +638,8 @@ __device__ __forceinline__ void chw16_unit(uint32_t tile, uint32_t aux, int t, i
                     if (mj & (1u << i)) {
 #pragma unroll
                         for (int k = 0; k < kJ; ++k) {
-                            const float *vk = reinterpret_cast<const float *>(&v[k]);
-                            const float2 f = widen2<F>(__float_as_uint(vk[i >> 1]));
+                            const uint32_t *vk = reinterpret_cast<const uint32_t *>(&v[k]);
+                            const float2 f = widen2<F>(vk[i >> 1]);
                             acc[k] = __fadd_rn(acc[k], (i & 1) ? f.y : f.x);
                         }
                     }
@@ -741,6 +669,15 @@ struct DetArgs {
     int cap;                     // runs per episode the workspace holds
 };
 
+// The sampled pixels (bit p = pixel p of a 32-pixel tile) of the deterministic run that starts at head p0; `later` holds the heads
+// after p0 only.  The run pre-passes (det_run_sampled) and both kDet consumers must find the same runs in the same order: a run's
+// rank among them is its slot in partials.
+__device__ __forceinline__ unsigned det_run_mask(unsigned later, unsigned samps, int p0)
+{
+    const int p1 = later ? (__ffs(later) - 1) : TILE_PX;
+    return samps & (0xffffffffu >> (32 - p1)) & (0xffffffffu << p0);
+}
+
 // F: feature element type (FEAT_BF16 / FEAT_F16 take the 64-pixel unit and chw16_unit; neither kPixN nor kDet)
 template <int C, bool kDry, bool kPixN, bool kDet, int F = FEAT_F32>
 __global__ void __launch_bounds__(TmaCfg<C, F>::kThreads, 1)
@@ -763,8 +700,8 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
     const bool has_samp = samp != nullptr;
     if (tid == 0) {
         for (int s = 0; s < Cfg::kStages; ++s) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(full0 + 8 * s), "r"(1));    // producer's arrive.expect_tx
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(empty0 + 8 * s), "r"(1));   // the owning warp's arrive
+            mbar_init(full0 + 8 * s, 1);        // producer's arrive.expect_tx
+            mbar_init(empty0 + 8 * s, 1);       // the owning warp's arrive
         }
         mbar_fence_init();
         fence_proxy_async();
@@ -807,13 +744,13 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
                     sts64(aux + Cfg::kAuxUnit, (uint32_t)t, (uint32_t)cb | (idle ? 0x100u : 0u));
                     if (idle) {
                         // idle slot of the batch: the stage is handed over empty, nothing is fetched
-                        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(fullb) : "memory");
+                        mbar_arrive(fullb);
                     } else {
-                        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(fullb), "r"(tx) : "memory");
+                        mbar_expect_tx(fullb, tx);
                         tma_load_3d_hint(base + stage * Cfg::kUnitBytes, &tmap, p0, cb * Cfg::kChanBlk, e, fullb, pol);
-                        bulk_load_1d_s(aux + Cfg::kAuxCells, idx + (size_t)e * HW + p0, kTilePx * 4, fullb);
-                        if (has_samp) bulk_load_1d_s(aux + Cfg::kAuxSamp, samp + (size_t)e * HW + p0, kTilePx, fullb);
-                        if (kPixN) bulk_load_1d_s(aux + Cfg::kAuxPixN, pix_n + (size_t)e * HW + p0, kTilePx * 4, fullb);
+                        bulk_load_1d(aux + Cfg::kAuxCells, idx + (size_t)e * HW + p0, kTilePx * 4, fullb);
+                        if (has_samp) bulk_load_1d(aux + Cfg::kAuxSamp, samp + (size_t)e * HW + p0, kTilePx, fullb);
+                        if (kPixN) bulk_load_1d(aux + Cfg::kAuxPixN, pix_n + (size_t)e * HW + p0, kTilePx * 4, fullb);
                     }
                     if (++stage == n_stages) { stage = 0; phase ^= 1; }
                 }
@@ -824,7 +761,7 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
             for (int s = 0; s < n_stages; ++s) {                              // one end marker per consumer warp
                 mbar_wait_hint(empty0 + 8 * stage, phase ^ 1, wait_hint);
                 sts64(aux0 + stage * Cfg::kAuxBytes + Cfg::kAuxUnit, 0xffffffffu, 0u);
-                asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(full0 + 8 * stage) : "memory");
+                mbar_arrive(full0 + 8 * stage);
                 if (++stage == n_stages) { stage = 0; phase ^= 1; }
             }
             if (work) {
@@ -876,12 +813,8 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
                 const int p0 = __ffs(heads) - 1;                       // first pixel of the run / group
                 heads &= heads - 1;
                 unsigned m;
-                if (kDet) {
-                    const int p1 = heads ? (__ffs(heads) - 1) : TILE_PX;
-                    m = samps & (0xffffffffu >> (32 - p1)) & (0xffffffffu << p0);
-                } else {
-                    m = samps & __shfl_sync(0xffffffffu, grp, p0);
-                }
+                if (kDet) m = det_run_mask(heads, samps, p0);
+                else m = samps & __shfl_sync(0xffffffffu, grp, p0);
                 if (m == 0) continue;                                  // no sampled pixel in this run / group
                 float acc[kJ];
 #pragma unroll
@@ -894,7 +827,10 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
                     const uint32_t a = tile + (((uint32_t)j ^ sw) << 4);
                     float4 v[kJ];
 #pragma unroll
-                    for (int k = 0; k < kJ; ++k) v[k] = lds128(a + k * 32 * TILE_PX * 4);
+                    for (int k = 0; k < kJ; ++k) {
+                        const uint4 u = lds128(a + k * 32 * TILE_PX * 4);
+                        v[k] = make_float4(__uint_as_float(u.x), __uint_as_float(u.y), __uint_as_float(u.z), __uint_as_float(u.w));
+                    }
                     if (mj == 15u) {                                   // whole chunk inside the run, all sampled
 #pragma unroll
                         for (int k = 0; k < kJ; ++k) acc[k] = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(acc[k], v[k].x), v[k].y), v[k].z), v[k].w);
@@ -938,7 +874,7 @@ write_mean_chw_tma_kernel(const __grid_constant__ CUtensorMap tmap, const int32_
             }
         }
         __syncwarp();                                                  // every lane's tile reads are done: release the stage
-        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(emptyb) : "memory");
+        if (lane == 0) mbar_arrive(emptyb);
     }
 }
 
@@ -1009,12 +945,8 @@ __global__ void __launch_bounds__(256, 3) write_mean_hwc_kernel(const void *__re
             const int lead = __ffs(leaders) - 1;
             leaders &= leaders - 1;
             unsigned rem;
-            if constexpr (kDet) {
-                const int p1 = leaders ? (__ffs(leaders) - 1) : TILE_PX;
-                rem = samps & (0xffffffffu >> (32 - p1)) & (0xffffffffu << lead);   // sampled pixels of this run
-            } else {
-                rem = __shfl_sync(0xffffffffu, grp, lead) & samps;                 // sampled pixels of this cell
-            }
+            if constexpr (kDet) rem = det_run_mask(leaders, samps, lead);       // sampled pixels of this run
+            else rem = __shfl_sync(0xffffffffu, grp, lead) & samps;             // sampled pixels of this cell
             if (rem == 0u) continue;
             const int cell = __shfl_sync(0xffffffffu, my_cell, lead);
             float4 acc[V];
@@ -1072,22 +1004,6 @@ __global__ void __launch_bounds__(256, 3) write_mean_hwc_kernel(const void *__re
 // ------------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------------
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                    const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-PFN_encodeTiled get_encode_fn()
-{
-    static PFN_encodeTiled fn = nullptr;
-    if (!fn) {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_encodeTiled>(p);
-    }
-    return fn;
-}
-
 template <int C, bool kDry, bool kPixN, bool kDet = false, int F = FEAT_F32>
 int launch_tma_kernel(const CUtensorMap &tmap, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const float *pix_n,
                       const int32_t *active, int E, int HW, int64_t n_cells, float *sums, cudaStream_t st, const DetArgs det = DetArgs{})
@@ -1121,8 +1037,6 @@ template <int C, int F = FEAT_F32>
 int make_feature_tmap(const void *feat, int E, int HW, CUtensorMap *tmap)
 {
     using Cfg = TmaCfg<C, F>;
-    PFN_encodeTiled enc = get_encode_fn();
-    EOD_REQUIRE(enc, EOD_ERR_LAUNCH, "eod_write_mean: cuTensorMapEncodeTiled entry point unavailable");
     constexpr cuuint64_t esz = F == FEAT_F32 ? 4 : 2;
     constexpr CUtensorMapDataType dtype = F == FEAT_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
                                           : (F == FEAT_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16);
@@ -1132,9 +1046,7 @@ int make_feature_tmap(const void *feat, int E, int HW, CUtensorMap *tmap)
     static const int promo_env = [] { const char *v = getenv("EOD_TMA_L2_PROMOTION"); return v ? atoi(v) : 256; }();   // tuning knob: 0 | 128 | 256
     const CUtensorMapL2promotion promo = promo_env == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE
                                          : (promo_env == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
-    const CUresult r = eod_encode_tmap_cached(enc, tmap, dtype, 3, feat, gdim, gstr, box, promo);
-    EOD_REQUIRE(r == CUDA_SUCCESS, EOD_ERR_LAUNCH, "eod_write_mean: cuTensorMapEncodeTiled failed (%d)", (int)r);
-    return EOD_OK;
+    return eod_encode_tmap("eod_write_mean", tmap, dtype, 3, feat, gdim, gstr, box, promo);
 }
 
 template <int C, bool kDry>
@@ -1186,10 +1098,7 @@ __device__ __forceinline__ void det_tile_masks(const int32_t *idx, const uint8_t
 // does the run starting at head bit p0 contain a sampled pixel?
 __device__ __forceinline__ bool det_run_sampled(unsigned heads, unsigned samps, int p0)
 {
-    const unsigned above = heads & ~((2u << p0) - 1u);
-    const int p1 = above ? (__ffs(above) - 1) : 32;
-    const unsigned m = samps & (0xffffffffu >> (32 - p1)) & (0xffffffffu << p0);
-    return m != 0;
+    return det_run_mask(heads & ~((2u << p0) - 1u), samps, p0) != 0;
 }
 
 __global__ void __launch_bounds__(256) det_tile_runs_kernel(const int32_t *__restrict__ idx, const uint8_t *__restrict__ samp,
