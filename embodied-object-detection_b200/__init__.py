@@ -8,7 +8,7 @@ from . import _lib, build, config, episodes, formats, fpn_fusion, geometry, memo
 from ._lib import EodError  # noqa: F401
 from .fpn_fusion import CustomRecurrentFPN, MemoryFusion  # noqa: F401
 from .geometry import Projector, compute_intrinsics, transform3d  # noqa: F401
-from .memory import EpisodeBatch, SpatialFeatureMemory  # noqa: F401
+from .memory import EpisodeBatch, HeightMaxBatch, SpatialFeatureMemory  # noqa: F401
 from .runner import EpisodeRunner, HostEpisodeProvider, LockStepSchedule  # noqa: F401
 
 __version__ = "0.1.0"

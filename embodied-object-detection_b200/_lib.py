@@ -47,6 +47,11 @@ SIGNATURES = {
     "eod_bilinear_lattice": [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P],
     "eod_write_max": [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int, c_int64, _P, _P, _P, _P, _P, _P],
     "eod_max_winner_list": [_P, c_int, c_int64, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, _P],
+    "eod_heightmax_contest_depth": [_P, c_int, c_double, _P, _P, c_int, c_int, c_int, c_float, c_float, c_float, c_float, c_float, c_int, c_int,
+                                    c_int, c_float, c_int, _P, _P, _P, c_int64, _P, _P, _P],
+    "eod_heightmax_contest_planes": [_P, _P, _P, c_int, c_int, c_int, c_int, c_int64, _P, _P, _P, c_int64, _P, _P, _P],
+    "eod_heightmax_update": [_P, c_int, c_int, c_int, c_int, c_int, c_int64, _P, c_int64, _P, _P, _P, _P, _P, _P, _P, c_int64, _P, _P],
+    "eod_heightmax_reset": [_P, c_int, c_int64, c_int, _P, _P, _P, _P],
     "eod_linear_rows": [_P, c_int64, c_int64, _P, _P, c_int64, c_int64, _P, c_float, c_int, _P, c_int, c_int, _P, c_int64, _P, _P],
     "eod_read_pool": [_P, c_int, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int64, _P, _P, _P, _P],
     "eod_normalize_memory": [_P, _P, c_int64, c_int, _P, c_int, _P],

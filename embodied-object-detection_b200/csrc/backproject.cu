@@ -5,28 +5,11 @@
 //   x_scale = ((u + 0.5) - cx) / fx         IEEE divide          (core.py:107)
 //   world_r = fma(T3,1, fma(T2,z, fma(T1,y, T0*x)))              (core.py:175, torch.bmm K=4 on CPU)
 //   q       = rint((world - shift0 - shift1) / cell)             (core.py:220, build_memory_data.py:135-136)
-// All arithmetic uses explicit _rn intrinsics so nvcc can neither contract nor reassociate.
-#include "eod_common.cuh"
+// All arithmetic uses explicit _rn intrinsics so nvcc can neither contract nor reassociate (the per-pixel helpers live in
+// backproject.cuh, shared with the height-max contest of write_max.cu).
+#include "backproject.cuh"
 
 namespace {
-
-// build_memory_data.py:136-142 / robot_demo.py:527-530: q.round().long() and THEN the clip.  On the x86 hosts the reference runs on,
-// float -> int64 of NaN, +-inf or anything beyond +-2^63 yields INT64_MIN, which clips to cell 0; finite values clip as usual.
-// (The outlier mask of core.py:253-256 compares the rounded FLOATS, so it needs no such rule.)
-__device__ __forceinline__ bool q_overflows(float q) { return !(fabsf(q) < 9.223372036854775808e18f); }
-__device__ __forceinline__ int clip_cell(float q, int n)
-{
-    return q_overflows(q) ? 0 : (int)fminf(fmaxf(q, 0.0f), (float)(n - 1));
-}
-
-// Depth as the sensor delivers it: fp32 metres (habitat: build_data.py:205-207), or uint16 sensor units divided by `depth_div`
-// (robot_demo.py:515: depth_image / 1000 - numpy true division in fp64, then torch.FloatTensor rounds to fp32).
-template <bool U16>
-__device__ __forceinline__ float load_depth(const void *depth, double div, size_t g)
-{
-    if (U16) return __double2float_rn(__ddiv_rn((double)__ldg(reinterpret_cast<const uint16_t *>(depth) + g), div));
-    return __ldg(reinterpret_cast<const float *>(depth) + g);
-}
 
 struct BackprojectParams {
     const void *depth;
@@ -59,8 +42,8 @@ __global__ void __launch_bounds__(256) backproject_quantize_kernel(const Backpro
     const float *T = P.pose + 12 * e;       // uniform across the block: served by the constant/L1 path
     const float *S = P.shifts + 6 * e;
 
-    const float xs = __fdiv_rn(__fsub_rn(__fadd_rn((float)u, 0.5f), P.cx), P.fx);
-    const float ys = __fdiv_rn(__fsub_rn(__fadd_rn((float)v, 0.5f), P.cy), P.fy);
+    const float xs = pixel_scale(u, P.cx, P.fx);
+    const float ys = pixel_scale(v, P.cy, P.fy);
     const size_t g = (size_t)e * HW + p;
     const float z = load_depth<U16>(P.depth, P.depth_div, g);
     const float x = __fmul_rn(z, xs);
@@ -70,7 +53,7 @@ __global__ void __launch_bounds__(256) backproject_quantize_kernel(const Backpro
 #pragma unroll
     for (int r = 0; r < 3; ++r) {
         const float t0 = __ldg(T + 4 * r), t1 = __ldg(T + 4 * r + 1), t2 = __ldg(T + 4 * r + 2), t3 = __ldg(T + 4 * r + 3);
-        w[r] = __fmaf_rn(t3, 1.0f, __fmaf_rn(t2, z, __fmaf_rn(t1, y, __fmul_rn(t0, x))));
+        w[r] = pose_row(t0, t1, t2, t3, x, y, z);
     }
     const float p0x = __fsub_rn(w[0], __ldg(S + 0)), p0y = __fsub_rn(w[1], __ldg(S + 1)), p0z = __fsub_rn(w[2], __ldg(S + 2));
     if (P.world) {
@@ -78,17 +61,15 @@ __global__ void __launch_bounds__(256) backproject_quantize_kernel(const Backpro
         o[0] = p0x; o[1] = p0y; o[2] = p0z;
     }
     const float p1x = __fsub_rn(p0x, __ldg(S + 3)), p1y = __fsub_rn(p0y, __ldg(S + 4)), p1z = __fsub_rn(p0z, __ldg(S + 5));
-    const float qx = rintf(__fdiv_rn(p1x, P.cell));
-    const float qz = rintf(__fdiv_rn(p1z, P.cell));
+    const float qx = quantize(p1x, P.cell);
+    const float qz = quantize(p1z, P.cell);
     if (P.q2) {
         P.q2[2 * g] = (int32_t)qx;
         P.q2[2 * g + 1] = (int32_t)qz;
     }
     if (P.outlier) {
         const float thr = __fadd_rn(__ldg(T + 7), P.z_clip);
-        const bool out = (qx >= (float)P.map_w) || (qz >= (float)P.map_h) || (qx < 0.0f) || (qz < 0.0f) ||
-                         (p1y > thr) || (z == 0.0f);
-        P.outlier[g] = out ? 1 : 0;
+        P.outlier[g] = is_outlier(qx, qz, p1y, thr, z, P.map_w, P.map_h) ? 1 : 0;
     }
     if (P.height) P.height[g] = p1y;
     if (P.idx) {
@@ -116,7 +97,7 @@ __global__ void __launch_bounds__(256) backproject_quantize_vec4_kernel(const Ba
     for (int i = 0; i < 12; ++i) t[i] = __ldg(T + i);
 #pragma unroll
     for (int i = 0; i < 6; ++i) sh[i] = __ldg(S + i);
-    const float ys = __fdiv_rn(__fsub_rn(__fadd_rn((float)v, 0.5f), P.cy), P.fy);
+    const float ys = pixel_scale(v, P.cy, P.fy);
     const float thr = __fadd_rn(t[7], P.z_clip);
     const size_t g = (size_t)e * HW + p;
     float zz[4];
@@ -135,23 +116,14 @@ __global__ void __launch_bounds__(256) backproject_quantize_vec4_kernel(const Ba
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
         const float z = zz[k];
-        const float xs = __fdiv_rn(__fsub_rn(__fadd_rn((float)(u0 + k), 0.5f), P.cx), P.fx);
-        const float x = __fmul_rn(z, xs);
-        const float y = __fmul_rn(z, ys);
-        float w[3];
-#pragma unroll
-        for (int r = 0; r < 3; ++r)
-            w[r] = __fmaf_rn(t[4 * r + 3], 1.0f, __fmaf_rn(t[4 * r + 2], z, __fmaf_rn(t[4 * r + 1], y, __fmul_rn(t[4 * r], x))));
-        const float p0x = __fsub_rn(w[0], sh[0]), p0y = __fsub_rn(w[1], sh[1]), p0z = __fsub_rn(w[2], sh[2]);
-        w12[3 * k] = p0x; w12[3 * k + 1] = p0y; w12[3 * k + 2] = p0z;
-        const float p1x = __fsub_rn(p0x, sh[3]), p1y = __fsub_rn(p0y, sh[4]), p1z = __fsub_rn(p0z, sh[5]);
-        const float qx = rintf(__fdiv_rn(p1x, P.cell));
-        const float qz = rintf(__fdiv_rn(p1z, P.cell));
+        float p0[3], p1[3];
+        world_point(z, pixel_scale(u0 + k, P.cx, P.fx), ys, t, sh, p0, p1);
+        w12[3 * k] = p0[0]; w12[3 * k + 1] = p0[1]; w12[3 * k + 2] = p0[2];
+        const float qx = quantize(p1[0], P.cell);
+        const float qz = quantize(p1[2], P.cell);
         q2v[2 * k] = (int32_t)qx; q2v[2 * k + 1] = (int32_t)qz;
-        const bool out = (qx >= (float)P.map_w) || (qz >= (float)P.map_h) || (qx < 0.0f) || (qz < 0.0f) ||
-                         (p1y > thr) || (z == 0.0f);
-        out4 |= (out ? 1u : 0u) << (8 * k);
-        h4[k] = p1y;
+        out4 |= (is_outlier(qx, qz, p1[1], thr, z, P.map_w, P.map_h) ? 1u : 0u) << (8 * k);
+        h4[k] = p1[1];
         const int ix = clip_cell(qx, P.map_w), iz = clip_cell(qz, P.map_h);
         idx4[k] = P.order == EOD_ORDER_XZ ? ix * P.map_h + iz : iz * P.map_w + ix;
     }
@@ -203,10 +175,7 @@ __global__ void __launch_bounds__(256) quantize_world_kernel(const float *__rest
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const float x = __ldg(world + 3 * i), z = __ldg(world + 3 * i + 2);
-    const float qx = rintf(__fdiv_rn(__fsub_rn(x, sx), cell));
-    const float qz = rintf(__fdiv_rn(__fsub_rn(z, sz), cell));
-    const int ix = clip_cell(qx, map_w), iz = clip_cell(qz, map_h);
-    idx[i] = order == EOD_ORDER_XZ ? ix * map_h + iz : iz * map_w + ix;
+    idx[i] = flat_cell(quantize(__fsub_rn(x, sx), cell), quantize(__fsub_rn(z, sz), cell), map_w, map_h, order);
 }
 
 }  // namespace

@@ -45,6 +45,25 @@ static inline int eod_ensure_dyn_smem(F func, int bytes, unsigned long long *don
 
 // ---- device helpers -------------------------------------------------------------------------------
 
+// feature element type: fp32, or bf16 / fp16 widened exactly to fp32 before any arithmetic
+enum { FEAT_F32 = 0, FEAT_BF16 = 1, FEAT_F16 = 2 };
+template <int F> struct FeatElem { using T = uint16_t; };
+template <> struct FeatElem<FEAT_F32> { using T = float; };
+template <int F>
+__device__ __forceinline__ float widen1(typename FeatElem<F>::T x)
+{
+    if constexpr (F == FEAT_F32) return x;
+    else if constexpr (F == FEAT_BF16) return __uint_as_float((uint32_t)x << 16);
+    else return __half2float(__ushort_as_half(x));
+}
+// the two 16-bit elements of a 32-bit word (element 0 in the low half), widened exactly
+template <int F>
+__device__ __forceinline__ float2 widen2(uint32_t w)
+{
+    if constexpr (F == FEAT_BF16) return make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u));
+    else return __half22float2(*reinterpret_cast<const __half2 *>(&w));
+}
+
 // 128-bit fp32 reduction to global memory (sm_90+): one L2 atomic transaction for four floats.
 __device__ __forceinline__ void red_add_v4(float *addr, float a, float b, float c, float d)
 {

@@ -7,6 +7,8 @@ Dataset names are the reference's, typos included, so files written by either si
                          detection_data, segmentation_data (SMNet/build_data.py:275-286)
   <out>/memory/<seq>     semmap i32 (cells,) | impicit_memory [sic] f32 (cells,512) | observations f32 (cells,)
                          (detic/modeling/meta_arch/custom_rcnn.py:527-530; re-read by SMNet/loader.py:216-223)
+  <out>/heightmax/<seq>  state f32 (cells,C) | observed u8 (cells,) | height_map f32 (cells,): the SMNet encoder's map after the
+                         episode's last frame, what its decoder takes (EpisodeRunner(regime="heightmax"))
 Containers: HDF5 through h5py when it is importable (it is not in this image), otherwise ``.npz`` with the same
 keys.  ``open_store`` picks by what exists on disk; a missing or unreadable file RAISES (the reference's silent
 zero-memory fallback, loader.py:208-211, is deliberately not reproduced).
@@ -92,6 +94,26 @@ def load_memory(path: str) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
     if missing:
         raise StoreError(f"{path}: missing datasets {missing}")
     return d["semmap"] + 1, d["impicit_memory"], d["observations"]
+
+
+# ---- height-max memory after an episode's last frame -------------------------------------------------------------
+HEIGHTMAX_KEYS = ("state", "observed", "height_map")
+
+
+def save_heightmax(path: str, state, observed, height_map, container: Optional[str] = None) -> str:
+    """{state float32 (cells,C), observed uint8 (cells,), height_map float32 (cells,)}; tensors are moved to the host here."""
+    to_np = lambda t: t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
+    return write_store(path, {"state": to_np(state).astype(np.float32), "observed": to_np(observed).astype(np.uint8),
+                              "height_map": to_np(height_map).astype(np.float32)}, container)
+
+
+def load_heightmax(path: str) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """-> (state, observed, height_map) as save_heightmax wrote them."""
+    d = open_store(path)
+    missing = [k for k in HEIGHTMAX_KEYS if k not in d]
+    if missing:
+        raise StoreError(f"{path}: missing datasets {missing}")
+    return d["state"], d["observed"], d["height_map"]
 
 
 # ---- memory_data (build_memory_data.py:108-153) ------------------------------------------------------------------

@@ -1,11 +1,15 @@
 """Spatial feature memory: grid state + write/read on the B200 kernels.
 
-Two host-side objects sit above the C ABI:
+Three host-side objects sit above the C ABI:
 
 ``EpisodeBatch``
     E independent episodes advanced in lock step (BASELINE config 2 "batched x64"): one launch per stage covers
     all E grids.  This is the throughput path the bench measures:
         project (depth, pose -> cell indices) -> read (pooled fp16 levels) -> write (features -> grid).
+
+``HeightMaxBatch``
+    E episodes of the SMNet height-max memory in lock step (BASELINE configs[2]): per frame a contest of the frame's pixels
+    for the highest point of every cell and the 'replace' update of the cells it raised.
 
 ``SpatialFeatureMemory``
     Single-episode mirror of the memory methods of ``CustomRCNNRecurrent``
@@ -513,6 +517,83 @@ class GraphedDetections:
         self.graph.replay()
         b._sync_next = True                                 # the next eager step must not run ahead of this replay (same planes)
         return self.levels
+
+
+class HeightMaxBatch:
+    """E episodes of the SMNet height-max memory (bytecode-only SMNet.encode, SURVEY 8a row A7') in lock step: BASELINE configs[2].
+
+    Per episode: ``state`` (cells, C_mem) f32, ``height_map`` (cells) f32 = highest inlier height + 1000 seen so far (0 before the
+    first), ``observed`` (cells) u8.  A frame is the contest of its [::pix_stride, ::pix_stride] pixels for the highest point of every
+    cell - geometry from depth (computed in registers) or from precomputed height / idx / outlier planes - and the update of the cells
+    it raised: the winner pixel's feature row is copied into ``state`` ('replace' without a layer), or, with ``linlayer=(weight (C_mem, C)
+    f32, bias (C_mem,) | None)``, ``state[cell] = weight @ row + bias`` on the tensor cores (fp32 features only).  Results equal
+    ``ops.backproject_quantize`` + ``ops.write_max`` (``write_max_linear``) over the same frames bit for bit.
+
+    ``feat`` is (E,C,H,W) or (E,H,W,C) in the dtype of ``layout`` (LAYOUT_CHW / _HWC fp32, the _BF16 / _F16 variants widened exactly).
+    Everything is ordered on the caller's stream, inputs included."""
+
+    def __init__(self, n_episodes: int, map_w: int, map_h: int, channels: int, height: int = 480, width: int = 640,
+                 device: torch.device = torch.device("cuda"), layout: int = LAYOUT_CHW, linlayer: Optional[Tuple[torch.Tensor, Optional[torch.Tensor]]] = None,
+                 pix_stride: int = 1, order: int = ORDER_ZX, z_clip: float = 0.5, depth_div: float = 1000.0):
+        if torch.device(device).type != "cuda":
+            raise EodError("HeightMaxBatch needs a CUDA device (no CPU fallback)")
+        if linlayer is not None and layout not in (LAYOUT_CHW, LAYOUT_HWC):
+            raise EodError("HeightMaxBatch: the linlayer update takes fp32 features (LAYOUT_CHW / LAYOUT_HWC)")
+        self.E, self.map_w, self.map_h, self.C, self.H, self.W = n_episodes, map_w, map_h, channels, height, width
+        self.n_cells = map_w * map_h
+        self.device, self.layout, self.pix_stride, self.order, self.z_clip, self.depth_div = torch.device(device), layout, pix_stride, order, z_clip, depth_div
+        self.linlayer = None
+        c_mem = channels
+        if linlayer is not None:
+            weight, bias = linlayer
+            if weight.dim() != 2 or weight.shape[1] != channels:
+                raise ValueError(f"linlayer weight must be (C_mem, {channels})")
+            self.linlayer = (weight.to(self.device, torch.float32).contiguous(),
+                             None if bias is None else bias.to(self.device, torch.float32).contiguous())
+            c_mem = weight.shape[0]
+        z = dict(device=self.device)
+        self.state = torch.zeros((self.E, self.n_cells, c_mem), dtype=torch.float32, **z)
+        self.height_map = torch.zeros((self.E, self.n_cells), dtype=torch.float32, **z)
+        self.observed = torch.zeros((self.E, self.n_cells), dtype=torch.uint8, **z)
+        lattice = -(-height // pix_stride) * -(-width // pix_stride)
+        self.scratch = ops.HeightMaxScratch(self.E, self.n_cells, lattice, self.device)
+
+    def reset(self, mask: Optional[torch.Tensor] = None) -> None:
+        """memory reset of every episode, or - ``mask`` (E) i32 - of the slots with mask[e] != 0 only."""
+        if mask is None:
+            mask = torch.ones((self.E,), dtype=torch.int32, device=self.device)
+        ops.heightmax_reset(self.height_map, self.observed, self.state, mask)
+
+    def step(self, feat: torch.Tensor, *, depth: Optional[torch.Tensor] = None, pose: Optional[torch.Tensor] = None,
+             shifts: Optional[torch.Tensor] = None, intr: Optional[Sequence[float]] = None, cell: Optional[float] = None,
+             height: Optional[torch.Tensor] = None, idx: Optional[torch.Tensor] = None, outlier: Optional[torch.Tensor] = None,
+             active: Optional[torch.Tensor] = None, reset_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """One frame of every episode.  Geometry: depth (E,H,W) f32 metres or uint16 (/ depth_div) + pose (E,12) + shifts (E,6) + intr +
+        cell, OR precomputed planes height (E,H,W) f32 + idx (E,H,W) i32 cell ids in [0, cells) + outlier (E,H,W) u8 | None.
+        active (E) i32: slots with active <= 0 read nothing and keep their state; reset_mask (E) i32: those slots are cleared before
+        the frame.  Returns the device count (1,) i32 of cells raised this frame over all episodes (valid until the next step)."""
+        geo = depth if depth is not None else height
+        if geo is None or tuple(geo.shape) != (self.E, self.H, self.W):
+            raise ValueError(f"HeightMaxBatch.step: depth or height of shape {(self.E, self.H, self.W)} is required")
+        # features are checked before the contest: a refused update would leave the frame's keys in the scratch
+        if ops._feat_hw(feat, self.layout, self.E, self.C, "HeightMaxBatch.step") != (self.H, self.W):
+            raise ValueError(f"HeightMaxBatch.step: feat must cover H={self.H}, W={self.W}")
+        if self.C % 4 or self.state.shape[2] % 4 or feat.data_ptr() % 16 or self.state.data_ptr() % 16:
+            raise EodError("HeightMaxBatch.step: feature and state rows need C % 4 == 0 and 16-byte aligned tensors")
+        if reset_mask is not None:
+            ops.heightmax_reset(self.height_map, self.observed, self.state, reset_mask)
+        if depth is not None:
+            if height is not None or idx is not None or outlier is not None:
+                raise ValueError("HeightMaxBatch.step: give depth + pose + shifts + intr + cell OR height + idx (+ outlier), not both")
+            if pose is None or shifts is None or intr is None or cell is None:
+                raise ValueError("HeightMaxBatch.step: depth needs pose, shifts, intr and cell")
+            ops.heightmax_contest_depth(depth, pose, shifts, intr, cell, self.map_w, self.map_h, self.scratch, active, self.pix_stride,
+                                        self.order, self.z_clip, self.depth_div)
+        else:
+            if idx is None:
+                raise ValueError("HeightMaxBatch.step: height needs idx")
+            ops.heightmax_contest_planes(height, idx, outlier, self.scratch, active, self.pix_stride)
+        return ops.heightmax_update(feat, self.layout, self.scratch, self.height_map, self.observed, self.state, self.linlayer)
 
 
 class SpatialFeatureMemory:

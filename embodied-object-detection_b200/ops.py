@@ -30,7 +30,8 @@ _LAUNCHES = {"eod_backproject_quantize": 1, "eod_backproject_quantize_u16": 1, "
              "eod_write_mean_det_layout": 9,
              "eod_finalize_counts": 1, "eod_box_to_image_features": 1, "eod_masks_observed": 1, "eod_paste_masks": 1, "eod_write_objects_pasted": 1, "eod_bilinear_lattice": 1, "eod_write_objects": 1, "eod_flush_slots": 2, "eod_write_max": 2, "eod_read_pool": 2,
              "eod_fuse": 1, "eod_project_split_weights": 1, "eod_project_fuse": 1, "eod_project_fuse_levels": 1, "eod_normalize_memory": 1, "eod_reset_touched": 1, "eod_semmap_update": 1, "eod_semmap_decode": 2,
-             "eod_reset_episodes": 1, "eod_refresh_norm16": 1, "eod_check_indices": 1, "eod_remap_indices": 1, "eod_max_winner_list": 1, "eod_linear_rows": 1, "eod_read_roi": 1}
+             "eod_reset_episodes": 1, "eod_refresh_norm16": 1, "eod_check_indices": 1, "eod_remap_indices": 1, "eod_max_winner_list": 1, "eod_linear_rows": 1, "eod_read_roi": 1,
+             "eod_heightmax_contest_depth": 1, "eod_heightmax_contest_planes": 1, "eod_heightmax_update": 1, "eod_heightmax_reset": 1}
 
 
 def _call(name: str, *args) -> None:
@@ -571,6 +572,122 @@ def max_winner_list(arg_pix: torch.Tensor, H: int, W: int, C: int, layout: int =
     _call("eod_max_winner_list", arg_pix.data_ptr(), E, n_cells, int(H), int(W), int(C), int(layout), src.data_ptr(), dst.data_ptr(),
           count.data_ptr(), cap, _stream())
     return src, dst, count
+
+
+class HeightMaxScratch:
+    """Per-frame scratch of the lock-step height-max write (eod_heightmax_*), all-zero between frames (the update leaves it so):
+    key64 (E,cells) i64 packed keys, cell_list (E,list_cap) i32 the cells a frame touched, n_list (E,2) i32, and ``raised`` (1,) i32:
+    the number of cells the last update raised (device)."""
+
+    def __init__(self, n_episodes: int, n_cells: int, lattice: int, device: torch.device):
+        self.E, self.n_cells, self.list_cap = int(n_episodes), int(n_cells), int(min(n_cells, lattice))
+        self.key64 = torch.zeros((self.E, self.n_cells), dtype=torch.int64, device=device)
+        self.cell_list = torch.zeros((self.E, self.list_cap), dtype=torch.int32, device=device)
+        self.n_list = torch.zeros((self.E, 2), dtype=torch.int32, device=device)
+        self.raised = torch.zeros((1,), dtype=torch.int32, device=device)
+
+    def args(self) -> tuple:
+        return self.key64.data_ptr(), self.cell_list.data_ptr(), self.list_cap, self.n_list.data_ptr(), self.raised.data_ptr()
+
+
+def _active(active: Optional[torch.Tensor], E: int) -> Optional[int]:
+    if active is None:
+        return None
+    _dev(active, torch.int32, "active")
+    if active.numel() != E:
+        raise ValueError("active must hold one int32 per episode")
+    return active.data_ptr()
+
+
+def heightmax_contest_depth(depth: torch.Tensor, pose: torch.Tensor, shifts: torch.Tensor, intr: Sequence[float], cell: float, map_w: int,
+                            map_h: int, scratch: HeightMaxScratch, active: Optional[torch.Tensor] = None, pix_stride: int = 1,
+                            order: int = ORDER_ZX, z_clip: float = 0.5, depth_div: float = 1000.0) -> None:
+    """Height-max contest of one frame with the geometry computed from depth in registers (no idx / outlier / height planes):
+    depth (E,H,W) f32 metres or uint16 (/ depth_div), pose (E,12), shifts (E,6); active (E) i32 | None."""
+    raw = depth.dtype == torch.uint16
+    _dev(depth, torch.uint16 if raw else torch.float32, "depth"), _dev(pose, torch.float32, "pose"), _dev(shifts, torch.float32, "shifts")
+    E, H, W = depth.shape
+    if pose.shape != (E, 12) or shifts.shape != (E, 6) or scratch.E != E or scratch.n_cells != map_w * map_h:
+        raise ValueError("heightmax_contest_depth: pose (E,12), shifts (E,6) and a scratch of E episodes x map_w*map_h cells")
+    fx, fy, cx, cy = (float(v) for v in intr)
+    _call("eod_heightmax_contest_depth", depth.data_ptr(), int(raw), float(depth_div), pose.data_ptr(), shifts.data_ptr(), E, H, W, fx, fy, cx, cy,
+          float(cell), int(map_w), int(map_h), int(order), float(z_clip), int(pix_stride), _active(active, E), *scratch.args(), _stream())
+
+
+def heightmax_contest_planes(height: torch.Tensor, idx: torch.Tensor, outlier: Optional[torch.Tensor], scratch: HeightMaxScratch,
+                             active: Optional[torch.Tensor] = None, pix_stride: int = 1) -> None:
+    """Height-max contest of one frame from precomputed planes (create_coco_mp3d.py:157-165): height (E,H,W) f32, idx (E,H,W) i32 cell
+    ids in [0, cells), outlier (E,H,W) u8 / bool | None; active (E) i32 | None."""
+    _dev(height, torch.float32, "height"), _dev(idx, torch.int32, "idx")
+    E, H, W = height.shape
+    if tuple(idx.shape) != (E, H, W) or scratch.E != E:
+        raise ValueError("heightmax_contest_planes: height and idx (E,H,W) and a scratch of E episodes")
+    if outlier is not None:
+        if outlier.dtype == torch.bool:
+            outlier = outlier.view(torch.uint8)
+        _dev(outlier, torch.uint8, "outlier")
+        if tuple(outlier.shape) != (E, H, W):
+            raise ValueError("heightmax_contest_planes: outlier must be (E,H,W)")
+    _call("eod_heightmax_contest_planes", height.data_ptr(), idx.data_ptr(), _ptr(outlier), E, H, W, int(pix_stride), scratch.n_cells,
+          _active(active, E), *scratch.args(), _stream())
+
+
+def _feat_hw(feat: torch.Tensor, layout: int, E: int, C: int, what: str) -> Tuple[int, int]:
+    """(H, W) of (E,H,W,C) channels-last or (E,C,H,W) features; EodError if the dtype does not belong to the layout."""
+    dtype = LAYOUT_DTYPE.get(int(layout), torch.float32)
+    if feat.dtype != dtype:
+        raise EodError(f"{what}: layout {int(layout)} takes {dtype} features, got {feat.dtype}")
+    _dev(feat, dtype, "feat")
+    hwc = int(layout) in (LAYOUT_HWC, LAYOUT_HWC_BF16, LAYOUT_HWC_F16)
+    if feat.dim() != 4 or feat.shape[0] != E or feat.shape[3 if hwc else 1] != C:
+        raise ValueError(f"{what}: feat must be {'(E,H,W,C)' if hwc else '(E,C,H,W)'} with E={E}, C={C}, got {tuple(feat.shape)}")
+    return (feat.shape[1], feat.shape[2]) if hwc else (feat.shape[2], feat.shape[3])
+
+
+def heightmax_update(feat: torch.Tensor, layout: int, scratch: HeightMaxScratch, height_map: torch.Tensor, observed: torch.Tensor,
+                     state: torch.Tensor, linlayer: Optional[Tuple[torch.Tensor, Optional[torch.Tensor]]] = None) -> torch.Tensor:
+    """Update of the cells the frame's contest listed: height_map (E,cells) f32 and observed (E,cells) u8 of the raised cells, and
+    state (E,cells,C_mem) f32 rows := the winners' feature rows (copy) or ``linlayer(feature rows)`` with linlayer = (weight (C_mem,C)
+    f32, bias (C_mem,) | None) on the tensor cores (eod_linear_rows; fp32 features only).  feat (E,C,H,W) [CHW layouts] or (E,H,W,C)
+    [HWC layouts] in the layout's dtype.  Returns the device count of raised cells (scratch.raised, valid until the next contest)."""
+    _dev(height_map, torch.float32, "height_map"), _dev(observed, torch.uint8, "observed"), _dev(state, torch.float32, "state")
+    E, n_cells = height_map.shape
+    if (E, n_cells) != (scratch.E, scratch.n_cells) or tuple(observed.shape) != (E, n_cells) or state.dim() != 3 or state.shape[:2] != (E, n_cells):
+        raise ValueError("heightmax_update: height_map / observed (E,cells), state (E,cells,C) matching the scratch")
+    if linlayer is None:
+        C = state.shape[2]
+        H, W = _feat_hw(feat, layout, E, C, "heightmax_update")
+        _call("eod_heightmax_update", feat.data_ptr(), int(layout), E, C, H, W, n_cells, scratch.cell_list.data_ptr(), scratch.list_cap,
+              scratch.n_list.data_ptr(), scratch.key64.data_ptr(), height_map.data_ptr(), observed.data_ptr(), state.data_ptr(), None, None, 0,
+              scratch.raised.data_ptr(), _stream())
+        return scratch.raised
+    weight, bias = linlayer
+    if int(layout) not in (LAYOUT_CHW, LAYOUT_HWC):
+        raise EodError("heightmax_update: the linlayer update takes fp32 features (LAYOUT_CHW / LAYOUT_HWC)")
+    c_in = weight.shape[1]
+    H, W = _feat_hw(feat, layout, E, c_in, "heightmax_update")
+    if state.shape[2] != weight.shape[0]:
+        raise ValueError("heightmax_update: state channels must equal weight.shape[0]")
+    cap = E * scratch.list_cap
+    if getattr(scratch, "_winners", None) is None or scratch._winners[0].numel() != cap:
+        scratch._winners = (torch.empty((cap,), dtype=torch.int64, device=feat.device), torch.empty((cap,), dtype=torch.int64, device=feat.device))
+    src, dst = scratch._winners
+    _call("eod_heightmax_update", None, int(layout), E, c_in, H, W, n_cells, scratch.cell_list.data_ptr(), scratch.list_cap,
+          scratch.n_list.data_ptr(), scratch.key64.data_ptr(), height_map.data_ptr(), observed.data_ptr(), None, src.data_ptr(), dst.data_ptr(),
+          cap, scratch.raised.data_ptr(), _stream())
+    linear_rows(feat, weight, bias, 1.0, out=state.view(-1, state.shape[2]), a_off=src, a_k_stride=1 if int(layout) == LAYOUT_HWC else H * W,
+                m_count=scratch.raised, n_rows=cap, y_dst=dst)
+    return scratch.raised
+
+
+def heightmax_reset(height_map: torch.Tensor, observed: torch.Tensor, state: torch.Tensor, mask: torch.Tensor) -> None:
+    """Per-slot reset of the height-max state: the episodes with mask[e] != 0 get height_map = 0, observed = 0 and zero state rows."""
+    _dev(height_map, torch.float32, "height_map"), _dev(observed, torch.uint8, "observed"), _dev(state, torch.float32, "state")
+    _dev(mask, torch.int32, "mask")
+    E, n_cells, C = state.shape
+    if mask.numel() != E or tuple(height_map.shape) != (E, n_cells) or tuple(observed.shape) != (E, n_cells):
+        raise ValueError("heightmax_reset: mask (E), height_map / observed (E,cells), state (E,cells,C)")
+    _call("eod_heightmax_reset", mask.data_ptr(), E, n_cells, C, height_map.data_ptr(), observed.data_ptr(), state.data_ptr(), _stream())
 
 
 def read_pool(table: torch.Tensor, counts: Optional[torch.Tensor], idx: torch.Tensor, out: Optional[Sequence[torch.Tensor]] = None):

@@ -20,6 +20,9 @@ R resident grid slots of one ``EpisodeBatch``; a slot that finishes its stream t
 keeps at most R grids resident however many episodes there are (BASELINE configs[4]: 512 episodes of 1000x1000x512
 grids in waves of R).  Slots without work are masked out (``active``).
 
+``regime="heightmax"`` runs the same schedule over a ``HeightMaxBatch`` (the SMNet height-max memory, BASELINE configs[2]): no read,
+and each episode's map is dumped after its LAST frame (SMNet's encoder hands the finished map to its decoder).
+
 ``LockStepSchedule`` is the host-only part (pure Python, tested without a GPU); ``EpisodeRunner`` issues the launches.
 """
 from __future__ import annotations
@@ -144,6 +147,7 @@ class HostEpisodeProvider:
     contract) plus whatever feeds the write.  Per frame: ``sequence_name``, ``memory_reset``, and
         geometry : ``proj_indices`` (H,W[,1]) int32  (memory_data/*.h5)   or   ``depth`` (H,W) f32 + ``pose`` (12,) f32
         write    : ``feat`` (C,H,W) f32 [dense]   or   ``box_features`` (K,C), ``mask_probs`` (K,S,S), ``boxes`` (K,4) [detections]
+        height-max planes (create_coco_mp3d.py:157-165), with ``proj_indices``: ``height`` (H,W) f32 and ``outlier`` (H,W) bool / u8
     ``shifts``: per episode (6,) f32 (world_shift_origin xyz, map_world_shift xyz), needed with depth.
     ``feat_dtype``: the dtype ``feat`` is staged in - torch.bfloat16 / torch.float16 feed the 16-bit layouts of ``EpisodeRunner``
     (LAYOUT_CHW_BF16 / _F16 for (C,H,W) frames, LAYOUT_HWC_BF16 / _F16 for (H,W,C) ones) at half the bytes; a frame's ``feat`` may
@@ -191,6 +195,9 @@ class HostEpisodeProvider:
                 put("depth", s, fr["depth"], np.asarray(fr["depth"]).shape, torch.float32)
                 put("pose", s, fr["pose"], (12,), torch.float32)
                 put("shifts", s, self.shifts[a[0]], (6,), torch.float32)
+            for key, dtype in (("height", torch.float32), ("outlier", torch.uint8)):
+                if key in fr:
+                    put(key, s, fr[key], np.asarray(fr[key]).shape, dtype)
             if "feat" in fr:
                 f = fr["feat"]
                 put("feat", s, f, tuple(f.shape) if torch.is_tensor(f) else np.asarray(f).shape, self.feat_dtype)
@@ -230,6 +237,10 @@ class EpisodeRunner:
     ``variant = WRITE_DET``: the dense write is the deterministic one, so a run reproduces bit for bit whatever the slot count and the
     wave a stream lands in (size its workspace with ``batch.det_runs_per_episode``); the detection regime has no deterministic write
     and raises EodError.
+    ``regime = "heightmax"``: the slots are a ``HeightMaxBatch`` (``layout`` and ``linlayer`` = (weight, bias) | None as it takes them);
+    frames carry ``feat`` and depth + pose or ``proj_indices`` + ``height`` (+ ``outlier``); anything else staged (detections, an index
+    plane without heights) raises EodError.  There is no read, so ``on_levels`` is not called; ``save_dir`` receives
+    <save_dir>/heightmax/<name> (``formats.save_heightmax``) after each episode's last frame.
     """
 
     def __init__(self, provider, map_w: int, map_h: int, channels: int, n_slots: int, *, height: int = 480, width: int = 640,
@@ -237,16 +248,24 @@ class EpisodeRunner:
                  intr: Optional[Sequence[float]] = None, cell: float = 0.2, order: int = ORDER_ZX, layout: int = LAYOUT_CHW,
                  save_dir: Optional[str] = None, zs_weight: Optional[torch.Tensor] = None, obs_score_thresh: float = 0.4,
                  n_semmap_classes: int = 20, sample_stride: int = 8, mask_thresh: float = 0.5, pipeline: bool = True,
-                 variant: int = WRITE_AUTO):
-        from .memory import EpisodeBatch
+                 variant: int = WRITE_AUTO, regime: str = "mean", linlayer=None):
+        from .memory import EpisodeBatch, HeightMaxBatch
         if test_type not in ("default", "episodic", "longterm"):
             raise ValueError(f"unknown TEST_TYPE {test_type!r}")           # detic/config.py:74
+        if regime not in ("mean", "heightmax"):
+            raise ValueError(f"unknown regime {regime!r} (mean | heightmax)")
+        if regime == "heightmax" and variant != WRITE_AUTO:
+            raise ValueError("variant selects the mean write; the height-max regime has one update")
+        self.regime = regime
         self.provider, self.test_type, self.device = provider, test_type, torch.device(device)
         n = provider.n_episodes
         self.schedule = LockStepSchedule([provider.n_frames(i) for i in range(n)],
                                          [provider.n_frames(i) > 0 and provider.reset_flag(i, 0) for i in range(n)], n_slots, rank, world)
-        self.batch = EpisodeBatch(n_slots, map_w, map_h, channels, height, width, self.device, layout=layout, variant=variant, pipeline=pipeline)
-        self.batch.read_frozen = test_type == "longterm"
+        if regime == "heightmax":
+            self.batch = HeightMaxBatch(n_slots, map_w, map_h, channels, height, width, self.device, layout=layout, linlayer=linlayer, order=order)
+        else:
+            self.batch = EpisodeBatch(n_slots, map_w, map_h, channels, height, width, self.device, layout=layout, variant=variant, pipeline=pipeline)
+            self.batch.read_frozen = test_type == "longterm"
         self.intr, self.cell, self.order = intr, float(cell), order
         self.save_dir, self.sample_stride, self.mask_thresh = save_dir, sample_stride, mask_thresh
         self.zs_weight = None if zs_weight is None else zs_weight.to(self.device, torch.float32).contiguous()
@@ -275,6 +294,21 @@ class EpisodeRunner:
         formats.save_memory(path, self._semmap(s), self.batch.sums[s], self.batch.counts[s])
         self.stats["saved"] += 1
 
+    def _step_heightmax(self, inp: dict, active: torch.Tensor, reset_mask: Optional[torch.Tensor]) -> None:
+        other = [k for k in ("box_features", "mask_probs", "boxes", "n_obj") if k in inp]
+        if other or "feat" not in inp or ("idx" in inp and "height" not in inp):
+            raise EodError(f"height-max runner: a frame needs feat and depth + pose or proj_indices + height (+ outlier); staged: {sorted(inp)}")
+        if "idx" in inp:
+            geo = dict(height=inp["height"], idx=inp["idx"], outlier=inp.get("outlier"))
+        else:
+            geo = dict(depth=inp["depth"], pose=inp["pose"], shifts=inp["shifts"], intr=self.intr, cell=self.cell)
+        self.batch.step(inp["feat"], active=active, reset_mask=reset_mask, **geo)
+
+    def _save_heightmax(self, s: int, name: str) -> None:
+        b = self.batch
+        formats.save_heightmax(os.path.join(self.save_dir, "heightmax", name), b.state[s], b.observed[s], b.height_map[s])
+        self.stats["saved"] += 1
+
     def run(self, on_levels: Optional[Callable[[Step, List[torch.Tensor]], None]] = None, max_steps: Optional[int] = None) -> dict:
         """Process this rank's share of the dataset.  on_levels(step, levels): consumer hook, called after every frame-step
         with the three pooled fp16 levels (R,C,h,w) ordered on the caller's stream (idle slots hold stale values).
@@ -287,7 +321,7 @@ class EpisodeRunner:
                 if max_steps is not None and k >= max_steps:
                     break
                 reset = [r or (a is not None and self.provider.reset_flag(a[0], a[1])) for r, a in zip(step.reset, step.assign)]
-                refresh = [self.batch.read_frozen and (st or r) for st, r in zip(step.seq_start, reset)]
+                refresh = [getattr(b, "read_frozen", False) and (st or r) for st, r in zip(step.seq_start, reset)]
                 self._masks.next()
                 pin, dev = self._masks.buf("masks", (3, self.R), torch.int32)
                 pin.copy_(torch.tensor([[int(a is not None) for a in step.assign], [int(r) for r in reset], [int(r) for r in refresh]], dtype=torch.int32))
@@ -299,7 +333,10 @@ class EpisodeRunner:
                     ops.check_indices(inp["idx"], b.n_cells)
                 masks = dict(reset_mask=dev[1] if any(reset) else None, refresh_mask=dev[2] if any(refresh) else None)
                 depth, pose, shifts = inp.get("depth"), inp.get("pose"), inp.get("shifts")
-                if "feat" in inp:
+                if self.regime == "heightmax":
+                    self._step_heightmax(inp, dev[0], masks["reset_mask"])
+                    levels = None
+                elif "feat" in inp:
                     levels = b.step(depth, pose, shifts, self.intr, self.cell, inp["feat"], None, self.order, active=dev[0],
                                     inputs_ready=False, **masks, **geo)
                 else:
@@ -312,12 +349,20 @@ class EpisodeRunner:
                 self.stats["slot_steps"] += self.R
                 self.stats["frames"] += sum(a is not None for a in step.assign)
                 self.stats["resets"] += sum(reset)
+                if self.regime == "heightmax":
+                    if self.save_dir:
+                        for s, a in enumerate(step.assign):
+                            if a is not None and a[1] == self.provider.n_frames(a[0]) - 1:
+                                self._save_heightmax(s, self.provider.name(a[0]))
+                    continue
                 if on_levels is not None:
                     on_levels(step, levels)
                 if self.save_dir:
                     for s, (a, st) in enumerate(zip(step.assign, step.seq_start)):
                         if a is not None and st:
                             self._save(s, self.provider.name(a[0]))
+            if self.regime == "heightmax":
+                return dict(self.stats)
             b.join()
             if b.variant == WRITE_DET:
                 self.stats["det_overflowed"] = b._det_ws is not None and b._det_ws.overflowed()

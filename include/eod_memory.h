@@ -252,6 +252,40 @@ int eod_write_max(const float *height, const int32_t *idx, const uint8_t *outlie
 int eod_max_winner_list(const int32_t *arg_pix, int n_episodes, int64_t n_cells, int H, int W, int C, int layout, int64_t *src_off,
                         int64_t *dst_row, int32_t *count, int capacity, eod_stream_t stream);
 
+/* Lock-step height-max regime: the contest and rule of eod_write_max (same key, same '>=' update, same results bit for bit)
+ * without the per-pixel idx / outlier / height planes, the arg_pix plane or its memset, and without a scan over the cells.
+ * Per frame: one contest entry point, then eod_heightmax_update.  Scratch, all-zero between frames (the update leaves it so):
+ *   key64 (E,cells) u64; n_list (E,2) i32 [listed cells, internal ticket]; cell_list (E,list_cap) i32 with
+ *   list_cap >= min(cells, lattice pixels) (else EOD_ERR_BADARG): the cells the frame touched, one entry each, in arbitrary order.
+ * raised (1) i32 device: set to 0 by the contest, = number of cells the update raised (all episodes) after it.
+ * active (E) i32 nullable: episodes with active <= 0 read nothing and list nothing (their state is left alone).
+ *
+ * Contest from DEPTH: geometry of eod_backproject_quantize (same device functions, bit-exact) computed in registers for the
+ * [::pix_stride, ::pix_stride] lattice; depth f32 metres or uint16 / depth_div (depth_is_u16); cells = map_w * map_h. */
+int eod_heightmax_contest_depth(const void *depth, int depth_is_u16, double depth_div, const float *pose, const float *shifts,
+                                int n_episodes, int H, int W, float fx, float fy, float cx, float cy, float cell, int map_w, int map_h,
+                                int order, float z_clip, int pix_stride, const int32_t *active, uint64_t *key64, int32_t *cell_list,
+                                int64_t list_cap, int32_t *n_list, int32_t *raised, eod_stream_t stream);
+/* Contest from PLANES: height (E,H,W) f32 world height, idx (E,H,W) i32 cell ids in [0, n_cells), outlier (E,H,W) u8 nullable -
+ * what create_coco_mp3d.py:157-165 stores, and what eod_write_max takes. */
+int eod_heightmax_contest_planes(const float *height, const int32_t *idx, const uint8_t *outlier, int n_episodes, int H, int W,
+                                 int pix_stride, int64_t n_cells, const int32_t *active, uint64_t *key64, int32_t *cell_list,
+                                 int64_t list_cap, int32_t *n_list, int32_t *raised, eod_stream_t stream);
+/* Update of the listed cells: height_map (E,cells) f32 and observed (E,cells) u8 of every raised cell, then either
+ *   copy:    state (E,cells,C) f32 row := the winner pixel's feature row; feat (E,C,H,W) [CHW] or (E,H,W,C) [HWC] in fp32
+ *            (EOD_LAYOUT_CHW / _HWC) or bf16 / fp16 (EOD_LAYOUT_*_BF16 / _F16, widened exactly: the state of feat.float());
+ *            C %% 4 == 0, feat and state 16-byte aligned (EOD_ERR_ALIGN);
+ *   replace: (src_off != NULL, state ignored) the compact winner list of eod_max_winner_list - src_off[i] element offset of the
+ *            winner's fp32 feature vector, dst_row[i] = e * cells + cell, count = raised - for eod_linear_rows (fp32 layouts only,
+ *            else EOD_ERR_UNSUPPORTED); win_cap entries. */
+int eod_heightmax_update(const void *feat, int layout, int n_episodes, int C, int H, int W, int64_t n_cells, const int32_t *cell_list,
+                         int64_t list_cap, int32_t *n_list, uint64_t *key64, float *height_map, uint8_t *observed, float *state,
+                         int64_t *src_off, int64_t *dst_row, int64_t win_cap, int32_t *raised, eod_stream_t stream);
+/* Per-slot reset of the height-max state (mask (E) i32, mask[e] != 0): height_map := 0 and observed := 0 for every cell, state rows
+ * := 0 for the observed cells only (the others are zero already), as eod_reset_episodes does for the mean grid.  C %% 4 == 0. */
+int eod_heightmax_reset(const int32_t *mask, int n_episodes, int64_t n_cells, int C, float *height_map, uint8_t *observed, float *state,
+                        eod_stream_t stream);
+
 /* Row GEMM with fp32 accuracy on tcgen05 tensor cores (3xTF32 split, fp32 accumulation in TMEM):
  *   Y[dst(i) * y_row_stride + j] = scale * ( sum_l A(i,l) * B(j,l) + bias[j] ),  i < min(M, *m_count), j < N, l < K
  *   A(i,l) = A[(a_off ? a_off[i] : i * a_row_stride) + l * a_k_stride]      B(j,l) = B[j * b_row_stride + l * b_k_stride]
