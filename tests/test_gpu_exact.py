@@ -14,6 +14,7 @@ import torch
 from oracle import reference_ops as R
 
 import exact_cases as X
+from test_gpu_scale import device_sms, semmap_update_sweeps
 
 pytestmark = pytest.mark.gpu
 
@@ -611,12 +612,16 @@ def test_write_max_replace_with_linlayer_exact(eod, cuda, layout):
 # ------------------------------------------------------------------------------------------------------------------------------
 # semmap_update
 # ------------------------------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("C", [128, 512])
-def test_semmap_update_exact(eod, cuda, C):
+@pytest.mark.parametrize("C,E,cells", [(128, 2, 900), (512, 2, 900), (128, 3, 250_007)], ids=["128", "512", "128-past-sweep"])
+def test_semmap_update_exact(eod, cuda, C, E, cells):
     """intensity = mean |sums| / count (custom_rcnn.py:747-748) bit for bit (C is a power of two); cls = the first argmax of the exact
-    float64 dot products with the classifier table (inputs built to have a unique maximum); cells not visible this frame untouched."""
+    float64 dot products with the classifier table (inputs built to have a unique maximum); cells not visible this frame untouched.
+    The last case has more rows than one sweep of the kernel's capped grid (606 208 on 148 SMs), with 32-row chunks straddling
+    episodes (250 007 % 32 != 0)."""
+    if cells > 900:
+        assert semmap_update_sweeps(E, cells, device_sms()) > 1 and cells % 32
     rng = np.random.default_rng(C)
-    E, cells, K, n_cls = 2, 900, 21, 20
+    K, n_cls = 21, 20
     zs = X.dyadic(rng, (C, K), 4, 4)
     sums = X.dyadic(rng, (E, cells, C), 8, 3)
     for _ in range(20):                                                    # make the maximum unique in every row

@@ -13,6 +13,7 @@ import torch
 
 import oracle
 from oracle import reference_ops as R
+from test_gpu_scale import FUSE_N, device_sms, fuse_trips
 
 pytestmark = pytest.mark.gpu
 
@@ -280,7 +281,8 @@ def test_explicit_map_read_mode(eod, cuda, golden):
 
 def test_fuse_bit_exact(eod, cuda):
     rng = np.random.default_rng(1)
-    for n in (1, 3, 4, 1000, 256 * 60 * 80 + 3):
+    assert fuse_trips(FUSE_N, device_sms()) > 1
+    for n in (1, 3, 4, 1000, 256 * 60 * 80 + 3, FUSE_N):              # FUSE_N: past the grid cap, so the grid-stride loop turns
         res = rng.standard_normal(n).astype(np.float32)
         mem = (rng.standard_normal(n) * 10).astype(np.float32)
         for w in (5.0, 500.0, 0.3):
