@@ -43,6 +43,8 @@ SIGNATURES = {
     "eod_write_objects": [_P, _P, _P, c_int, _P, _P, _P, c_int, c_int, c_int, c_int64, c_int, _P, _P],
     "eod_paste_masks": [_P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float, _P, _P, _P],
     "eod_write_objects_pasted": [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_float, _P, _P, _P, c_int, c_int, c_int64, c_int, _P, _P],
+    "eod_write_objects_det": [_P, _P, _P, c_int, _P, _P, _P, c_int, c_int, c_int, c_int64, _P, _P, c_int64, _P],
+    "eod_write_objects_pasted_det": [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_float, _P, _P, _P, c_int, c_int, c_int64, _P, _P, c_int64, _P],
     "eod_flush_slots": [_P, _P, _P, _P, c_int, c_int, c_int64, c_int, _P, _P, _P],
     "eod_bilinear_lattice": [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P],
     "eod_write_max": [_P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int, c_int64, _P, _P, _P, _P, _P, _P],

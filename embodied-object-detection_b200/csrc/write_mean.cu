@@ -27,14 +27,14 @@
 //   * deterministic variant (eod_write_mean_det_layout): fp32 CHW through the TMA ring, fp32 / bf16 / fp16 channels-last through the
 //     HWC kernel; both store raster-ordered run sums that the same segmented reduce adds in a fixed order.
 #include <cuda.h>
+#include <stdio.h>
 #include <stdlib.h>
 
+#include "det.cuh"
 #include "eod_common.cuh"
 #include "tmap_cache.cuh"
 
 namespace {
-
-constexpr int TILE_PX = 32;
 
 // ------------------------------------------------------------------------------------------------------
 // pre-pass / post-pass: one thread per pixel, warp-level run aggregation of the cell id
@@ -639,25 +639,8 @@ __device__ __forceinline__ void chw16_unit(uint32_t tile, uint32_t aux, int t, i
 // ceiling of this tile shape; selected with variant EOD_WRITE_TMA_DRY (bring-up / profiling only).
 // kPixN: the per-pixel reciprocal divisors 1/n_cell arrive with the tile (pix_n workspace); otherwise the
 // divisor of a run is a dependent global load from frame_cnt.
-// kDet: deterministic variant - a run's (unscaled) channel sums are STORED to partials[tile_off[tile] + r] (raster run
-// order, no atomics) for the segmented reduce of det_reduce_kernel; runs beyond the workspace capacity fall back to
-// the reductions of the default variant and raise *status.
-struct DetArgs {
-    const int32_t *tile_off;     // (E, tiles) exclusive scan of the per-tile run counts, restarting per episode
-    float *partials;             // (E, cap, C)
-    int32_t *run_cell;           // (E, cap)
-    int32_t *status;             // set to 1 when a run did not fit
-    int cap;                     // runs per episode the workspace holds
-};
-
-// The sampled pixels (bit p = pixel p of a 32-pixel tile) of the deterministic run that starts at head p0; `later` holds the heads
-// after p0 only.  The run pre-passes (det_run_sampled) and both kDet consumers must find the same runs in the same order: a run's
-// rank among them is its slot in partials.
-__device__ __forceinline__ unsigned det_run_mask(unsigned later, unsigned samps, int p0)
-{
-    const int p1 = later ? (__ffs(later) - 1) : TILE_PX;
-    return samps & (0xffffffffu >> (32 - p1)) & (0xffffffffu << p0);
-}
+// kDet: deterministic variant - the main pass of det.cuh: a run's (unscaled) channel sums are STORED to partials (DetArgs);
+// runs beyond the workspace capacity fall back to the reductions of the default variant and raise *status.
 
 // F: feature element type (FEAT_BF16 / FEAT_F16 take the 64-pixel unit and chw16_unit; neither kPixN nor kDet)
 template <int C, bool kDry, bool kPixN, bool kDet, int F = FEAT_F32>
@@ -1067,15 +1050,6 @@ int launch_tma16(const void *feat, const int32_t *idx, const uint8_t *samp, cons
 //                      => bitwise reproducible, and the reference's own arithmetic shape
 // List order and slot order depend on scheduling; the result does not: every cell is reduced on its own, in raster order.
 // ------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void det_tile_masks(const int32_t *idx, const uint8_t *samp, size_t g0, unsigned lane, int &cell, unsigned &heads,
-                                               unsigned &samps)
-{
-    cell = __ldg(idx + g0 + lane);
-    const int prev = __shfl_up_sync(0xffffffffu, cell, 1);
-    heads = __ballot_sync(0xffffffffu, lane == 0 || prev != cell);
-    samps = samp ? __ballot_sync(0xffffffffu, __ldg(samp + g0 + lane) != 0) : 0xffffffffu;
-}
-
 // does the run starting at head bit p0 contain a sampled pixel?
 __device__ __forceinline__ bool det_run_sampled(unsigned heads, unsigned samps, int p0)
 {
@@ -1442,13 +1416,6 @@ __global__ void __launch_bounds__(256) det_final_kernel(const int32_t *__restric
     }
 }
 
-struct DetWorkspace {
-    int32_t *tile_off, *n_runs, *n_list, *status, *cell_runs, *cell_off, *run_cell, *seg, *cell_list, *list_off;
-    float *partials;
-    DetLong L;
-    int cap;
-};
-
 size_t det_align(size_t x) { return (x + 255) & ~size_t(255); }
 
 // chunk rows per episode: every long segment (> DET_DIRECT runs) needs ceil(k / DET_CHUNK) <= k / DET_CHUNK + 1 rows and there
@@ -1469,24 +1436,96 @@ size_t det_carve(void *ws, int E, int C, int tiles_per_ep, int64_t n_cells, int 
     w.n_list = (int32_t *)take((size_t)E * 4);
     w.tile_off = (int32_t *)take((size_t)E * tiles_per_ep * 4);
     w.cell_off = (int32_t *)take((size_t)E * n_cells * 4);
-    w.L.chunk_rows = (int32_t *)take((size_t)E * 4);
-    w.L.n_long = (int32_t *)take((size_t)E * 4);
+    w.chunk_rows = (int32_t *)take((size_t)E * 4);
+    w.n_long = (int32_t *)take((size_t)E * 4);
     w.run_cell = (int32_t *)take((size_t)E * cap * 4);
     w.seg = (int32_t *)take((size_t)E * cap * 4);
     w.cell_list = (int32_t *)take((size_t)E * cap * 4);
     w.list_off = (int32_t *)take((size_t)E * cap * 4);
-    w.L.seg2 = (int32_t *)take((size_t)E * cap * 4);
-    w.L.task_start = (int32_t *)take((size_t)E * rows * 4);
-    w.L.task_len = (int32_t *)take((size_t)E * rows * 4);
-    w.L.long_i = (int32_t *)take((size_t)E * rows * 4);
-    w.L.long_base = (int32_t *)take((size_t)E * rows * 4);
-    w.L.cparts = (float *)take((size_t)E * rows * C * 4);
+    w.seg2 = (int32_t *)take((size_t)E * cap * 4);
+    w.task_start = (int32_t *)take((size_t)E * rows * 4);
+    w.task_len = (int32_t *)take((size_t)E * rows * 4);
+    w.long_i = (int32_t *)take((size_t)E * rows * 4);
+    w.long_base = (int32_t *)take((size_t)E * rows * 4);
+    w.cparts = (float *)take((size_t)E * rows * C * 4);
     w.partials = (float *)take((size_t)E * cap * C * 4);
-    w.L.rows = rows;
+    w.rows = rows;
     w.cap = cap;
     if (out) *out = w;
     return o;
 }
+
+// eod_check_launch with the stage of the deterministic write in the message ("<what>[<stage>]")
+int det_check_launch(const char *what, const char *stage)
+{
+    if (cudaPeekAtLastError() == cudaSuccess) return EOD_OK;
+    char buf[128];
+    snprintf(buf, sizeof buf, "%s[%s]", what, stage);
+    return eod_check_launch(buf);
+}
+
+template <int C>
+int launch_det_reduce(const char *what, const DetWorkspace &w, int E, int64_t n_cells, const uint32_t *frame_cnt, float *sums, cudaStream_t st)
+{
+    const DetLong L{w.seg2, w.task_start, w.task_len, w.long_i, w.long_base, w.chunk_rows, w.n_long, w.cparts, w.rows};
+    dim3 gc((w.cap + 255) / 256, E);
+    det_claim_kernel<<<gc, 256, 0, st>>>(w.run_cell, w.n_runs, w.cap, n_cells, w.cell_off, w.cell_runs, w.seg);
+    // at most min(cells, cap) cells carry runs; warps beyond n_list[e] exit at once
+    const int64_t max_list = n_cells < (int64_t)w.cap ? n_cells : (int64_t)w.cap;
+    const int64_t want_blocks = (max_list + DET_WARPS - 1) / DET_WARPS;
+    dim3 gr((unsigned)(want_blocks < 128 ? want_blocks : 128), E);          // warps stride over the episode's cell list
+    det_reduce_kernel<C><<<gr, 32 * DET_WARPS, 0, st>>>(w.cell_list, w.list_off, w.n_list, w.n_runs, w.cap, n_cells, w.seg, w.partials, frame_cnt, sums,
+                                                        L, w.status);
+    const int chunk_blocks = (L.rows + 7) / 8;
+    dim3 gk((unsigned)(chunk_blocks < 64 ? chunk_blocks : 64), E);
+    det_chunk_kernel<C><<<gk, 256, 0, st>>>(w.partials, w.cap, L);
+    dim3 gf(8, E);
+    det_final_kernel<C><<<gf, 256, 0, st>>>(w.cell_list, w.list_off, w.n_list, w.n_runs, w.cap, n_cells, frame_cnt, sums, L);
+    return det_check_launch(what, "reduce");
+}
+
+}  // namespace
+
+int det_prepass(const char *what, const int32_t *idx, const uint8_t *samp, const int32_t *active, int E, int C, int HW, int64_t n_cells,
+                void *ws, size_t ws_bytes, DetWorkspace *out, cudaStream_t st)
+{
+    EOD_REQUIRE(HW % TILE_PX == 0 && (!samp || (reinterpret_cast<uintptr_t>(samp) % 16 == 0)), EOD_ERR_UNSUPPORTED,
+                "%s: needs HW %% 32 == 0 and a 16-byte aligned sample mask", what);
+    EOD_REQUIRE(n_cells < (int64_t)INT32_MAX, EOD_ERR_BADARG, "%s: grid too large", what);
+    const int tiles_per_ep = HW / TILE_PX;
+    // capacity: whatever the workspace holds beyond the fixed planes (at most one run per pixel)
+    const size_t fixed = det_carve(nullptr, E, C, tiles_per_ep, n_cells, 0, nullptr);
+    EOD_REQUIRE(ws && eod_aligned16(ws) && ws_bytes > fixed + 4096, EOD_ERR_BADARG,
+                "%s: workspace missing or too small (see eod_write_mean_det_workspace_bytes)", what);
+    // per run: partial row + 5 ints; per chunk row (cap / 128 + cap / 256 of them): a partial row + 4 ints
+    const size_t per_run = (size_t)C * 4 + 20 + ((size_t)C * 4 + 16) * 3 / 256 + 1;
+    int64_t cap = ws_bytes > fixed + 16 * 256 ? (int64_t)((ws_bytes - fixed - 16 * 256) / ((size_t)E * per_run)) : 0;
+    if (cap > HW) cap = HW;
+    EOD_REQUIRE(cap >= 1, EOD_ERR_BADARG, "%s: workspace too small", what);
+    DetWorkspace w;
+    while (det_carve(ws, E, C, tiles_per_ep, n_cells, (int)cap, &w) > ws_bytes) --cap;
+    dim3 gt((tiles_per_ep + 7) / 8, E);
+    det_tile_runs_kernel<<<gt, 256, 0, st>>>(idx, samp, active, HW, tiles_per_ep, w.tile_off, w.n_list, w.chunk_rows, w.n_long);
+    det_scan_tiles_kernel<<<E, 1024, 0, st>>>(w.tile_off, tiles_per_ep, w.n_runs);
+    det_cell_runs_kernel<<<gt, 256, 0, st>>>(idx, samp, active, HW, tiles_per_ep, n_cells, w.tile_off, w.cap, w.cell_runs, w.cell_list, w.n_list);
+    det_scan_list_kernel<<<E, 1024, 0, st>>>(w.cell_runs, w.cell_list, w.n_list, w.cap, n_cells, w.list_off, w.cell_off);
+    *out = w;
+    return det_check_launch(what, "prepass");
+}
+
+int det_reduce(const char *what, const DetWorkspace &w, int C, int E, int64_t n_cells, const uint32_t *frame_cnt, float *sums, cudaStream_t st)
+{
+    switch (C) {
+    case 128: return launch_det_reduce<128>(what, w, E, n_cells, frame_cnt, sums, st);
+    case 256: return launch_det_reduce<256>(what, w, E, n_cells, frame_cnt, sums, st);
+    case 512: return launch_det_reduce<512>(what, w, E, n_cells, frame_cnt, sums, st);
+    default:
+        eod_set_error("%s: C=%d not compiled in (128, 256, 512)", what, C);
+        return EOD_ERR_UNSUPPORTED;
+    }
+}
+
+namespace {
 
 template <int C, bool kDet = false>
 int launch_hwc(const void *feat, int feat_type, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const int32_t *active, int E,
@@ -1498,50 +1537,19 @@ template <int C>
 int launch_det(const void *feat, int layout, const int32_t *idx, const uint8_t *samp, const uint32_t *frame_cnt, const int32_t *active, int E,
                int HW, int64_t n_cells, float *sums, void *ws, size_t ws_bytes, cudaStream_t st)
 {
-    EOD_REQUIRE(HW % TILE_PX == 0 && (!samp || (reinterpret_cast<uintptr_t>(samp) % 16 == 0)), EOD_ERR_UNSUPPORTED,
-                "eod_write_mean_det: needs HW %% 32 == 0 and a 16-byte aligned sample mask");
-    EOD_REQUIRE(n_cells < (int64_t)INT32_MAX, EOD_ERR_BADARG, "eod_write_mean_det: grid too large");
-    const int tiles_per_ep = HW / TILE_PX;
-    // capacity: whatever the workspace holds beyond the fixed planes (at most one run per pixel)
-    const size_t fixed = det_carve(nullptr, E, C, tiles_per_ep, n_cells, 0, nullptr);
-    EOD_REQUIRE(ws && eod_aligned16(ws) && ws_bytes > fixed + 4096, EOD_ERR_BADARG, "eod_write_mean_det: workspace missing or too small (see eod_write_mean_det_workspace_bytes)");
-    // per run: partial row + 5 ints; per chunk row (cap / 128 + cap / 256 of them): a partial row + 4 ints
-    const size_t per_run = (size_t)C * 4 + 20 + ((size_t)C * 4 + 16) * 3 / 256 + 1;
-    int64_t cap = ws_bytes > fixed + 16 * 256 ? (int64_t)((ws_bytes - fixed - 16 * 256) / ((size_t)E * per_run)) : 0;
-    if (cap > HW) cap = HW;
-    EOD_REQUIRE(cap >= 1, EOD_ERR_BADARG, "eod_write_mean_det: workspace too small");
-    DetWorkspace w;
-    while (det_carve(ws, E, C, tiles_per_ep, n_cells, (int)cap, &w) > ws_bytes) --cap;
+    // the tensor map is encoded before any launch: a failure must not leave the pre-passes' counts in the workspace
     CUtensorMap tmap;
-    int rc = layout == EOD_LAYOUT_CHW ? make_feature_tmap<C>(feat, E, HW, &tmap) : EOD_OK;
+    int rc = layout == EOD_LAYOUT_CHW && HW % TILE_PX == 0 ? make_feature_tmap<C>(feat, E, HW, &tmap) : EOD_OK;
     if (rc) return rc;
-    dim3 gt((tiles_per_ep + 7) / 8, E);
-    det_tile_runs_kernel<<<gt, 256, 0, st>>>(idx, samp, active, HW, tiles_per_ep, w.tile_off, w.n_list, w.L.chunk_rows, w.L.n_long);
-    det_scan_tiles_kernel<<<E, 1024, 0, st>>>(w.tile_off, tiles_per_ep, w.n_runs);
-    det_cell_runs_kernel<<<gt, 256, 0, st>>>(idx, samp, active, HW, tiles_per_ep, n_cells, w.tile_off, w.cap, w.cell_runs, w.cell_list, w.n_list);
-    det_scan_list_kernel<<<E, 1024, 0, st>>>(w.cell_runs, w.cell_list, w.n_list, w.cap, n_cells, w.list_off, w.cell_off);
-    if ((rc = eod_check_launch("eod_write_mean_det[prepass]"))) return rc;
-    DetArgs det{w.tile_off, w.partials, w.run_cell, w.status, w.cap};
+    DetWorkspace w;
+    if ((rc = det_prepass("eod_write_mean_det", idx, samp, active, E, C, HW, n_cells, ws, ws_bytes, &w, st))) return rc;
     if (layout == EOD_LAYOUT_CHW)
-        rc = launch_tma_kernel<C, false, false, true>(tmap, idx, samp, frame_cnt, nullptr, active, E, HW, n_cells, sums, st, det);
+        rc = launch_tma_kernel<C, false, false, true>(tmap, idx, samp, frame_cnt, nullptr, active, E, HW, n_cells, sums, st, det_args(w));
     else
         rc = launch_hwc<C, true>(feat, layout == EOD_LAYOUT_HWC_BF16 ? FEAT_BF16 : (layout == EOD_LAYOUT_HWC_F16 ? FEAT_F16 : FEAT_F32), idx, samp,
-                                 frame_cnt, active, E, HW, n_cells, sums, st, det);
+                                 frame_cnt, active, E, HW, n_cells, sums, st, det_args(w));
     if (rc) return rc;
-    dim3 gc((w.cap + 255) / 256, E);
-    det_claim_kernel<<<gc, 256, 0, st>>>(w.run_cell, w.n_runs, w.cap, n_cells, w.cell_off, w.cell_runs, w.seg);
-    // at most min(cells, cap) cells carry runs; warps beyond n_list[e] exit at once
-    const int64_t max_list = n_cells < (int64_t)w.cap ? n_cells : (int64_t)w.cap;
-    const int64_t want_blocks = (max_list + DET_WARPS - 1) / DET_WARPS;
-    dim3 gr((unsigned)(want_blocks < 128 ? want_blocks : 128), E);          // warps stride over the episode's cell list
-    det_reduce_kernel<C><<<gr, 32 * DET_WARPS, 0, st>>>(w.cell_list, w.list_off, w.n_list, w.n_runs, w.cap, n_cells, w.seg, w.partials, frame_cnt, sums,
-                                                        w.L, w.status);
-    const int chunk_blocks = (w.L.rows + 7) / 8;
-    dim3 gk((unsigned)(chunk_blocks < 64 ? chunk_blocks : 64), E);
-    det_chunk_kernel<C><<<gk, 256, 0, st>>>(w.partials, w.cap, w.L);
-    dim3 gf(8, E);
-    det_final_kernel<C><<<gf, 256, 0, st>>>(w.cell_list, w.list_off, w.n_list, w.n_runs, w.cap, n_cells, frame_cnt, sums, w.L);
-    return eod_check_launch("eod_write_mean_det[reduce]");
+    return det_reduce("eod_write_mean_det", w, C, E, n_cells, frame_cnt, sums, st);
 }
 
 template <int C, int F = FEAT_F32>

@@ -15,6 +15,10 @@
 //   eod_flush_slots      sums[cell] += scratch[slot] / n_cell ; scratch row, slot map and slot counter := 0
 //   eod_finalize_counts  counts += 1 for every visible cell                (write_mean.cu)
 //
+// Deterministic variant (eod_write_objects[_pasted]_det): eod_frame_count without slots, then the run pre-passes of the dense
+// deterministic write (det.cuh), write_objects_det_kernel storing one partial per run of equal cell id, and the dense write's
+// segmented reduce - the bits of eod_write_mean_det on the box_to_image_features image, reproducible run to run.
+//
 // The per-frame scratch keeps the arithmetic of the reference: the frame's samples of a cell are summed on their own,
 // divided by their count, and only that mean meets the (much larger) running sum - one rounding at grid magnitude per
 // frame instead of one per sample.
@@ -30,6 +34,7 @@
 // ix = fma(gx + 1, S/2, -0.5); out = fma(se_v, se, fma(sw_v, sw, fma(ne_v, ne, nw_v * nw)))), so the (K,480,640)
 // masks need never exist: eod_paste_masks folds them straight into `observed`, and the pasted variant of the write
 // re-evaluates the test for the ~1/8 sampled pixels only.
+#include "det.cuh"
 #include "eod_common.cuh"
 
 namespace {
@@ -487,6 +492,281 @@ __global__ void __launch_bounds__(256) flush_slots_kernel(const uint32_t *__rest
     }
 }
 
+// Deterministic variant (eod_write_objects[_pasted]_det): the main pass of det.cuh for the object regime.  It stores exactly the run
+// partials the dense deterministic write would store for the image eod_box_to_image_features builds - a run's sum, from +0, of the
+// values g of its sampled pixels in raster order - without building that image, so the pre-passes and the segmented reduce of the
+// dense write finish the job and the result is bitwise reproducible.
+// The CTA span, the sampled-pixel compaction and phase A's cover words are those of write_objects_kernel; phase B gives warps whole
+// 32-pixel tiles (one warp must own a run) in rounds of tiles whose sampled pixels fit the 256 cover rows.  Tiles without a sampled
+// pixel have no run and are skipped.  More than kCoverObjs objects: warp per tile, the cover set of a pixel by warp ballots.
+template <int C, bool kPasted>
+__global__ void __launch_bounds__(256) write_objects_det_kernel(const float *__restrict__ box_features, const uint8_t *__restrict__ masks,
+                                                                const float *__restrict__ probs, const float *__restrict__ boxes, int Sm, int W,
+                                                                float thr, const int32_t *__restrict__ n_obj, int Kmax, const int32_t *__restrict__ idx,
+                                                                const uint8_t *__restrict__ samp, const uint32_t *__restrict__ frame_cnt, int HW,
+                                                                int64_t n_cells, float *__restrict__ sums, const DetArgs det)
+{
+    constexpr int J = C / 32, J4 = C / 128;
+    constexpr int kTiles = kObjSpan / TILE_PX;
+    __shared__ int s_list[kObjSpan];
+    __shared__ __align__(16) uint32_t s_cover[256][kCoverObjs / 32];
+    __shared__ PasteObj s_obj[kPasted ? kCoverObjs : 1];
+    __shared__ int s_wcnt[8];
+    __shared__ int s_tstart[kTiles + 1];         // s_list index of each tile's first sampled pixel
+    __shared__ int s_busy[kTiles];               // tiles with a sampled pixel, in raster order
+    __shared__ int s_nbusy;
+    const int e = blockIdx.y;
+    const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (n_obj && __ldg(n_obj + e) <= 0) return;  // idle slot: the pre-passes gave it no runs; nothing of it is read
+    {   // raster-ordered list of the CTA's sampled pixels, as in write_objects_kernel, plus where each tile's pixels start in it
+        const int p0 = blockIdx.x * kObjSpan + threadIdx.x * 8;
+        const uint8_t *sp = samp + (size_t)e * HW + p0;
+        uint32_t lo = 0, hi = 0;
+        if (p0 + 7 < HW && (reinterpret_cast<uintptr_t>(sp) & 7u) == 0) {
+            const uint2 q = __ldg(reinterpret_cast<const uint2 *>(sp));
+            lo = q.x; hi = q.y;
+        } else {
+            for (int b = 0; b < 8 && p0 + b < HW; ++b) {
+                const uint32_t v = __ldg(sp + b);
+                if (b < 4) lo |= v << (8 * b); else hi |= v << (8 * (b - 4));
+            }
+        }
+        unsigned bits = 0;
+#pragma unroll
+        for (int b = 0; b < 4; ++b) bits |= (((lo >> (8 * b)) & 0xffu) ? 1u : 0u) << b | (((hi >> (8 * b)) & 0xffu) ? 1u : 0u) << (b + 4);
+        const int cnt = __popc(bits);
+        int incl = cnt;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int up = __shfl_up_sync(0xffffffffu, incl, o);
+            if ((int)lane >= o) incl += up;
+        }
+        if (lane == 31) s_wcnt[warp] = incl;
+        __syncthreads();
+        int pre = 0, tot = 0;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) { pre += w < (int)warp ? s_wcnt[w] : 0; tot += s_wcnt[w]; }
+        int pos = pre + incl - cnt;
+        if ((threadIdx.x & 3) == 0) s_tstart[threadIdx.x >> 2] = pos;          // four threads (32 pixels) per tile
+        if (threadIdx.x == 0) s_tstart[kTiles] = tot;
+        while (bits) {
+            s_list[pos++] = p0 + __ffs(bits) - 1;
+            bits &= bits - 1;
+        }
+        __syncthreads();
+        if (warp == 0) {
+            const bool b0 = s_tstart[lane + 1] > s_tstart[lane], b1 = s_tstart[lane + 33] > s_tstart[lane + 32];
+            const unsigned m0 = __ballot_sync(0xffffffffu, b0), m1 = __ballot_sync(0xffffffffu, b1);
+            if (b0) s_busy[__popc(m0 & ((1u << lane) - 1u))] = (int)lane;
+            if (b1) s_busy[__popc(m0) + __popc(m1 & ((1u << lane) - 1u))] = (int)lane + 32;
+            if (lane == 0) s_nbusy = __popc(m0) + __popc(m1);
+        }
+        __syncthreads();
+    }
+    const int n_busy = s_nbusy;
+    if (n_busy == 0) return;
+    const int K = n_obj ? min(__ldg(n_obj + e), Kmax) : Kmax;
+    const uint8_t *m = kPasted ? nullptr : masks + (size_t)e * Kmax * HW;
+    const float *f = box_features + (size_t)e * Kmax * C;
+    const int tiles_per_ep = HW / TILE_PX;
+
+    // warp-level run walk of one tile: for every run with a sampled pixel (det_run_mask order), value(p, acc) adds the pixel's g into the
+    // run's accumulator, then the run's sum is stored at its raster rank - or, past the workspace, reduced into sums as sum / n_cell
+    auto walk_tile = [&](int tt, auto &&begin_run, auto &&add_pixel, auto &&end_run) {
+        const int tile = (int)blockIdx.x * kTiles + tt;
+        int cell;
+        unsigned heads, samps;
+        det_tile_masks(idx, samp, (size_t)e * HW + (size_t)tile * TILE_PX, lane, cell, heads, samps);
+        int run_pos = __ldg(det.tile_off + (size_t)e * tiles_per_ep + tile);
+        while (heads) {
+            const int p0 = __ffs(heads) - 1;
+            heads &= heads - 1;
+            unsigned mr = det_run_mask(heads, samps, p0);
+            if (mr == 0) continue;
+            begin_run();
+            do {
+                const int p = __ffs(mr) - 1;
+                mr &= mr - 1;
+                add_pixel(tile * TILE_PX + p, __popc(samps & ((1u << p) - 1u)));
+            } while (mr);
+            end_run(__shfl_sync(0xffffffffu, cell, p0), run_pos++);
+        }
+    };
+    auto fallback_n = [&](int rc) {
+        if (lane == 0) *det.status = 1;                                    // workspace too small: correct, but not reproducible
+        return (float)(__ldg(frame_cnt + (size_t)e * n_cells + rc) & 0x7fffffffu);
+    };
+
+    if (K <= kCoverObjs) {
+        if (kPasted) {
+            if ((int)threadIdx.x < K) s_obj[threadIdx.x] = paste_prepare(boxes + ((size_t)e * Kmax + threadIdx.x) * 4, HW / W, W, thr);
+            __syncthreads();
+        }
+        for (int b0 = 0; b0 < n_busy;) {
+            // round: busy tiles [b0, b1) whose sampled pixels (contiguous in s_list) fit the 256 cover rows; one tile has at most 32
+            const int base = s_tstart[s_busy[b0]];
+            int b1 = b0 + 1;
+            while (b1 < n_busy && s_tstart[s_busy[b1] + 1] - base <= 256) ++b1;
+            const int nn = s_tstart[s_busy[b1 - 1] + 1] - base;
+            // ---- phase A: thread per sampled pixel, its cover words (write_objects_kernel's test) ----
+            if ((int)threadIdx.x < nn) {
+                const int px = s_list[base + threadIdx.x];
+                const int x = px % W, y = px / W;
+                unsigned w0 = 0u, w1 = 0u, w2 = 0u, w3 = 0u;
+                for (int k = 0; k < K; ++k) {
+                    bool mine;
+                    if (kPasted) {
+                        const PasteObj &o = s_obj[k];
+                        mine = x >= o.rx0 && x < o.rx1 && y >= o.ry0 && y < o.ry1 &&
+                               paste_eval(probs + ((size_t)e * Kmax + k) * Sm * Sm, Sm, paste_axis(x, o.x0, o.dx, Sm), paste_axis(y, o.y0, o.dy, Sm), thr);
+                    } else {
+                        mine = __ldg(m + (size_t)k * HW + px) != 0;
+                    }
+                    if (mine) {
+                        const unsigned bit = 1u << (k & 31);
+                        const int wd = k >> 5;
+                        w0 |= wd == 0 ? bit : 0u; w1 |= wd == 1 ? bit : 0u; w2 |= wd == 2 ? bit : 0u; w3 |= wd == 3 ? bit : 0u;
+                    }
+                }
+                s_cover[threadIdx.x][0] = w0; s_cover[threadIdx.x][1] = w1; s_cover[threadIdx.x][2] = w2; s_cover[threadIdx.x][3] = w3;
+            }
+            __syncthreads();
+            // ---- phase B: warp per busy tile; lanes own float4 channel groups 4*lane + 128*j ----
+            // g is recomputed only when the cover set changes (bit-identical either way); the empty set's g is +0, the image's value
+            // at a pixel no object covers
+            float4 g[J4], acc[J4];
+#pragma unroll
+            for (int j = 0; j < J4; ++j) g[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+            uint4 have = make_uint4(0u, 0u, 0u, 0u);
+            for (int bt = b0 + (int)warp; bt < b1; bt += 8) {
+                const int tt = s_busy[bt];
+                const int row0 = s_tstart[tt] - base;
+                walk_tile(
+                    tt,
+                    [&]() {
+#pragma unroll
+                        for (int j = 0; j < J4; ++j) acc[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+                    },
+                    [&](int, int rank) {
+                        const uint4 cw = *reinterpret_cast<const uint4 *>(&s_cover[row0 + rank][0]);
+                        if (cw.x != have.x || cw.y != have.y || cw.z != have.z || cw.w != have.w) {
+                            have = cw;
+#pragma unroll
+                            for (int j = 0; j < J4; ++j) g[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+                            int cnt = 0;
+                            const unsigned words[4] = {cw.x, cw.y, cw.z, cw.w};
+#pragma unroll
+                            for (int wd = 0; wd < 4; ++wd) {
+                                unsigned todo = words[wd];
+                                cnt += __popc(todo);
+                                while (todo) {                             // ascending object index
+                                    const int kk = wd * 32 + __ffs(todo) - 1;
+                                    todo &= todo - 1;
+                                    const float4 *row = reinterpret_cast<const float4 *>(f + (size_t)kk * C) + lane;
+#pragma unroll
+                                    for (int j = 0; j < J4; ++j) {
+                                        const float4 v = __ldg(row + 32 * j);
+                                        g[j].x = __fadd_rn(g[j].x, v.x); g[j].y = __fadd_rn(g[j].y, v.y);
+                                        g[j].z = __fadd_rn(g[j].z, v.z); g[j].w = __fadd_rn(g[j].w, v.w);
+                                    }
+                                }
+                            }
+                            if (cnt > 1) {                                 // / #objects; a power of two as the exact reciprocal
+                                if ((cnt & (cnt - 1)) == 0) {
+                                    const float r = 1.0f / (float)cnt;
+#pragma unroll
+                                    for (int j = 0; j < J4; ++j)
+                                        g[j] = make_float4(__fmul_rn(g[j].x, r), __fmul_rn(g[j].y, r), __fmul_rn(g[j].z, r), __fmul_rn(g[j].w, r));
+                                } else {
+                                    const float n_px = (float)cnt;
+#pragma unroll
+                                    for (int j = 0; j < J4; ++j)
+                                        g[j] = make_float4(__fdiv_rn(g[j].x, n_px), __fdiv_rn(g[j].y, n_px), __fdiv_rn(g[j].z, n_px), __fdiv_rn(g[j].w, n_px));
+                                }
+                            }
+                        }
+#pragma unroll
+                        for (int j = 0; j < J4; ++j) {
+                            acc[j].x = __fadd_rn(acc[j].x, g[j].x); acc[j].y = __fadd_rn(acc[j].y, g[j].y);
+                            acc[j].z = __fadd_rn(acc[j].z, g[j].z); acc[j].w = __fadd_rn(acc[j].w, g[j].w);
+                        }
+                    },
+                    [&](int rc, int pos) {
+                        if (pos < det.cap) {
+                            float *d = det.partials + ((size_t)e * det.cap + pos) * C + 4 * lane;
+#pragma unroll
+                            for (int j = 0; j < J4; ++j) *reinterpret_cast<float4 *>(d + 128 * j) = acc[j];
+                            if (lane == 0) det.run_cell[(size_t)e * det.cap + pos] = rc;
+                            return;
+                        }
+                        const float n = fallback_n(rc);
+                        float *d = sums + ((size_t)e * n_cells + rc) * C + 4 * lane;
+#pragma unroll
+                        for (int j = 0; j < J4; ++j)
+                            red_add_v4(d + 128 * j, __fdiv_rn(acc[j].x, n), __fdiv_rn(acc[j].y, n), __fdiv_rn(acc[j].z, n), __fdiv_rn(acc[j].w, n));
+                    });
+            }
+            __syncthreads();                                               // s_cover is rewritten by the next round
+            b0 = b1;
+        }
+        return;
+    }
+
+    // ---- more than kCoverObjs objects: warp per busy tile, lanes test 32 objects at once; lanes own channels lane + 32*j ----
+    float acc[J];
+    for (int bt = (int)warp; bt < n_busy; bt += 8) {
+        walk_tile(
+            s_busy[bt],
+            [&]() {
+#pragma unroll
+                for (int j = 0; j < J; ++j) acc[j] = 0.f;
+            },
+            [&](int px, int) {
+                float g[J];
+#pragma unroll
+                for (int j = 0; j < J; ++j) g[j] = 0.f;
+                int cnt = 0;
+                for (int k0 = 0; k0 < K; k0 += 32) {
+                    const int k = k0 + (int)lane;
+                    bool mine = false;
+                    if (k < K) {
+                        if (kPasted) {
+                            const PasteObj o = paste_prepare(boxes + ((size_t)e * Kmax + k) * 4, HW / W, W, thr);
+                            mine = paste_covers(probs + ((size_t)e * Kmax + k) * Sm * Sm, o, Sm, px % W, px / W, thr);
+                        } else {
+                            mine = __ldg(m + (size_t)k * HW + px) != 0;
+                        }
+                    }
+                    unsigned todo = __ballot_sync(0xffffffffu, mine);
+                    cnt += __popc(todo);
+                    while (todo) {                                         // ascending object index
+                        const int kk = k0 + __ffs(todo) - 1;
+                        todo &= todo - 1;
+                        const float *row = f + (size_t)kk * C + lane;
+#pragma unroll
+                        for (int j = 0; j < J; ++j) g[j] = __fadd_rn(g[j], __ldg(row + 32 * j));
+                    }
+                }
+                const float n_px = (float)cnt;
+#pragma unroll
+                for (int j = 0; j < J; ++j) acc[j] = __fadd_rn(acc[j], cnt ? __fdiv_rn(g[j], n_px) : 0.f);
+            },
+            [&](int rc, int pos) {
+                if (pos < det.cap) {
+                    float *d = det.partials + ((size_t)e * det.cap + pos) * C + lane;
+#pragma unroll
+                    for (int j = 0; j < J; ++j) d[32 * j] = acc[j];
+                    if (lane == 0) det.run_cell[(size_t)e * det.cap + pos] = rc;
+                    return;
+                }
+                const float n = fallback_n(rc);
+                float *d = sums + ((size_t)e * n_cells + rc) * C + lane;
+#pragma unroll
+                for (int j = 0; j < J; ++j) red_add_f32(d + 32 * j, __fdiv_rn(acc[j], n));
+            });
+    }
+}
+
 __global__ void zero_i32_kernel(int32_t *p, int n)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -570,6 +850,63 @@ extern "C" int eod_write_objects_pasted(const float *box_features, const float *
     EOD_REQUIRE(threshold >= 0.f, EOD_ERR_UNSUPPORTED, "eod_write_objects_pasted: threshold < 0 is not supported");
     return launch_write_objects("eod_write_objects_pasted", true, box_features, nullptr, mask_probs, boxes, S, W, threshold, n_obj, Kmax, idx,
                                 samp, slot_of_cell, n_episodes, C, H * W, n_cells, n_slots_max, scratch, (cudaStream_t)stream);
+}
+
+static int launch_write_objects_det(const char *what, bool pasted, const float *box_features, const uint8_t *masks, const float *probs,
+                                    const float *boxes, int S, int W, float thr, const int32_t *n_obj, int Kmax, const int32_t *idx,
+                                    const uint8_t *samp, const uint32_t *frame_cnt, int n_episodes, int C, int HW, int64_t n_cells, float *sums,
+                                    void *ws, int64_t ws_bytes, cudaStream_t st)
+{
+    EOD_REQUIRE(C == 128 || C == 256 || C == 512, EOD_ERR_UNSUPPORTED, "%s: C=%d not compiled in (128, 256, 512)", what, C);
+    EOD_REQUIRE(eod_aligned16(box_features) && eod_aligned16(sums), EOD_ERR_ALIGN, "%s: box_features and sums must be 16-byte aligned", what);
+    DetWorkspace w;
+    int rc = det_prepass(what, idx, samp, n_obj, n_episodes, C, HW, n_cells, ws, (size_t)ws_bytes, &w, st);
+    if (rc) return rc;
+    const DetArgs det = det_args(w);
+    dim3 grid((HW + kObjSpan - 1) / kObjSpan, n_episodes);
+#define EOD_WOD(CC)                                                                                                                        \
+    case CC:                                                                                                                               \
+        if (pasted)                                                                                                                        \
+            write_objects_det_kernel<CC, true><<<grid, 256, 0, st>>>(box_features, masks, probs, boxes, S, W, thr, n_obj, Kmax, idx, samp,  \
+                                                                     frame_cnt, HW, n_cells, sums, det);                                  \
+        else                                                                                                                               \
+            write_objects_det_kernel<CC, false><<<grid, 256, 0, st>>>(box_features, masks, probs, boxes, S, W, thr, n_obj, Kmax, idx, samp, \
+                                                                      frame_cnt, HW, n_cells, sums, det);                                 \
+        break;
+    switch (C) {
+        EOD_WOD(128)
+        EOD_WOD(256)
+        EOD_WOD(512)
+    }
+#undef EOD_WOD
+    if ((rc = eod_check_launch(what))) return rc;
+    return det_reduce(what, w, C, n_episodes, n_cells, frame_cnt, sums, st);
+}
+
+extern "C" int eod_write_objects_det(const float *box_features, const uint8_t *masks, const int32_t *n_obj, int Kmax, const int32_t *idx,
+                                     const uint8_t *samp, const uint32_t *frame_cnt, int n_episodes, int C, int HW, int64_t n_cells, float *sums,
+                                     void *workspace, int64_t workspace_bytes, eod_stream_t stream)
+{
+    EOD_REQUIRE(box_features && masks && idx && samp && frame_cnt && sums && workspace, EOD_ERR_BADARG, "eod_write_objects_det: null pointer");
+    EOD_REQUIRE(n_episodes > 0 && n_episodes <= 65535 && Kmax > 0 && HW > 0 && n_cells > 0 && workspace_bytes > 0, EOD_ERR_BADARG,
+                "eod_write_objects_det: bad sizes");
+    return launch_write_objects_det("eod_write_objects_det", false, box_features, masks, nullptr, nullptr, 0, 1, 0.f, n_obj, Kmax, idx, samp,
+                                    frame_cnt, n_episodes, C, HW, n_cells, sums, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int eod_write_objects_pasted_det(const float *box_features, const float *mask_probs, const float *boxes, const int32_t *n_obj,
+                                            int Kmax, int S, int H, int W, float threshold, const int32_t *idx, const uint8_t *samp,
+                                            const uint32_t *frame_cnt, int n_episodes, int C, int64_t n_cells, float *sums, void *workspace,
+                                            int64_t workspace_bytes, eod_stream_t stream)
+{
+    EOD_REQUIRE(box_features && mask_probs && boxes && idx && samp && frame_cnt && sums && workspace, EOD_ERR_BADARG,
+                "eod_write_objects_pasted_det: null pointer");
+    EOD_REQUIRE(n_episodes > 0 && n_episodes <= 65535 && Kmax > 0 && S > 0 && S <= 4096 && H > 0 && W > 0 && (int64_t)H * W < (1ll << 31) - 1024 &&
+                    n_cells > 0 && workspace_bytes > 0,
+                EOD_ERR_BADARG, "eod_write_objects_pasted_det: bad sizes");
+    EOD_REQUIRE(threshold >= 0.f, EOD_ERR_UNSUPPORTED, "eod_write_objects_pasted_det: threshold < 0 is not supported");
+    return launch_write_objects_det("eod_write_objects_pasted_det", true, box_features, nullptr, mask_probs, boxes, S, W, threshold, n_obj, Kmax,
+                                    idx, samp, frame_cnt, n_episodes, C, H * W, n_cells, sums, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int eod_flush_slots(const uint32_t *frame_cnt, int32_t *slot_of_cell, const int32_t *slot_cell, int32_t *n_slots, int n_episodes,

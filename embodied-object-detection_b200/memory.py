@@ -43,11 +43,20 @@ def _slot_workspace(slots: Optional[ops.ObjectSlots], E: int, n_cells: int, C: i
     return slots
 
 
-def _write_objects(idx: torch.Tensor, samp: torch.Tensor, frame_cnt: torch.Tensor, slots: ops.ObjectSlots, sums: torch.Tensor,
+def _write_objects(idx: torch.Tensor, samp: torch.Tensor, frame_cnt: torch.Tensor, slots: Optional[ops.ObjectSlots], sums: torch.Tensor,
                    box_features: torch.Tensor, n_obj: Optional[torch.Tensor], masks: Optional[torch.Tensor] = None,
-                   mask_probs: Optional[torch.Tensor] = None, boxes: Optional[torch.Tensor] = None, mask_thresh: float = 0.5) -> None:
+                   mask_probs: Optional[torch.Tensor] = None, boxes: Optional[torch.Tensor] = None, mask_thresh: float = 0.5,
+                   det_ws: Optional[ops.DetWorkspace] = None) -> None:
     """count -> object write -> flush of one frame into ``sums``, with the objects' ``masks``, or with their un-pasted
-    ``mask_probs`` and ``boxes`` (pasted inside the write).  frame_cnt stays set for the finalize."""
+    ``mask_probs`` and ``boxes`` (pasted inside the write).  frame_cnt stays set for the finalize.
+    det_ws: the deterministic write instead (count without the slot table, no flush; ``slots`` is unused)."""
+    if det_ws is not None:
+        ops.frame_count(idx, samp, frame_cnt, n_obj)
+        if masks is not None:
+            ops.write_objects_det(box_features, masks, n_obj, idx, samp, frame_cnt, sums, det_ws)
+        else:
+            ops.write_objects_pasted_det(box_features, mask_probs, boxes, n_obj, idx, samp, frame_cnt, sums, det_ws, mask_thresh)
+        return
     ops.frame_count(idx, samp, frame_cnt, n_obj, slots)
     if masks is not None:
         ops.write_objects(box_features, masks, n_obj, idx, samp, slots)
@@ -88,15 +97,18 @@ class EpisodeBatch:
 
     def __init__(self, n_episodes: int, map_w: int, map_h: int, channels: int, height: int = 480, width: int = 640,
                  device: torch.device = torch.device("cuda"), layout: int = LAYOUT_CHW, variant: int = WRITE_AUTO,
-                 pipeline: bool = False, fp16_table: bool = True):
+                 pipeline: bool = False, fp16_table: bool = True, object_variant: int = WRITE_AUTO):
         if torch.device(device).type != "cuda":
             raise EodError("EpisodeBatch needs a CUDA device (no CPU fallback)")
+        if object_variant not in (WRITE_AUTO, WRITE_DET):
+            raise ValueError(f"object_variant must be WRITE_AUTO or WRITE_DET, got {object_variant!r}")
         if variant == WRITE_DET and layout in (LAYOUT_CHW_BF16, LAYOUT_CHW_F16):
             raise EodError("variant=WRITE_DET has no deterministic write for 16-bit CHW features (use LAYOUT_HWC_BF16 / _HWC_F16 "
                            "channels-last features, or feed feat.float() with LAYOUT_CHW)")
         self.E, self.map_w, self.map_h, self.C, self.H, self.W = n_episodes, map_w, map_h, channels, height, width
         self.n_cells = map_w * map_h
         self.device, self.layout, self.variant, self.pipeline = torch.device(device), layout, variant, pipeline
+        self.object_variant = object_variant
         z = dict(device=self.device)
         self.sums = torch.zeros((self.E, self.n_cells, self.C), dtype=torch.float32, **z)
         self.counts = torch.zeros((self.E, self.n_cells), dtype=torch.float32, **z)
@@ -121,8 +133,9 @@ class EpisodeBatch:
         self._e_read: Optional[torch.cuda.Event] = None
         self._sync_next = True
         self._slots: Optional[ops.ObjectSlots] = None      # workspace of write_objects, created on first use
-        self._det_ws: Optional[ops.DetWorkspace] = None    # workspace of the deterministic write (variant=WRITE_DET)
-        self.det_runs_per_episode = 0                      # 0: HW/4 runs per episode and frame
+        # workspace of the deterministic writes (variant=WRITE_DET and / or object_variant=WRITE_DET: one serves both)
+        self._det_ws: Optional[ops.DetWorkspace] = None
+        self.det_runs_per_episode = 0                      # 0: HW/4 runs per episode and frame (every object frame with sample_stride >= 4)
         # CHW write: True = the divisors 1/n_cell travel with the tile (expand_counts pre-pass + 4 B per pixel); False = the consumer
         # looks a group's divisor up in frame_cnt itself (one dependent L2 load per group, no pre-pass)
         # (round 2: with the pixels of a tile grouped by cell there are few look-ups, and the pre-pass plus its 158 MB per 64-episode
@@ -247,11 +260,22 @@ class EpisodeBatch:
         if self._per_pixel_divisors:
             self._timed("expand", ops.expand_counts, self.idx, self.frame_cnt, self.pix_inv_n)
 
+    def _det_workspace(self) -> ops.DetWorkspace:
+        if self._det_ws is None:
+            self._det_ws = ops.DetWorkspace(self.E, self.C, self.H * self.W, self.n_cells, self.device, self.det_runs_per_episode)
+        return self._det_ws
+
+    def _object_workspace(self, sample_stride: int) -> dict:
+        """The workspace of this frame's object write, as the keywords of _write_objects: the deterministic write's
+        (object_variant=WRITE_DET) or the slot table of the reduction-based one."""
+        if self.object_variant == WRITE_DET:
+            return dict(slots=None, det_ws=self._det_workspace())
+        self._slots = _slot_workspace(self._slots, self.E, self.n_cells, self.C, self.H * self.W, sample_stride, self.device)
+        return dict(slots=self._slots)
+
     def _write(self, feat: torch.Tensor, samp: Optional[torch.Tensor], active: Optional[torch.Tensor] = None) -> None:
         if self.variant == WRITE_DET:
-            if self._det_ws is None:
-                self._det_ws = ops.DetWorkspace(self.E, self.C, self.H * self.W, self.n_cells, self.device, self.det_runs_per_episode)
-            self._timed("write", ops.write_mean_det, feat, self.idx, samp, self.frame_cnt, self.sums, self._det_ws, self.layout, active)
+            self._timed("write", ops.write_mean_det, feat, self.idx, samp, self.frame_cnt, self.sums, self._det_workspace(), self.layout, active)
             return
         self._timed("write", ops.write_mean, feat, self.idx, samp, self.frame_cnt, self.sums, self.layout, self.variant,
                     self.pix_inv_n if self._per_pixel_divisors else None, active)
@@ -275,11 +299,12 @@ class EpisodeBatch:
                       sample_stride: int = 8) -> None:
         """Object-feature regime (the reference's live path, custom_rcnn.py:681-743) for one frame of every episode,
         fused: box_features (E,Kmax,C) f32 (= 50*normalize(feat), :848), masks (E,Kmax,H,W) bool, n_obj (E) i32 kept
-        detections per episode (None = Kmax).  Episodes with n_obj == 0 are skipped entirely, counts included (:686)."""
-        self._slots = _slot_workspace(self._slots, self.E, self.n_cells, self.C, self.H * self.W, sample_stride, self.device)
+        detections per episode (None = Kmax).  Episodes with n_obj == 0 are skipped entirely, counts included (:686).
+        With ``object_variant=WRITE_DET`` the write is the deterministic one (bitwise reproducible, see ops.write_objects_det)."""
+        ws = self._object_workspace(sample_stride)
         observed = ops.masks_observed(masks, n_obj)
         samp = ops.sample_mask(observed, sample_stride)
-        _write_objects(self.idx, samp, self.frame_cnt, self._slots, self.sums, box_features, n_obj, masks=masks)
+        _write_objects(self.idx, samp, self.frame_cnt, ws["slots"], self.sums, box_features, n_obj, masks=masks, det_ws=ws.get("det_ws"))
         self._finalize()
 
     def write_detections(self, box_features: torch.Tensor, mask_probs: torch.Tensor, boxes: torch.Tensor,
@@ -288,11 +313,11 @@ class EpisodeBatch:
         mask head's 28x28 probabilities), boxes (E,Kmax,4) f32 XYXY.  paste_masks_in_image is folded into the write: the
         (K,480,640) masks are never built - one pass ORs the pasted test into ``observed``, the write re-evaluates it for
         the sampled pixels only."""
-        self._slots = _slot_workspace(self._slots, self.E, self.n_cells, self.C, self.H * self.W, sample_stride, self.device)
+        ws = self._object_workspace(sample_stride)
         _, observed = ops.paste_masks(mask_probs, boxes, (self.H, self.W), mask_thresh, n_obj, want_masks=False, want_observed=True)
         samp = ops.sample_mask(observed, sample_stride)
-        _write_objects(self.idx, samp, self.frame_cnt, self._slots, self.sums, box_features, n_obj,
-                       mask_probs=mask_probs, boxes=boxes, mask_thresh=mask_thresh)
+        _write_objects(self.idx, samp, self.frame_cnt, ws["slots"], self.sums, box_features, n_obj,
+                       mask_probs=mask_probs, boxes=boxes, mask_thresh=mask_thresh, det_ws=ws.get("det_ws"))
         self._finalize()
 
     # ---- one frame, overlapped -------------------------------------------------------------------------------
@@ -407,12 +432,12 @@ class EpisodeBatch:
         promise of ``pipeline=True`` covers depth / pose / shifts / proj_indices AND box_features / mask_probs / boxes / n_obj
         (``inputs_ready=False`` drops it for one call); reset_mask / refresh_mask are ordered on the caller's stream, as in ``step``.
         A step's inputs may be overwritten once the next step has returned.  Slots whose episode has ended pass n_obj == 0
-        (nothing is written, :686)."""
+        (nothing is written, :686).  ``object_variant=WRITE_DET``: the write is the deterministic one (count without slots, no flush)."""
         capturing = torch.cuda.is_current_stream_capturing()
         if self._pre is None:
             with torch.cuda.device(self.device):
                 self._pre = torch.cuda.Stream(priority=0)
-        self._slots = _slot_workspace(self._slots, self.E, self.n_cells, self.C, self.H * self.W, sample_stride, self.device)
+        ws = self._object_workspace(sample_stride)
         # a side stream joins a capture only by waiting for the capturing stream
         s0, strict, e_in = self._begin_frame(inputs_ready, force_strict=capturing)
         e_state = self._reset_refresh(e_in, reset_mask, refresh_mask)
@@ -442,8 +467,8 @@ class EpisodeBatch:
                 self._wr.wait_event(e_in)                  # the detection inputs are inside the pipeline promise
             self._wr.wait_event(e_geo)
             self._wr.wait_event(e_samp)
-            _write_objects(self.idx, samp, self.frame_cnt, self._slots, self.sums, box_features, n_obj,
-                           mask_probs=mask_probs, boxes=boxes, mask_thresh=mask_thresh)
+            _write_objects(self.idx, samp, self.frame_cnt, ws["slots"], self.sums, box_features, n_obj,
+                           mask_probs=mask_probs, boxes=boxes, mask_thresh=mask_thresh, det_ws=ws.get("det_ws"))
         # a capture must join every side stream back into the capturing stream
         e_fin = self._end_frame(s0, e_read, wait_fin=not self.pipeline or capturing,
                                 inputs=(box_features, mask_probs, boxes) + ((n_obj,) if n_obj is not None else ()))
@@ -482,7 +507,8 @@ class GraphedDetections:
         with torch.cuda.device(batch.device):
             batch.join()
             torch.cuda.current_stream().synchronize()
-            # everything the step allocates lazily (slot workspace, the library's per-device state) must exist before the capture; the
+            # everything the step allocates lazily (slot or deterministic-write workspace, the library's per-device state) must exist
+            # before the capture; the
             # warm-up frame runs with n_obj = 0, which writes nothing and leaves the grid as it is
             zero_obj = torch.zeros((batch.E,), dtype=torch.int32, device=batch.device)
             batch.step_detections(*args[:8], zero_obj, **kw)

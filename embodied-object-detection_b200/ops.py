@@ -28,7 +28,7 @@ launch_count = 0
 
 _LAUNCHES = {"eod_backproject_quantize": 1, "eod_backproject_quantize_u16": 1, "eod_backproject_count": 1, "eod_quantize_world": 1, "eod_sample_mask": 1, "eod_frame_count": 1, "eod_expand_counts": 1, "eod_write_mean": 1, "eod_write_mean_det": 9,
              "eod_write_mean_det_layout": 9,
-             "eod_finalize_counts": 1, "eod_box_to_image_features": 1, "eod_masks_observed": 1, "eod_paste_masks": 1, "eod_write_objects_pasted": 1, "eod_bilinear_lattice": 1, "eod_write_objects": 1, "eod_flush_slots": 2, "eod_write_max": 2, "eod_read_pool": 2,
+             "eod_finalize_counts": 1, "eod_box_to_image_features": 1, "eod_masks_observed": 1, "eod_paste_masks": 1, "eod_write_objects_pasted": 1, "eod_bilinear_lattice": 1, "eod_write_objects": 1, "eod_write_objects_det": 9, "eod_write_objects_pasted_det": 9, "eod_flush_slots": 2, "eod_write_max": 2, "eod_read_pool": 2,
              "eod_fuse": 1, "eod_project_split_weights": 1, "eod_project_fuse": 1, "eod_project_fuse_levels": 1, "eod_normalize_memory": 1, "eod_reset_touched": 1, "eod_semmap_update": 1, "eod_semmap_decode": 2,
              "eod_reset_episodes": 1, "eod_refresh_norm16": 1, "eod_check_indices": 1, "eod_remap_indices": 1, "eod_max_winner_list": 1, "eod_linear_rows": 1, "eod_read_roi": 1,
              "eod_heightmax_contest_depth": 1, "eod_heightmax_contest_planes": 1, "eod_heightmax_update": 1, "eod_heightmax_reset": 1}
@@ -305,7 +305,7 @@ def remap_indices(idx: torch.Tensor, lut: torch.Tensor, n_rows: int, add: int = 
 
 
 class DetWorkspace:
-    """Caller-owned workspace of the deterministic write (eod_write_mean_det), zero-filled once."""
+    """Caller-owned workspace of the deterministic writes (write_mean_det, write_objects[_pasted]_det), zero-filled once."""
 
     def __init__(self, n_episodes: int, channels: int, hw: int, n_cells: int, device: torch.device, runs_per_episode: int = 0):
         lib = _lib.lib()
@@ -451,6 +451,42 @@ def write_objects_pasted(box_features: torch.Tensor, mask_probs: torch.Tensor, b
     _call("eod_write_objects_pasted", box_features.data_ptr(), mask_probs.data_ptr(), boxes.data_ptr(), _ptr(n_obj), Kmax, S, H, W,
           float(threshold), idx.data_ptr(), samp.data_ptr(), slots.slot_of_cell.data_ptr(), E, slots.C, slots.n_cells, slots.S,
           slots.scratch.data_ptr(), _stream())
+
+
+def write_objects_det(box_features: torch.Tensor, masks: torch.Tensor, n_obj: Optional[torch.Tensor], idx: torch.Tensor,
+                      samp: torch.Tensor, frame_cnt: torch.Tensor, sums: torch.Tensor, ws: DetWorkspace) -> None:
+    """Deterministic object write (HW % 32 == 0): sums[cell] += the cell's mean of the sampled pixels' object means, bit for bit
+    what write_mean_det(LAYOUT_CHW) adds for the box_to_image_features image, without building it.  frame_cnt from
+    frame_count(idx, samp, frame_cnt, n_obj) (no slots); ws is the DetWorkspace of write_mean_det, sized the same way."""
+    masks = _masks_u8(masks)
+    _dev(box_features, torch.float32, "box_features"), _dev(idx, torch.int32, "idx"), _dev(samp, torch.uint8, "samp")
+    _dev(frame_cnt, torch.int32, "frame_cnt"), _dev(sums, torch.float32, "sums")
+    E, Kmax, H, W = masks.shape
+    _, n_cells, C = sums.shape
+    if box_features.shape != (E, Kmax, C) or sums.shape[0] != E:
+        raise ValueError("box_features must be (E,Kmax,C) matching masks (E,Kmax,H,W) and sums (E,cells,C)")
+    if n_obj is not None:
+        _dev(n_obj, torch.int32, "n_obj")
+    _call("eod_write_objects_det", box_features.data_ptr(), masks.data_ptr(), _ptr(n_obj), Kmax, idx.data_ptr(), samp.data_ptr(),
+          frame_cnt.data_ptr(), E, C, H * W, n_cells, sums.data_ptr(), ws.buf.data_ptr(), ws.nbytes, _stream())
+
+
+def write_objects_pasted_det(box_features: torch.Tensor, mask_probs: torch.Tensor, boxes: torch.Tensor, n_obj: Optional[torch.Tensor],
+                             idx: torch.Tensor, samp: torch.Tensor, frame_cnt: torch.Tensor, sums: torch.Tensor, ws: DetWorkspace,
+                             threshold: float = 0.5) -> None:
+    """write_objects_det with the pasted-mask test evaluated on the fly: mask_probs (E,Kmax,S,S), boxes (E,Kmax,4), idx (E,H,W)."""
+    E, Kmax, S = _paste_args(mask_probs, boxes, n_obj)
+    _dev(box_features, torch.float32, "box_features"), _dev(idx, torch.int32, "idx"), _dev(samp, torch.uint8, "samp")
+    _dev(frame_cnt, torch.int32, "frame_cnt"), _dev(sums, torch.float32, "sums")
+    if idx.dim() != 3:
+        raise ValueError("idx must be (E,H,W)")
+    _, H, W = idx.shape
+    _, n_cells, C = sums.shape
+    if box_features.shape != (E, Kmax, C) or sums.shape[0] != E:
+        raise ValueError("box_features must be (E,Kmax,C) matching mask_probs and sums (E,cells,C)")
+    _call("eod_write_objects_pasted_det", box_features.data_ptr(), mask_probs.data_ptr(), boxes.data_ptr(), _ptr(n_obj), Kmax, S, H, W,
+          float(threshold), idx.data_ptr(), samp.data_ptr(), frame_cnt.data_ptr(), E, C, n_cells, sums.data_ptr(), ws.buf.data_ptr(), ws.nbytes,
+          _stream())
 
 
 def flush_slots(frame_cnt: torch.Tensor, slots: ObjectSlots, sums: torch.Tensor) -> None:

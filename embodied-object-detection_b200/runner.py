@@ -235,8 +235,9 @@ class EpisodeRunner:
     ``feat`` (R,C,H,W) [dense regime] or ``box_features`` (R,K,C) + ``mask_probs`` (R,K,S,S) + ``boxes`` (R,K,4) + ``n_obj`` (R).
     ``trusted_indices = True`` on the provider skips the range check of staged ``idx`` planes.
     ``variant = WRITE_DET``: the dense write is the deterministic one, so a run reproduces bit for bit whatever the slot count and the
-    wave a stream lands in (size its workspace with ``batch.det_runs_per_episode``); the detection regime has no deterministic write
-    and raises EodError.
+    wave a stream lands in (size its workspace with ``batch.det_runs_per_episode``).  ``object_variant = WRITE_DET`` does the same for
+    the detection regime (``EpisodeBatch(object_variant=)``); a detection frame with ``variant = WRITE_DET`` but the default
+    ``object_variant`` raises EodError, since that run would not reproduce.
     ``regime = "heightmax"``: the slots are a ``HeightMaxBatch`` (``layout`` and ``linlayer`` = (weight, bias) | None as it takes them);
     frames carry ``feat`` and depth + pose or ``proj_indices`` + ``height`` (+ ``outlier``); anything else staged (detections, an index
     plane without heights) raises EodError.  There is no read, so ``on_levels`` is not called; ``save_dir`` receives
@@ -248,7 +249,7 @@ class EpisodeRunner:
                  intr: Optional[Sequence[float]] = None, cell: float = 0.2, order: int = ORDER_ZX, layout: int = LAYOUT_CHW,
                  save_dir: Optional[str] = None, zs_weight: Optional[torch.Tensor] = None, obs_score_thresh: float = 0.4,
                  n_semmap_classes: int = 20, sample_stride: int = 8, mask_thresh: float = 0.5, pipeline: bool = True,
-                 variant: int = WRITE_AUTO, regime: str = "mean", linlayer=None):
+                 variant: int = WRITE_AUTO, regime: str = "mean", linlayer=None, object_variant: int = WRITE_AUTO):
         from .memory import EpisodeBatch, HeightMaxBatch
         if test_type not in ("default", "episodic", "longterm"):
             raise ValueError(f"unknown TEST_TYPE {test_type!r}")           # detic/config.py:74
@@ -256,6 +257,8 @@ class EpisodeRunner:
             raise ValueError(f"unknown regime {regime!r} (mean | heightmax)")
         if regime == "heightmax" and variant != WRITE_AUTO:
             raise ValueError("variant selects the mean write; the height-max regime has one update")
+        if regime == "heightmax" and object_variant != WRITE_AUTO:
+            raise ValueError("object_variant selects the object write; the height-max regime has one update")
         self.regime = regime
         self.provider, self.test_type, self.device = provider, test_type, torch.device(device)
         n = provider.n_episodes
@@ -264,7 +267,8 @@ class EpisodeRunner:
         if regime == "heightmax":
             self.batch = HeightMaxBatch(n_slots, map_w, map_h, channels, height, width, self.device, layout=layout, linlayer=linlayer, order=order)
         else:
-            self.batch = EpisodeBatch(n_slots, map_w, map_h, channels, height, width, self.device, layout=layout, variant=variant, pipeline=pipeline)
+            self.batch = EpisodeBatch(n_slots, map_w, map_h, channels, height, width, self.device, layout=layout, variant=variant, pipeline=pipeline,
+                                      object_variant=object_variant)
             self.batch.read_frozen = test_type == "longterm"
         self.intr, self.cell, self.order = intr, float(cell), order
         self.save_dir, self.sample_stride, self.mask_thresh = save_dir, sample_stride, mask_thresh
@@ -312,7 +316,7 @@ class EpisodeRunner:
     def run(self, on_levels: Optional[Callable[[Step, List[torch.Tensor]], None]] = None, max_steps: Optional[int] = None) -> dict:
         """Process this rank's share of the dataset.  on_levels(step, levels): consumer hook, called after every frame-step
         with the three pooled fp16 levels (R,C,h,w) ordered on the caller's stream (idle slots hold stale values).
-        With WRITE_DET the stats carry ``det_overflowed``: some run did not fit the workspace (since it was created) and took the
+        With WRITE_DET (either write) the stats carry ``det_overflowed``: some run did not fit the workspace (since it was created) and took the
         order-dependent reductions - the result is correct but no longer reproducible."""
         b = self.batch
         self.stats = {k: 0 for k in self.stats}                  # per run() call
@@ -340,8 +344,9 @@ class EpisodeRunner:
                     levels = b.step(depth, pose, shifts, self.intr, self.cell, inp["feat"], None, self.order, active=dev[0],
                                     inputs_ready=False, **masks, **geo)
                 else:
-                    if b.variant == WRITE_DET:
-                        raise EodError("EpisodeRunner(variant=WRITE_DET): the object-regime write (detections) is not deterministic")
+                    if b.variant == WRITE_DET and b.object_variant != WRITE_DET:
+                        raise EodError("EpisodeRunner(variant=WRITE_DET): the object-regime write (detections) is not deterministic "
+                                       "(pass object_variant=WRITE_DET)")
                     n_obj = torch.where(dev[0] > 0, inp["n_obj"], torch.zeros_like(inp["n_obj"]))
                     levels = b.step_detections(depth, pose, shifts, self.intr, self.cell, inp["box_features"], inp["mask_probs"], inp["boxes"],
                                                n_obj, self.sample_stride, self.mask_thresh, self.order, inputs_ready=False, **masks, **geo)
@@ -364,7 +369,7 @@ class EpisodeRunner:
             if self.regime == "heightmax":
                 return dict(self.stats)
             b.join()
-            if b.variant == WRITE_DET:
+            if b.variant == WRITE_DET or b.object_variant == WRITE_DET:
                 self.stats["det_overflowed"] = b._det_ws is not None and b._det_ws.overflowed()
         return dict(self.stats)
 

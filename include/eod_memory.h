@@ -218,6 +218,24 @@ int eod_write_objects_pasted(const float *box_features, const float *mask_probs,
                              const int32_t *slot_of_cell, int n_episodes, int C, int64_t n_cells, int n_slots_max,
                              float *scratch, eod_stream_t stream);
 
+/* Deterministic object-regime write (custom_rcnn.py:903-934 accumulated as in :696-697,742): eod_write_objects /
+ * eod_write_objects_pasted, then the per-cell mean added to sums, bitwise reproducible run to run and independent of how episodes
+ * are batched (HW %% 32 == 0, 16-byte aligned samp, else EOD_ERR_UNSUPPORTED).  The result is, bit for bit, what
+ * eod_write_mean_det_layout(EOD_LAYOUT_CHW) gives for the (C,HW) image eod_box_to_image_features builds from the same objects
+ * (the pasted masks for the _pasted entry), with the same samp, frame_cnt and active = n_obj - without building that image.
+ * frame_cnt: from eod_frame_count WITHOUT the slot table, with n_obj as its active mask: a slot with n_obj[e] <= 0 gets no runs,
+ * its inputs are not read and its sums are left alone.  Any Kmax; box_features and sums 16-byte aligned.
+ * workspace: the workspace of eod_write_mean_det - the same eod_write_mean_det_workspace_bytes sizing, zero-filled once, one
+ * workspace may serve both writes; runs that do not fit fall back to fp32 reductions and set the int32 at byte offset
+ * eod_write_mean_det_status_offset(E, cells) to 1. */
+int eod_write_objects_det(const float *box_features, const uint8_t *masks, const int32_t *n_obj, int Kmax, const int32_t *idx,
+                          const uint8_t *samp, const uint32_t *frame_cnt, int n_episodes, int C, int HW, int64_t n_cells, float *sums,
+                          void *workspace, int64_t workspace_bytes, eod_stream_t stream);
+int eod_write_objects_pasted_det(const float *box_features, const float *mask_probs, const float *boxes, const int32_t *n_obj,
+                                 int Kmax, int S, int H, int W, float threshold, const int32_t *idx, const uint8_t *samp,
+                                 const uint32_t *frame_cnt, int n_episodes, int C, int64_t n_cells, float *sums, void *workspace,
+                                 int64_t workspace_bytes, eod_stream_t stream);
+
 /* sums[cell] += scratch[slot] / n_cell for every claimed slot (the per-cell mean of custom_rcnn.py:931-934 added
  * once, :696-697,742); scratch rows, slot_of_cell entries and n_slots return to zero.  Run before
  * eod_finalize_counts (which clears frame_cnt). */
