@@ -8,13 +8,14 @@
 // memory levels L (what eod_read_pool produces) with the same boxes gives the per-ROI map feature that the fused path
 // carries implicitly.  This kernel is that pooling, for all proposals of all episodes in one launch:
 //   * level assignment in the kernel, detectron2 assign_boxes_to_levels: floor(4 + log2(sqrt(area) / 224 + eps)) clamped
-//     to [min_level, max_level] - fp32 like torch;
+//     to [min_level, max_level] - fp32 like torch.  A box with no level there (NaN size: inverted in exactly one axis, or a NaN
+//     coordinate) and a box whose batch_idx names no episode pool nothing: zero bins, valid 0, level -1;
 //   * bilinear sampling with the exact point set, clamping rules and operation order of the ROIAlign CPU kernel
 //     (torchvision/csrc/ops/cpu/roi_align_kernel.cpp, which tests/ execute as the oracle): per bin, samples row-major,
 //     val = w1*v1 + w2*v2 + w3*v3 + w4*v4 accumulated in fp32, then / count;
 //   * a warp owns one (proposal, bin); lanes own C/32 consecutive channels, so every tap is one coalesced C*2-byte row of a
 //     channels-last fp16 level (the levels of a frame, 6 300 pixels x C, live in L2).
-// Output: (R, P, P, C) fp32 channels-last (logical (R, C, P, P)), plus the level each proposal was assigned to.
+// Output: (R, P, P, C) fp32 channels-last (logical (R, C, P, P)), plus the level each proposal was assigned to (-1: none).
 #include "eod_common.cuh"
 
 namespace {
@@ -49,7 +50,7 @@ __device__ __forceinline__ void load_tap<4>(const __half *row, int lane, float (
     v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y;
 }
 
-// detectron2 modeling/poolers.py assign_boxes_to_levels (fp32 tensor arithmetic)
+// detectron2 modeling/poolers.py assign_boxes_to_levels (fp32 tensor arithmetic); -1 for no level
 __device__ __forceinline__ int assign_level(float x1, float y1, float x2, float y2, int n_levels, int min_level, float canonical_size,
                                             int canonical_level)
 {
@@ -57,14 +58,15 @@ __device__ __forceinline__ int assign_level(float x1, float y1, float x2, float 
     const float s = __fsqrt_rn(area);
     const float lg = log2f(__fadd_rn(__fdiv_rn(s, canonical_size), 2.220446049250313e-16f));
     float lvl = floorf(__fadd_rn((float)canonical_level, lg));
-    // NaN (negative area) -> torch's float->int64 cast of NaN is INT64_MIN on x86, which the clamp turns into min_level
-    if (!(lvl == lvl)) lvl = -1e30f;
+    // NaN (negative area, NaN coordinate): torch.clamp keeps the NaN and the cast to int64 after it yields an integer outside every
+    // level, so ROIPooler pools the box from no level
+    if (!(lvl == lvl)) return -1;
     lvl = fminf(fmaxf(lvl, (float)min_level), (float)(min_level + n_levels - 1));
     return (int)lvl - min_level;
 }
 
 template <int C>
-__global__ void __launch_bounds__(256) read_roi_kernel(RoiLevels L, const float *__restrict__ boxes, const int32_t *__restrict__ batch_idx, int R, int P,
+__global__ void __launch_bounds__(256) read_roi_kernel(RoiLevels L, const float *__restrict__ boxes, const int32_t *__restrict__ batch_idx, int n_episodes, int P,
                                                        int sampling_ratio, int min_level, float canonical_size, int canonical_level,
                                                        float *__restrict__ out, int32_t *__restrict__ out_level, float *__restrict__ out_valid)
 {
@@ -72,19 +74,21 @@ __global__ void __launch_bounds__(256) read_roi_kernel(RoiLevels L, const float 
     const int r = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
     const float x1 = __ldg(boxes + 4 * r), y1 = __ldg(boxes + 4 * r + 1), x2 = __ldg(boxes + 4 * r + 2), y2 = __ldg(boxes + 4 * r + 3);
-    const int lv = assign_level(x1, y1, x2, y2, L.n, min_level, canonical_size, canonical_level);
-    if (threadIdx.x == 0 && out_level) out_level[r] = lv;
+    int lv = assign_level(x1, y1, x2, y2, L.n, min_level, canonical_size, canonical_level);
     const int e = batch_idx ? __ldg(batch_idx + r) : 0;
-    const int h = L.h[lv], w = L.w[lv];
-    const float sc = L.scale[lv];
-    const __half *base = L.ptr[lv] + (size_t)e * h * w * C;
+    if (e < 0 || e >= n_episodes) lv = -1;
+    if (threadIdx.x == 0 && out_level) out_level[r] = lv;
+    const bool none = lv < 0;                       // takes no samples below: zero bins, valid 0
+    const int h = L.h[none ? 0 : lv], w = L.w[none ? 0 : lv];
+    const float sc = L.scale[none ? 0 : lv];
+    const __half *base = L.ptr[none ? 0 : lv] + (size_t)(none ? 0 : e) * h * w * C;
     // ROIAlign, aligned = true (detectron2 ROIAlignV2): half-pixel offset, no minimum roi size
     const float rsw = __fsub_rn(__fmul_rn(x1, sc), 0.5f), rsh = __fsub_rn(__fmul_rn(y1, sc), 0.5f);
     const float rew = __fsub_rn(__fmul_rn(x2, sc), 0.5f), reh = __fsub_rn(__fmul_rn(y2, sc), 0.5f);
     const float roi_w = __fsub_rn(rew, rsw), roi_h = __fsub_rn(reh, rsh);
     const float bin_h = __fdiv_rn(roi_h, (float)P), bin_w = __fdiv_rn(roi_w, (float)P);
-    const int gh = sampling_ratio > 0 ? sampling_ratio : (int)ceilf(__fdiv_rn(roi_h, (float)P));
-    const int gw = sampling_ratio > 0 ? sampling_ratio : (int)ceilf(__fdiv_rn(roi_w, (float)P));
+    const int gh = none ? 0 : sampling_ratio > 0 ? sampling_ratio : (int)ceilf(__fdiv_rn(roi_h, (float)P));
+    const int gw = none ? 0 : sampling_ratio > 0 ? sampling_ratio : (int)ceilf(__fdiv_rn(roi_w, (float)P));
     const float count = (float)max(gh * gw, 1);
 
     for (int bin = warp; bin < P * P; bin += n_warps) {
@@ -121,7 +125,7 @@ __global__ void __launch_bounds__(256) read_roi_kernel(RoiLevels L, const float 
             }
         }
         // what ROIAlign makes of a constant-1 plane: the share of this bin's sample points that fall on the level (the bias of a 1x1
-        // projection applied BEFORE the pooling survives it with exactly this factor; 0 for empty / inverted boxes)
+        // projection applied BEFORE the pooling survives it with exactly this factor; 0 for empty / inverted boxes and boxes without a level)
         if (out_valid && lane == 0) out_valid[(size_t)r * P * P + bin] = __fdiv_rn((float)n_valid, count);
         float *dst = out + ((size_t)r * P * P + bin) * C + (size_t)lane * V;
 #pragma unroll
@@ -153,9 +157,9 @@ extern "C" int eod_read_roi(int n_levels, const void *const *levels, const int *
     EOD_REQUIRE(eod_aligned16(out), EOD_ERR_ALIGN, "eod_read_roi: out must be 16-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
     switch (C) {
-    case 128: read_roi_kernel<128><<<n_rois, 256, 0, st>>>(L, boxes, batch_idx, n_rois, pooled, sampling_ratio, min_level, canonical_size, canonical_level, out, out_level, out_valid); break;
-    case 256: read_roi_kernel<256><<<n_rois, 256, 0, st>>>(L, boxes, batch_idx, n_rois, pooled, sampling_ratio, min_level, canonical_size, canonical_level, out, out_level, out_valid); break;
-    case 512: read_roi_kernel<512><<<n_rois, 256, 0, st>>>(L, boxes, batch_idx, n_rois, pooled, sampling_ratio, min_level, canonical_size, canonical_level, out, out_level, out_valid); break;
+    case 128: read_roi_kernel<128><<<n_rois, 256, 0, st>>>(L, boxes, batch_idx, n_episodes, pooled, sampling_ratio, min_level, canonical_size, canonical_level, out, out_level, out_valid); break;
+    case 256: read_roi_kernel<256><<<n_rois, 256, 0, st>>>(L, boxes, batch_idx, n_episodes, pooled, sampling_ratio, min_level, canonical_size, canonical_level, out, out_level, out_valid); break;
+    case 512: read_roi_kernel<512><<<n_rois, 256, 0, st>>>(L, boxes, batch_idx, n_episodes, pooled, sampling_ratio, min_level, canonical_size, canonical_level, out, out_level, out_valid); break;
     default:
         eod_set_error("eod_read_roi: C=%d not compiled in (128, 256, 512)", C);
         return EOD_ERR_UNSUPPORTED;

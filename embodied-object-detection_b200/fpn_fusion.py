@@ -118,7 +118,8 @@ class MemoryFusion(nn.Module):
         roi, lvl, valid = ops.read_roi(levels, bx, bi, pooled, want_levels=True, want_valid=True)
         if not project:
             return roi
-        out = torch.empty((roi.shape[0], self.merge_map_projections[0].weight.shape[0], pooled, pooled), dtype=torch.float32, device=dev)
+        # a box without a level (lvl -1) pools nothing from the fused levels either: its memory term is zero
+        out = torch.zeros((roi.shape[0], self.merge_map_projections[0].weight.shape[0], pooled, pooled), dtype=torch.float32, device=dev)
         for k, conv in enumerate(self.merge_map_projections):
             sel = (lvl == k).nonzero().squeeze(1)
             if sel.numel():

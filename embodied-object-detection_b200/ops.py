@@ -756,7 +756,9 @@ def read_roi(levels: Sequence[torch.Tensor], boxes: torch.Tensor, batch_idx: Opt
     the FPN level assignment (detic_roi_heads.py:331-334 applied to the memory levels; see eod_read_roi).
     levels: what read_pool returns - logical (E,C,h,w) fp16 tensors in channels-last memory; boxes (R,4) f32 XYXY image pixels;
     batch_idx (R) i32.  Returns logical (R,C,pooled,pooled) f32 in channels-last memory [, assigned level (R) i32] [, valid (R,pooled,
-    pooled) f32: the share of each bin's sample points that lie on the level = ROIAlign of a constant-1 plane]."""
+    pooled) f32: the share of each bin's sample points that lie on the level = ROIAlign of a constant-1 plane].
+    Level -1 means the box pools nothing (zero features, valid 0): detectron2 assigns it no level (its size is NaN: inverted in
+    exactly one axis, or a NaN coordinate), or its batch_idx lies outside [0, E)."""
     import ctypes
     n = len(levels)
     if not (1 <= n <= 4) or len(strides) != n:

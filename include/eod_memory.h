@@ -342,11 +342,14 @@ int eod_read_pool(const void *table, int mem_is_f16, const float *counts, const 
  *     (E, h_l, w_l, C) fp16 channels-last level exactly as eod_read_pool stores it; level_scale[l] = 1 / stride
  *   boxes (R,4) f32 XYXY in image pixels, batch_idx (R) i32 episode of each box (nullable = 0)
  *   out (R, pooled, pooled, C) f32 channels-last (logical (R, C, pooled, pooled)); out_level (R) i32 nullable: assigned level
- * Sample points, clamping and summation order of torchvision's CPU ROIAlign (ops/cpu/roi_align_kernel.cpp); accumulated fp32:
- * within 1e-5 of scale of the executed reference op, level assignments exact.  min_level: index of levels[0] in the pyramid
- * (3 for p3); canonical_size 224, canonical_level 4 in detectron2.  out_valid (nullable, (R,P,P) f32): per bin, the share of its sample
- * points that lie on the level = ROIAlign of a constant-1 plane (1 for boxes inside the image, 0 for empty / inverted boxes): the factor
- * with which the bias of a 1x1 projection applied before the pooling survives it. */
+ * Sample points, clamping and operation order of torchvision's CPU ROIAlign (ops/cpu/roi_align_kernel.cpp), one fp32 rounding per
+ * operation: bit for bit the executed reference op, level assignments exact.  A box that detectron2 assigns to no level (NaN size:
+ * inverted in exactly one axis, or a NaN coordinate) and a box whose batch_idx lies outside [0, n_episodes) pool nothing: zero bins,
+ * valid 0, out_level -1.  min_level: index of levels[0] in the pyramid (3 for p3); canonical_size 224, canonical_level 4 in detectron2.
+ * out_valid (nullable, (R,P,P) f32): per bin, n_valid / count, the share of its sample points that lie on the level = ROIAlign of a
+ * constant-1 plane up to rounding (1 for boxes inside the image, fractional for boxes across the border, 0 for empty / inverted boxes):
+ * the factor with which the bias of a 1x1 projection applied before the pooling survives it.  Coordinates must be finite and within a
+ * few image sizes of the frame: like torchvision, with sampling_ratio 0 a bin takes ceil(roi_h / pooled) x ceil(roi_w / pooled) samples. */
 int eod_read_roi(int n_levels, const void *const *levels, const int *level_h, const int *level_w, const float *level_scale,
                  int n_episodes, int C, const float *boxes, const int32_t *batch_idx, int n_rois, int pooled, int sampling_ratio,
                  int min_level, float canonical_size, int canonical_level, float *out, int32_t *out_level, float *out_valid, eod_stream_t stream);

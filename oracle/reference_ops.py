@@ -352,15 +352,80 @@ def assign_boxes_to_levels(boxes: torch.Tensor, min_level: int = 3, max_level: i
     return lvl.to(torch.int64) - min_level
 
 
+def roi_levels(boxes: torch.Tensor, n_levels: int) -> torch.Tensor:
+    """The level ROIPooler pools each box from: assign_boxes_to_levels with levels 3 .. 3 + n_levels - 1, and -1 where that lies outside
+    [0, n_levels).  A box inverted in exactly one axis (negative area) or with a NaN coordinate has a NaN size; torch.clamp keeps the
+    NaN and the int64 cast turns it into an out-of-range integer, so ROIPooler's `level_assignments == level` matches no level and the
+    box pools zeros.  eod_read_roi reports such a box as level -1."""
+    lvl = assign_boxes_to_levels(boxes, 3, 3 + n_levels - 1)
+    return torch.where((lvl >= 0) & (lvl < n_levels), lvl, torch.full_like(lvl, -1))
+
+
+def _f2i(v):
+    """C's (int) of an fp32 array as the GPU converts it (cvt.rzi.s32.f32): truncation, saturating, NaN -> 0."""
+    import numpy as np
+    v = np.asarray(v, np.float32)
+    return np.where(np.isnan(v), 0, np.clip(np.trunc(np.nan_to_num(v)), -2.0 ** 31, 2.0 ** 31 - 1)).astype(np.int64)
+
+
+def roi_align_f32(level, box, scale: float, pooled: int = 7, sampling_ratio: int = 0):
+    """ROIAlign (aligned=True, detectron2 ROIAlignV2) of one level over one box, restated in eod_read_roi's arithmetic: level (C,h,w)
+    f32 numpy, box 4 XYXY image-pixel coordinates -> (bins (C,pooled,pooled) f32, valid (pooled,pooled) f32 = n_valid / count, the
+    share of each bin's sample points that lie on the level, i.e. ROIAlign of a constant-1 plane up to the rounding of w1+w2+w3+w4).
+    Every operation is one fp32 rounding, in the order of torchvision's CPU kernel (torchvision/csrc/ops/cpu/roi_align_kernel.cpp):
+    sample point, the (-1, h] x (-1, w] test, the clamps, the bilinear weights, val = ((w1 v1 + w2 v2) + w3 v3) + w4 v4, accumulated
+    sample by sample (iy outer, ix inner), then / count.  The bins and channels of one box are independent of each other, so the
+    arrays run over them while the samples stay sequential: every output element sees exactly the kernel's operation order.
+    fp32 -> int casts follow the GPU (NaN -> 0)."""
+    import numpy as np
+    f = np.float32
+    C, h, w = level.shape
+    P = f(pooled)
+    x1, y1, x2, y2 = (f(v) for v in box)
+    sc = f(scale)
+    rsw, rsh = f(f(x1 * sc) - f(0.5)), f(f(y1 * sc) - f(0.5))
+    rew, reh = f(f(x2 * sc) - f(0.5)), f(f(y2 * sc) - f(0.5))
+    roi_w, roi_h = f(rew - rsw), f(reh - rsh)
+    bin_h, bin_w = f(roi_h / P), f(roi_w / P)
+    gh = sampling_ratio if sampling_ratio > 0 else int(_f2i(np.ceil(f(roi_h / P))))
+    gw = sampling_ratio if sampling_ratio > 0 else int(_f2i(np.ceil(f(roi_w / P))))
+    count = f(max(gh * gw, 1))
+    pb = np.arange(pooled, dtype=f)
+    start_y, start_x = (rsh + pb * bin_h).astype(f), (rsw + pb * bin_w).astype(f)           # rs + p * bin, per bin row / column
+    acc = np.zeros((C, pooled, pooled), f)
+    n_valid = np.zeros((pooled, pooled), np.int64)
+    for iy in range(gh):
+        yy = (start_y + f(f(f(iy + 0.5) * bin_h) / f(gh))).astype(f)
+        for ix in range(gw):
+            xx = (start_x + f(f(f(ix + 0.5) * bin_w) / f(gw))).astype(f)
+            y, x = np.broadcast_to(yy[:, None], (pooled, pooled)).copy(), np.broadcast_to(xx[None, :], (pooled, pooled)).copy()
+            empty = (y < -1.0) | (y > f(h)) | (x < -1.0) | (x > f(w))                       # NaN compares false: not empty
+            n_valid += ~empty
+            y[y <= 0] = 0
+            x[x <= 0] = 0
+            y_low, x_low = _f2i(y), _f2i(x)
+            top, right = y_low >= h - 1, x_low >= w - 1
+            y_low[top], x_low[right] = h - 1, w - 1
+            y[top], x[right] = f(h - 1), f(w - 1)
+            y_high, x_high = np.where(top, y_low, y_low + 1), np.where(right, x_low, x_low + 1)
+            ly, lx = (y - y_low.astype(f)).astype(f), (x - x_low.astype(f)).astype(f)
+            hy, hx = (f(1) - ly).astype(f), (f(1) - lx).astype(f)
+            w1, w2, w3, w4 = hy * hx, hy * lx, ly * hx, ly * lx
+            val = ((w1 * level[:, y_low, x_low] + w2 * level[:, y_low, x_high]) + w3 * level[:, y_high, x_low]) + w4 * level[:, y_high, x_high]
+            acc = np.where(empty, acc, acc + val)
+    return (acc / count).astype(f), (n_valid.astype(f) / count).astype(f)
+
+
 def roi_read(levels: Sequence[torch.Tensor], boxes_per_image: Sequence[torch.Tensor], pooled: int = 7, strides=(8, 16, 32)):
     """The box pooling of detic_roi_heads.py:331-334 (detectron2 ROIPooler, ROIAlignV2 = torchvision roi_align(aligned=True),
-    sampling_ratio 0) applied to the pooled MEMORY levels: levels[l] (B,C,h,w) -> (sum n_i, C, pooled, pooled) f32, levels (sum n_i).
-    torchvision's CPU ROIAlign is EXECUTED here; the level assignment is the restatement above."""
+    sampling_ratio 0) applied to the pooled MEMORY levels: levels[l] (B,C,h,w) -> (sum n_i, C, pooled, pooled) f32, levels (sum n_i;
+    -1 for a box ROIPooler pools from no level, see roi_levels).  torchvision's CPU ROIAlign is EXECUTED here; the level assignment is
+    the restatement above."""
     from torchvision.ops import roi_align
     boxes = torch.cat(list(boxes_per_image), 0).float()
     bidx = torch.cat([torch.full((b.shape[0], 1), float(i)) for i, b in enumerate(boxes_per_image)], 0)
     rois = torch.cat([bidx, boxes], 1)
-    lvl = assign_boxes_to_levels(boxes, 3, 3 + len(levels) - 1)
+    lvl = roi_levels(boxes, len(levels))
     out = torch.zeros(boxes.shape[0], levels[0].shape[1], pooled, pooled)
     for k, (x, s) in enumerate(zip(levels, strides)):
         sel = (lvl == k).nonzero().squeeze(1)
